@@ -20,6 +20,9 @@ three cells of the TIMED run replayed through the CPU oracle over every TTI of t
 
   --cells-total N   BASELINE configs[4]: N cells in total, block-partitioned over the ranks (strong
                     sharding: 65536 cells -> 8192 per GPU at 8 GPUs) instead of --cells per GPU.
+  --dump-outputs D  after the timed steps, write what the last timed step returned (rbg_to_ue, tbs_bits, mcs of
+                    rank 0's cells, [TTI][cell][...]) as D/<name>.npy: a fixed, seeded sample of cells within 64 MB.
+                    Inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -261,6 +264,25 @@ def pinned(nbytes, write_combined=False):
     return arr, ptr
 
 
+DUMP_BYTES = 60_000_000   # data of all --dump-outputs files: under 64 MB with room for the .npy headers
+DUMP_TYPES = {"rbg_to_ue": np.float32, "tbs_bits": np.float64, "mcs": np.float32}   # exact for int16 / int32 / uint8
+
+
+def dump_outputs(path, outs):
+    """Writes the [TTI][cell][...] device arrays `outs` as path/<name>.npy.  A batch over DUMP_BYTES keeps a seeded
+    choice of cells (the same on every run with the same arguments) and, for very long steps, the last TTIs."""
+    import torch
+    TT, B = outs["rbg_to_ue"].shape[:2]
+    per_cell_tti = sum(t[0, 0].numel() * np.dtype(DUMP_TYPES[k]).itemsize for k, t in outs.items())
+    n_tti = min(TT, DUMP_BYTES // per_cell_tti)
+    n_cells = min(B, DUMP_BYTES // (per_cell_tti * n_tti))
+    cells = np.sort(np.random.default_rng(SEED).choice(B, n_cells, replace=False))
+    idx = torch.from_numpy(cells).to(outs["rbg_to_ue"].device)
+    os.makedirs(path, exist_ok=True)
+    for k, t in outs.items():
+        np.save(os.path.join(path, k + ".npy"), t[TT - n_tti:].index_select(1, idx).cpu().numpy().astype(DUMP_TYPES[k]))
+
+
 def oracle_spot_check(args, g, cells, cell0, n_ttis, period, dts, last_out, last_t0):
     """Replays `cells` of the timed device-resident run through the CPU oracle for all n_ttis TTIs (TTI n read CQI /
     rand() slab n % period) and compares the final state of those cells and the outputs of the run's last step."""
@@ -391,6 +413,8 @@ def run_cuda_arm(args, n_gpus):
         dist.all_reduce(tl, op=dist.ReduceOp.SUM)
     ms_max = float(tms.item())
     value = total_cells * TT * K / (ms_max * 1e-3)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"rbg_to_ue": d_rbg, "tbs_bits": d_bits, "mcs": d_mcs})
 
     # ---- the run that was just timed, checked: three of its cells through the CPU oracle, every TTI ----------
     parity_spot = None
@@ -664,7 +688,11 @@ def main():
                     help="timed region of the reference arm: all of DoSchedule, or without DoStopSchedule")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--kernel-only", action="store_true", help="development: skip the e2e and CPU legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's results (a seeded sample of rank 0's cells) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs needs --impl cuda")
     if args.gpus > 1 and "WORLD_SIZE" not in os.environ:
         # convenience: launch ourselves the way the driver does
         os.execv(sys.executable, [sys.executable, "-m", "torch.distributed.run", "--nnodes=1",

@@ -1,8 +1,15 @@
-"""GPU: the drop-in itself.  oracle/_ref/ref_harness_gpu is the reference's own LTE-Sim
-(SingleCellWithI scenario, unmodified sources) with the product's host plug-in
-(radiosaber_b200/host/rs_gpu_scheduler.h -> C ABI -> CUDA) installed in the eNB instead of the
-reference scheduler class (ids 1, 7, 8, 9, 10, 11, 101, 103).  It must reproduce, record for record, what the reference classes
-produced on the same CQI / rand() inputs (tests/golden)."""
+"""GPU: the drop-in itself.  The product's host plug-in (radiosaber_b200/host/rs_gpu_scheduler.h -> C ABI -> CUDA)
+installed in place of the reference scheduler class (ids 1, 7, 8, 9, 10, 11, 101, 103) must reproduce, record for record,
+what the reference classes produced on the same CQI / rand() inputs (tests/golden).
+
+Where oracle/_ref/ref_harness_gpu is built (it needs the reference LTE-Sim sources, which are not part of this repository)
+the plug-in runs inside the reference's own SingleCellWithI scenario.  Otherwise build/dropin/dropin_replay runs the same
+header against the stand-in LTE-Sim classes of oracle/dropin/ltesim.h, fed each TTI with what the record says the
+simulator handed the reference scheduler (clock, CQI, queues, head-of-line delays, rand() values); the bearers' rates and
+counters and the slice state chain on their own from the first TTI, and the record is compared field for field.  The
+two-bearer cell is replayed from per-bearer records and compared through its log text.  Which path ran is named in
+every failure message."""
+import gzip
 import json
 import os
 import subprocess
@@ -10,11 +17,50 @@ import subprocess
 import numpy as np
 import pytest
 
+from radiosaber_b200 import workload
 from tests.helpers import ROOT, load_golden
 from tools import golden_io
 
 pytestmark = pytest.mark.gpu
-HARNESS = os.path.join(ROOT, "oracle", "_ref", "ref_harness_gpu")
+HARNESS = os.path.join(ROOT, "oracle", "_ref", "ref_harness_gpu")   # make -C oracle ref gpu REF=<reference source tree>
+REPLAY = os.path.join(ROOT, "build", "dropin", "dropin_replay")       # make -C oracle dropin (__graft_entry__.build())
+
+
+def write_replay(path, now, cqi, exists, app_id, avg0, tx0, last0, state0, queue, hol, draws):
+    """dropin_replay's --replay file (layout in oracle/dropin/dropin_replay.cpp); per-bearer arrays are [..][U][NB]."""
+    T, U, G = cqi.shape
+    NB = exists.shape[1]
+    with open(path, "wb") as f:
+        # PacketScheduler counts TTIs from the start of the run: 1 ms each
+        f.write(np.array([T, U, len(state0), G, NB, int(round(now[0] * 1000))], "<i4").tobytes())
+        f.write(exists.astype(np.uint8).tobytes() + app_id.astype("<i4").tobytes())
+        f.write(avg0.astype("<f8").tobytes() + tx0.astype("<i4").tobytes())
+        f.write(np.float64(last0).tobytes() + np.asarray(state0, "<f8").tobytes())
+        f.write(np.ascontiguousarray(cqi, dtype=np.uint8).tobytes())
+        for t in range(T):
+            f.write(np.float64(now[t]).tobytes())
+            f.write((queue[t] > 0).astype(np.uint8).tobytes() + queue[t].astype("<i4").tobytes() + hol[t].astype("<f8").tobytes())
+            f.write(np.array([len(draws[t])], "<i4").tobytes() + np.asarray(draws[t], "<i4").tobytes())
+
+
+def scripted_draws(rec, algo):
+    """The rand() values the reference's DoSchedule drew, per TTI (ids 1 and 7 draw none)."""
+    if algo == 11:
+        return [rec["rand_ng"][t, :int(rec["rand_ng_n"][t])] for t in range(int(rec["T"]))]
+    if algo in (8, 9, 10, 101, 103):
+        return list(rec["rand2"])
+    return [np.zeros(0)] * int(rec["T"])
+
+
+def write_replay_inputs(path, rec):
+    """dropin_replay's --replay file from a golden record: one bearer per UE."""
+    T, U = int(rec["T"]), int(rec["U"])
+    queue = rec["queue"] if "queue" in rec else np.full((T, U), 100000000, np.int32)
+    hol = rec["hol"] if "hol" in rec else np.zeros((T, U))
+    write_replay(path, rec["now"], rec["cqi"], np.ones((U, 1)), np.arange(U)[:, None], rec["avg_before"][0][:, None],
+                 rec["tx_before"][0][:, None], rec["now"][0] - rec["dt"][0], rec["state_before"][0], queue[:, :, None],
+                 hol[:, :, None], scripted_draws(rec, int(rec["algo"])))
+
 
 CASES = ["a9_fix20x5_synth", "a9_diffw_synth", "a9_diffw_trace", "a9_small_synth", "a8_fix20x5_synth", "a8_small_synth",
          "a7_fix20x5_synth", "a7_mix20_synth", "a7_small_synth", "a1_fix20x5_synth", "a1_small_synth",
@@ -30,8 +76,6 @@ CASES = ["a9_fix20x5_synth", "a9_diffw_synth", "a9_diffw_trace", "a9_small_synth
 
 @pytest.mark.parametrize("name", CASES)
 def test_plugin_inside_lte_sim_matches_reference(name, tmp_path):
-    if not os.path.exists(HARNESS):
-        pytest.fail("oracle/_ref/ref_harness_gpu missing: run __graft_entry__.build() where /root/reference is mounted")
     rec = load_golden(name)
     S, U, T = int(rec["S"]), int(rec["U"]), int(rec["T"])
     cfg = {"slices": [], "ues_per_slice": [int((rec["ue_to_slice"] == s).sum()) for s in range(S)]}
@@ -51,12 +95,22 @@ def test_plugin_inside_lte_sim_matches_reference(name, tmp_path):
     extra = ["--alloc-log", str(tmp_path / "alloc.bin")] if algo == 10 else []
     if algo == 11:
         extra = ["--rand-log", str(tmp_path / "draws.bin")]
-    r = subprocess.run([HARNESS, "--gpu", "--algo", str(algo), "--config", str(tmp_path / "cfg.json"),
-                        "--ttis", str(T), "--cqi", str(tmp_path / "cqi.bin"), "--rand", str(tmp_path / "rand.bin"),
-                        "--out", str(out), "--seed", str(int(rec["seed"]))] + extra, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, (r.stdout[-500:], r.stderr[-500:])
+    # which path ran is part of every failure message: inside the reference's LTE-Sim, or the stand-in replay (where the
+    # rand() values are the record's own, so rand2 checks only that the plug-in draws them in the same number and order)
+    how = "reference LTE-Sim" if os.path.exists(HARNESS) else "stand-in replay"
+    name = f"{name} ({how})"
+    if os.path.exists(HARNESS):
+        cmd = [HARNESS, "--gpu", "--ttis", str(T), "--cqi", str(tmp_path / "cqi.bin"), "--rand", str(tmp_path / "rand.bin"),
+               "--seed", str(int(rec["seed"]))]
+    else:
+        assert os.path.exists(REPLAY), "build/dropin/dropin_replay missing: run __graft_entry__.build()"
+        write_replay_inputs(tmp_path / "replay.bin", rec)
+        cmd = [REPLAY, "--replay", str(tmp_path / "replay.bin")]
+    r = subprocess.run(cmd + ["--algo", str(algo), "--config", str(tmp_path / "cfg.json"), "--out", str(out)] + extra,
+                       capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, (name, r.stdout[-500:], r.stderr[-500:])
     got = golden_io.compact(golden_io.parse_record_stream(str(out)))
-    assert int(got["T"]) == T
+    assert int(got["T"]) == T, name
     fields = ["rbg_to_ue", "bits", "final_cqi", "avg_before", "avg_after", "tx_after", "cum_bytes", "cum_rbs",
               "state_before", "state_after", "dt"]
     if algo in (8, 9, 10, 101, 103):
@@ -87,11 +141,15 @@ def test_plugin_inside_lte_sim_matches_reference(name, tmp_path):
 
 
 # ---- two bearers per UE (internet_flow: 2) ---------------------------------------------------------------------
-# The record format is per UE, so here the golden is the reference's own log text (tools/make_golden_logs_two_bearers.py):
-# the plug-in inside LTE-Sim must print the same allocation dump (stdout) and the same per-bearer cumu_bytes / cumu_rbs
-# lines (stderr) -- which only happens if every TTI's allocation, every bearer's share of the bytes and, through the
-# bearers' own EWMA, every later TTI are identical.
+# The record format is per UE, so here the golden is the reference's own log text: the plug-in must print the same
+# allocation dump (stdout) and the same per-bearer cumu_bytes / cumu_rbs lines (stderr) -- which only happens if every
+# TTI's allocation, every bearer's share of the bytes and, through the bearers' own EWMA, every later TTI are identical.
+# Inside the reference's LTE-Sim: tests/golden/logs_two_bearers (tools/make_golden_logs_two_bearers.py).  Stand-in replay:
+# the per-bearer records of tests/golden/two_bearers (tools/make_golden_two_bearers.py; every bearer's queue and
+# head-of-line delay per TTI, application ids) with the reference's text of the same run beside them, plus every
+# bearer's rate and byte / RB counters after each TTI.
 TWO_BEARER_LOGS = os.path.join(ROOT, "tests", "golden", "logs_two_bearers")
+TWO_BEARER_RECS = os.path.join(ROOT, "tests", "golden", "two_bearers")
 
 
 def _scheduler_lines(text):
@@ -99,20 +157,52 @@ def _scheduler_lines(text):
     return [l for l in text.splitlines() if not l.startswith("ipflow ") and not l.startswith("all_bytes")]
 
 
+def _compare_logs(want_text, got_text, T, what):
+    want, got = _scheduler_lines(want_text), _scheduler_lines(got_text)
+    assert len(want) > T, what
+    for k, (a, b) in enumerate(zip(want, got)):
+        assert a == b, (what, k, a, b)
+    assert len(got) == len(want), what
+
+
 @pytest.mark.parametrize("algo", [9, 8, 7, 10, 101, 103])
 def test_two_bearers_per_ue_inside_lte_sim(algo, tmp_path):
     from tools import make_golden_logs_two_bearers as mb
-    if not os.path.exists(HARNESS):
-        pytest.fail("oracle/_ref/ref_harness_gpu missing: run __graft_entry__.build() where /root/reference is mounted")
     cfg = json.load(open(mb.CFG))
-    cqi, rnd = mb.write_inputs(str(tmp_path), cfg)
-    cmd = mb.command(HARNESS, algo, cqi, rnd, str(tmp_path / "got"), cfg)
-    r = subprocess.run(cmd[:1] + ["--gpu"] + cmd[1:], capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, (r.stdout[-500:], r.stderr[-500:])
+    if os.path.exists(HARNESS):
+        cqi, rnd = mb.write_inputs(str(tmp_path), cfg)
+        cmd = mb.command(HARNESS, algo, cqi, rnd, str(tmp_path / "got"), cfg)
+        r = subprocess.run(cmd[:1] + ["--gpu"] + cmd[1:], capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, (r.stdout[-500:], r.stderr[-500:])
+        for ext in ("stdout", "stderr"):
+            _compare_logs(open(os.path.join(TWO_BEARER_LOGS, f"a{algo}.{ext}")).read(), (tmp_path / f"got.{ext}").read_text(),
+                          mb.TTIS, (algo, ext, "reference LTE-Sim"))
+        return
+
+    assert os.path.exists(REPLAY), "build/dropin/dropin_replay missing: run __graft_entry__.build()"
+    rec = golden_io.load_npz(os.path.join(TWO_BEARER_RECS, f"a{algo}.npz"))
+    T, U, G = int(rec["T"]), int(rec["U"]), int(rec["G"])
+    now, dts = workload.tti_clock(T)    # the reference's clock from 0.1 s, when the applications start
+    assert np.array_equal(dts, rec["dt"])
+    cqi = workload.synth_cqi(int(rec["seed"]), 0, 1, 0, T, U, G)[:, 0]
+    write_replay(tmp_path / "replay.bin", now, cqi, rec["exists"], rec["app_id"], rec["avg_before"][0], rec["tx_before"][0],
+                 now[0] - dts[0], rec["state_before"][0], rec["queue"], rec["hol"], scripted_draws(rec, algo))
+    extra = ["--alloc-log", str(tmp_path / "alloc.bin")] if algo == 10 else []
+    r = subprocess.run([REPLAY, "--replay", str(tmp_path / "replay.bin"), "--algo", str(algo), "--config", mb.CFG,
+                        "--out", str(tmp_path / "rec.bin"), "--bearer-out", str(tmp_path / "bearers.bin"),
+                        "--log-out", str(tmp_path / "got")] + extra, capture_output=True, text=True, timeout=600)
+    what = (algo, "stand-in replay")
+    assert r.returncode == 0, (what, r.stdout[-500:], r.stderr[-500:])
     for ext in ("stdout", "stderr"):
-        want = _scheduler_lines(open(os.path.join(TWO_BEARER_LOGS, f"a{algo}.{ext}")).read())
-        got = _scheduler_lines((tmp_path / f"got.{ext}").read_text())
-        assert len(want) > mb.TTIS
-        for k, (a, b) in enumerate(zip(want, got)):
-            assert a == b, (algo, ext, k, a, b)
-        assert len(got) == len(want), (algo, ext)
+        with gzip.open(os.path.join(TWO_BEARER_RECS, f"a{algo}.{ext}.gz"), "rt") as f:
+            _compare_logs(f.read(), (tmp_path / f"got.{ext}").read_text(), T, what + (ext,))
+    got = golden_io.parse_record_stream(str(tmp_path / "rec.bin"))
+    fields = ["bits", "final_cqi", "state_after"] + (["rbg_to_ue"] if algo != 10 else [])
+    fields += ["target", "quota"] if algo != 7 else ["nvs_slice"]
+    for f in fields:
+        assert np.array_equal(np.asarray(got[f]), np.asarray(rec[f])), what + (f,)
+    post = np.dtype([("avg", "<f8"), ("tx", "<i4"), ("pad", "<i4"), ("cum_bytes", "<u8"), ("cum_rbs", "<u8")])
+    per_bearer = np.fromfile(tmp_path / "bearers.bin", dtype=post).reshape(T, U, 2)
+    ex = rec["exists"].astype(bool)
+    for k, gk in (("avg", "avg_after"), ("tx", "tx_after"), ("cum_bytes", "cum_bytes"), ("cum_rbs", "cum_rbs")):
+        assert np.array_equal(per_bearer[k][:, ex], rec[gk][:, ex]), what + (gk,)

@@ -14,7 +14,8 @@ from radiosaber_b200 import sched, workload
 from tests.helpers import GOLDEN, load_golden
 
 FIX = os.path.join(GOLDEN, "traces", "trace_subset.npz")
-REF_TRACES = "/root/reference/cqi-traces-noise0"
+# the reference's own trace files (a RadioSaber checkout named by RS_REFERENCE), for the provenance check of the fixture
+REF_TRACES = os.path.join(os.environ["RS_REFERENCE"], "cqi-traces-noise0") if os.environ.get("RS_REFERENCE") else ""
 TRACE_GOLDENS = ["a9_fix20x5_trace", "a8_fix20x5_trace", "a7_fix20x5_trace", "a1_fix20x5_trace", "a9_diffw_trace",
                  "a10_fix20x5_trace", "a11_fix20x5_trace"]
 
@@ -86,7 +87,8 @@ def test_parsers_round_trip(tmp_path):
     assert got.tolist() == [7] and np.array_equal(tr[0], a)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_TRACES), reason="reference traces not mounted")
+@pytest.mark.skipif(not os.path.isdir(REF_TRACES), reason="needs the reference's cqi-traces-noise0 files (RS_REFERENCE=<checkout>), "
+                    "which are not part of this repository: the fixture's provenance and the full-file parse go unchecked")
 def test_fixture_equals_reference_files():
     mapping, ids, rows, slot = _fixture()
     assert np.array_equal(sched.parse_mapping_file(os.path.join(REF_TRACES, "mapping1.config")), mapping)
