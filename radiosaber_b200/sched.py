@@ -362,10 +362,16 @@ class Scheduler:
         return out
 
     # ---- device-resident path (raw device pointers, e.g. torch tensors' data_ptr()) -----------
+    def _device_queues(self, d_queue, d_hol):
+        """Hand the next run call DEVICE queue state ([T][B][U] or [T][B][U][2] int32 / float64, rs_set_queues)."""
+        if d_queue or d_hol:
+            _check(lib().rs_set_queues(self._h, C.c_void_p(d_queue or None), C.c_void_p(d_hol or None)))
+
     def run_device(self, n_ttis, d_cqi, cqi_tti_stride, d_rand2, dt, d_out=None, d_active=0,
-                   active_tti_stride=0, ttis_per_launch=0, cqi_refresh=1):
+                   active_tti_stride=0, ttis_per_launch=0, cqi_refresh=1, d_queue=0, d_hol=0):
         dt = np.ascontiguousarray(dt, dtype=np.float64)
         assert dt.shape[0] >= n_ttis
+        self._device_queues(d_queue, d_hol)
         o = _Out(*[(d_out or {}).get(k) for k in ("rbg_to_ue", "tbs_bits", "mcs", "final_cqi", "slice_target",
                                                     "slice_quota", "nvs_slice", "alloc_n", "alloc_ue", "alloc_rbg")])
         _check(lib().rs_run_device(self._h, int(n_ttis), C.c_void_p(d_cqi), int(cqi_tti_stride), int(cqi_refresh),
@@ -382,8 +388,10 @@ class Scheduler:
         _check(lib().rs_set_traces(self._h, _ptr(traces), traces.shape[0], traces.shape[1], _ptr(ue_trace)))
         self.trace_rows = int(traces.shape[1])
 
-    def run_traces_host(self, trace_row, rand2, dt, active=None, want_aux=False, ttis_per_launch=0):
-        """T TTIs with the CQI replayed from the loaded traces; trace_row: int32 [T] (-1 = no report yet)."""
+    def run_traces_host(self, trace_row, rand2, dt, active=None, want_aux=False, ttis_per_launch=0, queue=None,
+                        hol=None):
+        """T TTIs with the CQI replayed from the loaded traces; trace_row: int32 [T] (-1 = no report yet); queue / hol
+        as run_host."""
         B, U = self.B, self.U
         dt = np.ascontiguousarray(dt, dtype=np.float64)
         T = int(dt.shape[0])
@@ -392,15 +400,17 @@ class Scheduler:
         rand2 = None if rand2 is None else self._draws(rand2, (T, B))
         act = None if active is None else np.ascontiguousarray(active, dtype=np.uint8).reshape(T, B, U)
         out, o = self._host_outputs(T, want_aux)
+        keep = self._queues(queue, hol, (T, B))
         _check(lib().rs_run_traces_host(self._h, T, _ptr(trace_row), _ptr(rand2), _ptr(act), _ptr(dt), C.byref(o),
                                         int(ttis_per_launch)))
         return out
 
     def run_traces_device(self, n_ttis, trace_row, d_rand2, dt, d_out=None, d_active=0, active_tti_stride=0,
-                          ttis_per_launch=0):
+                          ttis_per_launch=0, d_queue=0, d_hol=0):
         dt = np.ascontiguousarray(dt, dtype=np.float64)
         trace_row = np.ascontiguousarray(trace_row, dtype=np.int32)
         assert dt.shape[0] >= n_ttis and trace_row.shape[0] >= n_ttis
+        self._device_queues(d_queue, d_hol)
         o = _Out(*[(d_out or {}).get(k) for k in ("rbg_to_ue", "tbs_bits", "mcs", "final_cqi", "slice_target",
                                                     "slice_quota", "nvs_slice", "alloc_n", "alloc_ue", "alloc_rbg")])
         _check(lib().rs_run_traces_device(self._h, int(n_ttis), _ptr(trace_row), C.c_void_p(d_rand2 or None),
