@@ -36,8 +36,8 @@ int rs_comm_unique_id(void* id_out /* RS_NCCL_ID_BYTES */);
 int rs_comm_init_rank(int32_t n_ranks, int32_t rank, const void* id /* RS_NCCL_ID_BYTES */, int32_t device, void** comm);
 void rs_comm_destroy(void* comm);
 
-/* rs_stats_device() of this rank's cells, then ncclReduce(sum, root) of the uint64 [4][S] block on the handle's
- * stream; on the root the totals over all ranks' cells are copied to stats_out (HOST uint64 [4][S]; ignored on the
+/* rs_stats_device() of this rank's cells, then ncclReduce(sum, root) of the uint64 [P][4][S] block on the handle's
+ * stream; on the root the totals over all ranks' cells are copied to stats_out (HOST uint64 [P][4][S]; ignored on the
  * other ranks).  nccl_comm is an ncclComm_t passed as void*.  Every rank of the communicator must call it;
  * synchronous. */
 int rs_reduce_stats(rs_handle* h, void* nccl_comm, int32_t root, uint64_t* stats_out);

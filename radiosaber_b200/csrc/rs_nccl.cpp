@@ -71,18 +71,19 @@ int rs_reduce_stats(rs_handle* h, void* nccl_comm, int32_t root, uint64_t* stats
   ncclComm_t comm = (ncclComm_t)nccl_comm;
   int32_t S = 0, dev = 0;
   if (rs_dims(h, nullptr, &S, nullptr, nullptr, &dev) != RS_OK || S < 1) return nfail("rs_dims", rs_last_error());
+  const size_t n = (size_t)4 * S * rs_n_profiles(h);   /* [P][4][S] */
   int rank = -1;
   NC(ncclCommUserRank(comm, &rank));
   CUR(cudaSetDevice(dev));
   cudaStream_t st = (cudaStream_t)rs_get_stream(h);
   uint64_t* d = nullptr;
-  CUR(cudaMalloc((void**)&d, sizeof(uint64_t) * 4 * (size_t)S));
+  CUR(cudaMalloc((void**)&d, sizeof(uint64_t) * n));
   int rc = rs_stats_device(h, d);
   if (rc != RS_OK) { cudaFree(d); return nfail("rs_stats_device", rs_last_error()); }
-  ncclResult_t r = ncclReduce(d, d, (size_t)4 * S, ncclUint64, ncclSum, root, comm, st);
+  ncclResult_t r = ncclReduce(d, d, n, ncclUint64, ncclSum, root, comm, st);
   cudaError_t e = cudaSuccess;
   if (r == ncclSuccess && rank == root && stats_out)
-    e = cudaMemcpyAsync(stats_out, d, sizeof(uint64_t) * 4 * (size_t)S, cudaMemcpyDeviceToHost, st);
+    e = cudaMemcpyAsync(stats_out, d, sizeof(uint64_t) * n, cudaMemcpyDeviceToHost, st);
   if (r == ncclSuccess && e == cudaSuccess) e = cudaStreamSynchronize(st);
   cudaFree(d);
   if (r != ncclSuccess) return nfail("ncclReduce", ncclGetErrorString(r));
