@@ -50,7 +50,9 @@ extern "C" {
 typedef struct rs_config {
   int32_t algo;             /* 1 PF, 7 NVS, 8 Sequential, 9 RadioSaber, 10 UpperBound, 11 NVS non-greedy, 101 SubOpt, 103 Vogel */
   int32_t n_slices;         /* S  <= RS_MAX_SLICES */
-  int32_t n_ues;            /* U; user j == UE id j (flows/application/Application.cpp:72-123) */
+  int32_t n_ues;            /* U; user j == UE id j (flows/application/Application.cpp:72-123).  1..32767 (user ids are
+                               int16), and a cell's shared-memory layout must fit one CTA: some thousands of UEs,
+                               fewer for ids 7 / 11 with big slices; else RS_ERR_UNSUPPORTED saying which */
   int32_t n_rbs;            /* 512 for 100 MHz (core/spectrum/bandwidth-manager.cpp:98-102) */
   int32_t rbg_size;         /* get_rbg_size(): 8 (utility/eesm-effective-sinr.h:82-103) */
   int32_t cqi_per_rb;       /* CQI layout per UE: 0 = u8 [G], one value per RBG; 1 = u8 [n_rbs], one per RB
@@ -86,10 +88,12 @@ typedef struct rs_outputs {
   /* id 10 (UpperBound, downlink-transport-scheduler.cpp:223-246, 603-616) grants an RBG to every slice that
    * ranks it among its own best quota RBGs, so the grants are a list: slice-major, each slice's grants in
    * the order of its std::sort (the order the RBs are appended to the winners' lists).  For id 10
-   * rbg_to_ue[g] is the highest user id holding RBG g. */
-  int32_t* alloc_n;      /* [B]     number of (user, RBG) grants; entries past 2G are dropped */
-  int16_t* alloc_ue;     /* [B][2G] user of grant e, -1 past alloc_n */
-  int16_t* alloc_rbg;    /* [B][2G] RBG of grant e */
+   * rbg_to_ue[g] is the highest user id holding RBG g.  The slices can make up to S*G grants; every one is
+   * scheduled (RB lists, TBS, counters, slice offsets).  The list arrays hold L = rs_grant_list_len(h) entries per
+   * cell (default 2G): grants past L are left out of the list only, and alloc_n still counts them. */
+  int32_t* alloc_n;      /* [B]     number of (user, RBG) grants, all of them */
+  int16_t* alloc_ue;     /* [B][L]  user of grant e, -1 past alloc_n (or no listed user of the slice on that RBG) */
+  int16_t* alloc_rbg;    /* [B][L]  RBG of grant e */
 } rs_outputs;
 
 typedef struct rs_handle rs_handle;
@@ -117,6 +121,11 @@ int rs_create_profiles(const rs_config* cfgs, int32_t n_profiles, const int32_t*
 int rs_set_cell_profiles(rs_handle* h, const int32_t* cell_profile);
 int32_t rs_n_profiles(const rs_handle* h);
 void rs_destroy(rs_handle* h);
+/* Id 10: entries per cell of the alloc_ue / alloc_rbg outputs, 2G (the default) .. max(S*G, 2G); S*G holds every grant.
+ * Only the list changes, never the schedule.  Synchronous: waits for the handle's work in flight.  RS_ERR_ARG for
+ * other ids or a length outside the range.  rs_grant_list_len: the current length (0 for other ids). */
+int rs_set_grant_list_len(rs_handle* h, int32_t n);
+int32_t rs_grant_list_len(const rs_handle* h);
 
 /* Use an existing CUDA stream (a cudaStream_t passed as void*); NULL = the handle's own. */
 int rs_set_stream(rs_handle* h, void* cuda_stream);
@@ -324,7 +333,8 @@ int rs_log_tti(rs_log* lg, uint64_t timestamp, const uint8_t* cqi, const int16_t
 /* Id 10 (UpperBound, :223-246) books an RBG to several slices: its TTI is logged from the grant list the device
  * returns (rs_outputs.alloc_n / alloc_ue / alloc_rbg of that cell: slice by slice in the order the grants were made,
  * user -1 = a slice without a listed user on that RBG), which is the order of the users' RB lists and of the
- * efficiency sum behind "all_bytes". */
+ * efficiency sum behind "all_bytes".  grant_ue / grant_rbg hold n_grants entries, every grant of the TTI: set the
+ * handle's list length (rs_set_grant_list_len) to S*G, or at least alloc_n, to log a TTI whole. */
 int rs_log_tti_grants(rs_log* lg, uint64_t timestamp, const uint8_t* cqi, int32_t n_grants, const int16_t* grant_ue,
                       const int16_t* grant_rbg, const int32_t* tbs_bits, const uint8_t* final_cqi,
                       const int32_t* slice_target, const int32_t* slice_quota);

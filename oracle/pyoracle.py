@@ -35,7 +35,7 @@ class _Io(C.Structure):
         ("slice_target", C.c_void_p), ("slice_quota", C.c_void_p), ("nvs_slice", C.c_void_p),
         ("alloc_n", C.c_void_p), ("alloc_ue", C.c_void_p), ("alloc_rbg", C.c_void_p),
         ("rand_stride", C.c_int32),
-        ("queue_bytes", C.c_void_p), ("hol_delay", C.c_void_p),
+        ("queue_bytes", C.c_void_p), ("hol_delay", C.c_void_p), ("alloc_len", C.c_int32),
     ]
 
 
@@ -83,7 +83,10 @@ class OracleScheduler:
     """
 
     def __init__(self, algo, weight, params, ue_to_slice, n_cells, n_rbs=512, rbg_size=8, cqi_per_rb=0,
-                 data_to_transmit=100000000, dead_work=0, tbs_row_m1=None, n_threads=1, n_bearers=1):
+                 data_to_transmit=100000000, dead_work=0, tbs_row_m1=None, n_threads=1, n_bearers=1,
+                 grant_list_len=None):
+        """grant_list_len: id 10, entries per cell of the alloc_ue / alloc_rbg outputs (default 2G, S*G lists every
+        grant); alloc_n counts every grant whatever the length."""
         self.algo = int(algo)
         self.ue_to_slice = np.ascontiguousarray(ue_to_slice, dtype=np.int32)
         self.U = int(self.ue_to_slice.shape[0])
@@ -98,6 +101,7 @@ class OracleScheduler:
         self.n_threads = int(n_threads)
         self._row_m1 = None if tbs_row_m1 is None else np.ascontiguousarray(tbs_row_m1, dtype=np.int32)
         self.nb = 2 if int(n_bearers) == 2 else 1
+        self.grant_list_len = 2 * self.G if grant_list_len is None else int(grant_list_len)
         self._cfg = _Cfg(self.algo, self.S, self.U, self.R, self.rbg_size, self.cqi_per_rb,
                          int(data_to_transmit), int(dead_work), int(n_bearers), 0,
                          _ptr(self.weight), _ptr(self.params), _ptr(self.ue_to_slice), _ptr(self._row_m1))
@@ -147,15 +151,16 @@ class OracleScheduler:
                 "nvs_slice": np.empty((B,), dtype=np.int32),
             }
             if self.algo == 10:
-                aux.update({"alloc_n": np.empty((B,), dtype=np.int32), "alloc_ue": np.empty((B, 2 * G), dtype=np.int16),
-                            "alloc_rbg": np.empty((B, 2 * G), dtype=np.int16)})
+                L = self.grant_list_len
+                aux.update({"alloc_n": np.empty((B,), dtype=np.int32), "alloc_ue": np.empty((B, L), dtype=np.int16),
+                            "alloc_rbg": np.empty((B, L), dtype=np.int16)})
         io = _Io(_ptr(self.avg_rate), _ptr(self.tx_bytes), _ptr(self.cum_bytes), _ptr(self.cum_rbs),
                  _ptr(self.slice_offset), _ptr(self.nvs_ewma),
                  _ptr(cqi), _ptr(act), _ptr(rand2), float(dt),
                  _ptr(out["rbg_to_ue"]), _ptr(out["tbs_bits"]), _ptr(out["mcs"]), _ptr(aux.get("final_cqi")),
                  _ptr(aux.get("slice_target")), _ptr(aux.get("slice_quota")), _ptr(aux.get("nvs_slice")),
                  _ptr(aux.get("alloc_n")), _ptr(aux.get("alloc_ue")), _ptr(aux.get("alloc_rbg")),
-                 int(rand2.shape[1]), _ptr(q), _ptr(h))
+                 int(rand2.shape[1]), _ptr(q), _ptr(h), self.grant_list_len)
         rc = lib().rso_step(C.byref(self._cfg), B, C.byref(io), self.n_threads)
         if rc != 0:
             raise RuntimeError(f"rso_step failed: {rc}")

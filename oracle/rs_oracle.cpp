@@ -131,6 +131,7 @@ struct CellView {
   int32_t* alloc_n;
   int16_t* alloc_ue;
   int16_t* alloc_rbg;
+  int alloc_len = 0;       /* entries of alloc_ue / alloc_rbg */
   const int32_t* queue;   /* [U] bytes queued per bearer this TTI, NULL = cfg->data_to_transmit for everyone */
   const double* hol;      /* [U] head-of-line delay, NULL = 0 */
   int nb = 1;             /* bearers per UE; per-bearer arrays are [U][nb] */
@@ -468,7 +469,7 @@ void ClearOutputs(const CellView& c) {
   if (c.quota) std::fill(c.quota, c.quota + cfg->n_slices, 0);
   if (c.nvs_slice) *c.nvs_slice = -1;
   if (c.alloc_n) *c.alloc_n = 0;
-  if (c.alloc_ue) { std::fill(c.alloc_ue, c.alloc_ue + 2 * G, (int16_t)-1); std::fill(c.alloc_rbg, c.alloc_rbg + 2 * G, (int16_t)-1); }
+  if (c.alloc_ue) { std::fill(c.alloc_ue, c.alloc_ue + c.alloc_len, (int16_t)-1); std::fill(c.alloc_rbg, c.alloc_rbg + c.alloc_len, (int16_t)-1); }
 }
 
 /* DownlinkTransportScheduler::DoSchedule, transport.cpp:152-168, ids 8 and 9. */
@@ -566,7 +567,7 @@ void StepTransport(const CellView& c, const int32_t* row_m1) {
         if (uindex < 0) continue;             /* assert in the reference */
         final_rbgs[j] += 1;
         for (int r = rbg * rbg_size; r < (rbg + 1) * rbg_size; ++r) users[uindex].rbs.push_back(r);
-        if (c.alloc_ue && n_alloc < 2 * G) { c.alloc_ue[n_alloc] = (int16_t)users[uindex].id; c.alloc_rbg[n_alloc] = (int16_t)rbg; }
+        if (c.alloc_ue && n_alloc < c.alloc_len) { c.alloc_ue[n_alloc] = (int16_t)users[uindex].id; c.alloc_rbg[n_alloc] = (int16_t)rbg; }
         n_alloc++;
       }
     }
@@ -823,8 +824,9 @@ void StepCell(const rso_config* cfg, rso_io* io, int b, const int32_t* row_m1) {
   c.quota = io->slice_quota ? io->slice_quota + (size_t)b * S : nullptr;
   c.nvs_slice = io->nvs_slice ? io->nvs_slice + b : nullptr;
   c.alloc_n = io->alloc_n ? io->alloc_n + b : nullptr;
-  c.alloc_ue = (io->alloc_ue && io->alloc_rbg) ? io->alloc_ue + (size_t)b * 2 * G : nullptr;
-  c.alloc_rbg = (io->alloc_ue && io->alloc_rbg) ? io->alloc_rbg + (size_t)b * 2 * G : nullptr;
+  c.alloc_len = io->alloc_len > 0 ? io->alloc_len : 2 * G;
+  c.alloc_ue = (io->alloc_ue && io->alloc_rbg) ? io->alloc_ue + (size_t)b * c.alloc_len : nullptr;
+  c.alloc_rbg = (io->alloc_ue && io->alloc_rbg) ? io->alloc_rbg + (size_t)b * c.alloc_len : nullptr;
   c.queue = io->queue_bytes ? io->queue_bytes + (size_t)b * U * nb : nullptr;
   c.hol = io->hol_delay ? io->hol_delay + (size_t)b * U * nb : nullptr;
   ClearOutputs(c);

@@ -65,8 +65,9 @@ typedef struct rso_io {
   int32_t* slice_quota;  /* [B][S] slice_quota_rbgs (ids 8/9) */
   int32_t* nvs_slice;    /* [B] slice served (ids 7/11) */
   int32_t* alloc_n;      /* [B] id 10: number of (user, RBG) grants (an RBG can go to several slices) */
-  int16_t* alloc_ue;     /* [B][2G] id 10: user of grant e, slice-major, each slice's grants in its sorted order; -1 past n */
-  int16_t* alloc_rbg;    /* [B][2G] id 10: RBG of grant e */
+  int16_t* alloc_ue;     /* [B][L] id 10: user of grant e, slice-major, each slice's grants in its sorted order; -1 past n
+                            (the first L of up to S*G grants; alloc_n counts them all) */
+  int16_t* alloc_rbg;    /* [B][L] id 10: RBG of grant e */
   int32_t rand_stride;   /* int32 values per cell in rand2: 0 or 2 for ids 8/9; id 11: >= 300 x the users of a
                             slice, the rand() draws of nvs.cpp:437-446 in call order */
   /* queue state of the (single) bearer of each UE this TTI (SURVEY 8 f3); both optional */
@@ -74,6 +75,7 @@ typedef struct rso_io {
                                  0 = no packets (the bearer is not listed), 100000000 = infinite buffer, else the queue
                                  size; NULL = cfg.data_to_transmit for every UE */
   const double* hol_delay;    /* [B][U] RadioBearer::GetHeadOfLinePacketDelay; NULL = 0 */
+  int32_t alloc_len;          /* L, entries per cell of alloc_ue / alloc_rbg; 0 = 2G */
 } rso_io;
 
 /* One TTI for n_cells cells, n_threads host threads (cells are independent). */

@@ -117,6 +117,7 @@ struct DevCfg {
    * ue_to_slice and slice_ues [P][U], slice_ptr [P][S+1] ([P][2] for id 1), chunk_slice [P][n_chunks+1] (profiles with
    * fewer chunks end in empty ones); cell b uses row cell_profile[b], null = row 0 for every cell */
   const int* cell_profile;
+  int grant_len;           /* id 10: entries per cell of the alloc_ue / alloc_rbg outputs (rs_set_grant_list_len), 2G..S*G */
 };
 
 /* The dimensions of a cell as the device code reads them (see rs_tti_kernel and the shape policies below). */
@@ -141,7 +142,7 @@ struct RunArgs {
   int cell_off;            /* first cell of this launch (the host may run the two halves of a batch on two streams) */
   short* rbg_to_ue; int* tbs_bits; uint8_t* mcs; uint8_t* final_cqi;
   int* slice_target; int* slice_quota; int* nvs_slice;
-  int* alloc_n; short* alloc_ue; short* alloc_rbg;   /* id 10: [T][B], [T][B][2G], [T][B][2G] */
+  int* alloc_n; short* alloc_ue; short* alloc_rbg;   /* id 10: [T][B], [T][B][grant_len], [T][B][grant_len] */
 };
 
 /* ---- shared-memory layout (same function on host and device) --------------------------------- */
@@ -1788,11 +1789,13 @@ __global__ void __launch_bounds__(kThreads, min_cells_per_sm<ALGO, TRACE, SH>())
         /* UpperBound (transport.cpp:223-246, 603-616): every slice with a positive quota takes the first
          * quota entries of ITS OWN std::sort of the G (rbg, efficiency) pairs, so an RBG can be granted
          * to several slices.  One sort of G entries per slice (warp_sort_desc); the grants are parked in
-         * shared memory (slice-major, sorted order) next to the sort buffers. */
-        /* up to five slices at a time, one warp each, on private buffers in the (dead) right slot array; the grant
-         * lists g_ue / g_rbg [2G] sit in the left one */
-        unsigned short* g_ue = c.sb.posl;            /* [2G] */
-        unsigned short* g_rbg = c.sb.posl + 2 * G;   /* [2G] */
+         * shared memory (slice-major, sorted order) next to the sort buffers.  Every grant is booked: the slices
+         * together make at most S * G of them, and the slot arrays hold n >= S * G entries. */
+        /* up to five slices at a time, one warp each, on private buffers in the (dead) right slot array; g_rbg
+         * [S*G] (the RBG of grant wd[s] + k, the k-th of slice s) sits in the left one.  The user of that grant is
+         * win[g * S + s]; once the sorts are done g_ue [S*G] keeps it in grant order in the (then dead) key array. */
+        unsigned short* g_rbg = c.sb.posl;
+        unsigned short* g_ue = c.sb.a;
         constexpr int kSorters = kWarps < 5 ? kWarps : 5;
         int base = 0;
         for (int s = 0; s < S; ++s) {   /* every thread: where each slice's grants start */
@@ -1815,26 +1818,20 @@ __global__ void __launch_bounds__(kThreads, min_cells_per_sm<ALGO, TRACE, SH>())
             for (int i = lane; i < G; i += 32) s2.a[i] = (unsigned short)((c.sb.a[i * S + s] & 0xf000u) | (unsigned)i);
             __syncwarp();
             warp_sort_desc(s2, stack, G, d.sort_depth_g, lane);
-            for (int k = lane; k < q; k += 32) {
-              const int g = s2.out[k] & 0xfff;
-              if (b0 + k < 2 * G) {
-                g_ue[b0 + k] = c.win[g * S + s];
-                g_rbg[b0 + k] = (unsigned short)g;
-              }
-            }
+            for (int k = lane; k < q; k += 32) g_rbg[b0 + k] = s2.out[k] & 0xfff;
             __syncwarp();
           }
         }
         __syncthreads();
-        const int n_grants = min(base, 2 * G);
         for (int u = tid; u < U; u += kThreads) c.den[u] = 0.0;   /* the metric denominators are dead: EESM sums */
         __syncthreads();
         /* per slice, in grant order: the winner's RB list grows by the RBG's RBs (EESM summand per RB) */
         for (int s = tid; s < S; s += kThreads) {
           const int q = c.frb[s], b0 = c.wd[s];
           int cnt = 0;
-          for (int k = 0; k < q && b0 + k < 2 * G; ++k) {
-            const int ue = g_ue[b0 + k], g = g_rbg[b0 + k];
+          for (int k = 0; k < q; ++k) {
+            const int g = g_rbg[b0 + k], ue = c.win[g * S + s];
+            g_ue[b0 + k] = (unsigned short)ue;
             if (ue == kNoUe) continue;
             cnt++;
             double sum = c.den[ue];
@@ -1854,18 +1851,24 @@ __global__ void __launch_bounds__(kThreads, min_cells_per_sm<ALGO, TRACE, SH>())
           else { if (o_tgt) o_tgt[s] = 0; if (o_quo) o_quo[s] = 0; }
         }
         __syncthreads();
-        short* o_au = r.alloc_ue ? r.alloc_ue + tb * 2 * G : nullptr;
-        short* o_ar = r.alloc_rbg ? r.alloc_rbg + tb * 2 * G : nullptr;
-        for (int e = tid; e < 2 * G; e += kThreads) {
-          const bool in = e < n_grants && g_ue[e] != kNoUe;
+        /* the reported list: the first grant_len grants (rs_set_grant_list_len), the schedule holds all of them */
+        const int n_list = d.grant_len;
+        short* o_au = r.alloc_ue ? r.alloc_ue + tb * n_list : nullptr;
+        short* o_ar = r.alloc_rbg ? r.alloc_rbg + tb * n_list : nullptr;
+        for (int e = tid; e < n_list; e += kThreads) {
+          const bool in = e < base && g_ue[e] != kNoUe;
           if (o_au) o_au[e] = in ? (short)g_ue[e] : (short)-1;
           if (o_ar) o_ar[e] = in ? (short)g_rbg[e] : (short)-1;
         }
         if (tid == 0 && r.alloc_n) r.alloc_n[tb] = base;
-        for (int g = tid; g < G; g += kThreads) {   /* single-valued view: the highest UE id holding the RBG */
+        /* single-valued view: the highest UE id holding the RBG.  Slice s granted RBG g to its winner w there exactly
+         * when w's RB mask has g (w is in slice s only) */
+        for (int g = tid; g < G; g += kThreads) {
           int ue = -1;
-          for (int e = 0; e < n_grants; ++e)
-            if (g_rbg[e] == g && g_ue[e] != kNoUe) ue = max(ue, (int)g_ue[e]);
+          for (int s = 0; s < S; ++s) {
+            const int w = c.win[g * S + s];
+            if (w != kNoUe && ((c.mask[2 * w + (g >> 5)] >> (g & 31)) & 1u)) ue = max(ue, w);
+          }
           if (o_rbg) o_rbg[g] = (short)ue;
         }
       } else if (ALGO == 103) {

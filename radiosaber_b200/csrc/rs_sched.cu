@@ -413,8 +413,8 @@ int alloc_slot(rs_handle* h, rs_handle::Slot& s, int T, const rs_outputs* out, b
     if (out->nvs_slice) CU(s.nvs_slice.alloc((size_t)T * B));
     if (h->d.algo == 10) {
       if (out->alloc_n) CU(s.alloc_n.alloc((size_t)T * B));
-      if (out->alloc_ue) CU(s.alloc_ue.alloc((size_t)T * B * 2 * G));
-      if (out->alloc_rbg) CU(s.alloc_rbg.alloc((size_t)T * B * 2 * G));
+      if (out->alloc_ue) CU(s.alloc_ue.alloc((size_t)T * B * h->d.grant_len));
+      if (out->alloc_rbg) CU(s.alloc_rbg.alloc((size_t)T * B * h->d.grant_len));
     }
   }
   if (!s.in_done) {
@@ -551,6 +551,7 @@ int rs_create_profiles(const rs_config* cfgs, int32_t n_profiles, const int32_t*
 
   rs::DevCfg& d = h->d;
   d.algo = algo; d.S = S; d.U = U; d.G = G; d.R = cfg->n_rbs; d.rbg = cfg->rbg_size;
+  d.grant_len = 2 * G;   /* id 10's reported grant list; rs_set_grant_list_len */
   if (cfg->cqi_per_rb < 0 || cfg->cqi_per_rb > 2) { delete h; return fail(RS_ERR_ARG, "cqi_per_rb must be 0, 1 or 2"); }
   if (cfg->cqi_per_rb == 2 && (G % 8) != 0) { delete h; return fail(RS_ERR_UNSUPPORTED, "4-bit CQI layout needs a multiple of 8 RBGs"); }
   d.cqi_per_rb = cfg->cqi_per_rb;
@@ -704,7 +705,7 @@ int rs_create_profiles(const rs_config* cfgs, int32_t n_profiles, const int32_t*
    * 300 x users of the served slice (id 11; the stride is sized for the largest slice) */
   d.rand_stride = (algo == 11) ? 300 * max_slice : (is_transport(algo) ? 2 : 0);
   /* id 10 sorts G entries at a time next to the parked grants; ids 101/103 keep their scratch in the slot arrays */
-  /* id 10: left slot array = the grant lists [4G]; right = five warps x 3G sort buffers; 1024 entries also make the
+  /* id 10: left slot array = the grants' RBGs [S*G]; right = five warps x 3G sort buffers; 1024 entries also make the
    * range lists (5 x 16 stack entries) and the counters (5 x 32) of those warps fit whatever G is */
   const int min_sort_n = (algo == 10) ? std::max(16 * G, 1024)
                          : ((algo == 101 || algo == 103) ? (rs::inter_scratch_bytes(G, S) + 3) / 4 : 0);   /* posl + posr = 4 n bytes */
@@ -893,6 +894,19 @@ int rs_set_cell_profiles(rs_handle* h, const int32_t* cell_profile) {
   return RS_OK;
 }
 
+int rs_set_grant_list_len(rs_handle* h, int32_t n) {
+  if (!h) return fail(RS_ERR_ARG, "null handle");
+  if (h->d.algo != 10) return fail(RS_ERR_ARG, "rs_set_grant_list_len: the grant list is id 10's output");
+  const int G = h->d.G, S = h->d.S;
+  if (n < 2 * G || n > std::max(S * G, 2 * G))
+    return fail(RS_ERR_ARG, "rs_set_grant_list_len: %d outside 2G..max(S*G, 2G) = %d..%d", n, 2 * G, std::max(S * G, 2 * G));
+  const int rc = rs_sync(h);     /* the launches in flight (rs_run_*_async included) write lists of the old length */
+  if (rc != RS_OK) return rc;
+  h->d.grant_len = n;
+  return RS_OK;
+}
+int32_t rs_grant_list_len(const rs_handle* h) { return (h && h->d.algo == 10) ? h->d.grant_len : 0; }
+
 int rs_get_state(rs_handle* h, double* avg_rate, int32_t* tx_bytes, uint64_t* cum_bytes, uint64_t* cum_rbs,
                  double* slice_offset, double* nvs_ewma) {
   if (!h) return fail(RS_ERR_ARG, "null handle");
@@ -942,8 +956,8 @@ void point_outputs(const rs_handle* h, rs::RunArgs* a, const rs_outputs* o, size
   if (wants(h, 1)) a->nvs_slice = o->nvs_slice ? o->nvs_slice + t0 * B : nullptr;
   if (h->d.algo == 10) {
     a->alloc_n = o->alloc_n ? o->alloc_n + t0 * B : nullptr;
-    a->alloc_ue = o->alloc_ue ? o->alloc_ue + t0 * B * 2 * G : nullptr;
-    a->alloc_rbg = o->alloc_rbg ? o->alloc_rbg + t0 * B * 2 * G : nullptr;
+    a->alloc_ue = o->alloc_ue ? o->alloc_ue + t0 * B * h->d.grant_len : nullptr;
+    a->alloc_rbg = o->alloc_rbg ? o->alloc_rbg + t0 * B * h->d.grant_len : nullptr;
   }
 }
 
@@ -1025,7 +1039,7 @@ int run_host_impl(rs_handle* h, int32_t n_ttis, const uint8_t* cqi, int32_t cqi_
   if (ttis_per_launch <= 0) ttis_per_launch = trace_row ? 16 : 8;
   const size_t NB = (size_t)h->d.nb;
   const int TC = std::max(1, std::min(std::min<int>(ttis_per_launch, rs::kMaxTtisPerLaunch), n_ttis));
-  const size_t B = h->B, U = h->d.U, S = h->d.S, G = h->d.G, C = h->cqi_cols;
+  const size_t B = h->B, U = h->d.U, S = h->d.S, G = h->d.G, C = h->cqi_cols, NL = h->d.grant_len;
   const bool slabs = !trace_row && cqi_refresh > 1;   /* consecutive chunks share a CQI slab */
   const bool split = h->parts > 1;
   const int P = h->parts;
@@ -1138,8 +1152,8 @@ int run_host_impl(rs_handle* h, int32_t n_ttis, const uint8_t* cqi, int32_t cqi_
       if (a.slice_quota) CU_DRAIN(cudaMemcpyAsync(out->slice_quota + (size_t)t0 * B * S, s.slice_quota.p, (size_t)T * B * S * 4, cudaMemcpyDeviceToHost, h->copy_out));
       if (a.nvs_slice) CU_DRAIN(cudaMemcpyAsync(out->nvs_slice + (size_t)t0 * B, s.nvs_slice.p, (size_t)T * B * 4, cudaMemcpyDeviceToHost, h->copy_out));
       if (a.alloc_n) CU_DRAIN(cudaMemcpyAsync(out->alloc_n + (size_t)t0 * B, s.alloc_n.p, (size_t)T * B * 4, cudaMemcpyDeviceToHost, h->copy_out));
-      if (a.alloc_ue) CU_DRAIN(cudaMemcpyAsync(out->alloc_ue + (size_t)t0 * B * 2 * G, s.alloc_ue.p, (size_t)T * B * 2 * G * 2, cudaMemcpyDeviceToHost, h->copy_out));
-      if (a.alloc_rbg) CU_DRAIN(cudaMemcpyAsync(out->alloc_rbg + (size_t)t0 * B * 2 * G, s.alloc_rbg.p, (size_t)T * B * 2 * G * 2, cudaMemcpyDeviceToHost, h->copy_out));
+      if (a.alloc_ue) CU_DRAIN(cudaMemcpyAsync(out->alloc_ue + (size_t)t0 * B * NL, s.alloc_ue.p, (size_t)T * B * NL * 2, cudaMemcpyDeviceToHost, h->copy_out));
+      if (a.alloc_rbg) CU_DRAIN(cudaMemcpyAsync(out->alloc_rbg + (size_t)t0 * B * NL, s.alloc_rbg.p, (size_t)T * B * NL * 2, cudaMemcpyDeviceToHost, h->copy_out));
     }
     CU_DRAIN(cudaEventRecord(s.out_done, h->copy_out));
     s.out_rec = true;
@@ -1482,7 +1496,7 @@ int rs_log_tti_grants(rs_log* lg, uint64_t timestamp, const uint8_t* cqi, int32_
   const int U = lg->U, G = lg->G;
   std::vector<std::vector<int>> rbgs(U);
   double sum_bits = 0;   /* :240-244: sum over the grants in the order they were made (slice by slice) */
-  for (int e = 0; e < n_grants && e < 2 * G; ++e) {
+  for (int e = 0; e < n_grants; ++e) {
     const int u = grant_ue[e], g = grant_rbg[e];
     if (u < 0) continue;   /* a slice without a listed user on that RBG: efficiency 0, nobody's RB list grows */
     if (u >= U || g < 0 || g >= G) return fail(RS_ERR_ARG, "rs_log_tti_grants: grant %d = (%d, %d)", e, u, g);
@@ -1551,8 +1565,8 @@ int rs_step_cell(rs_handle* h, const rs_cell_io* io) {
   const size_t o_rbg = take(o.rbg_to_ue, B * G * 2), o_bits = take(o.tbs_bits, B * U * 4), o_mcs = take(o.mcs, B * U),
                o_fc = take(o.final_cqi, B * U), o_tgt = take(o.slice_target && tr, B * S * 4),
                o_quo = take(o.slice_quota && tr, B * S * 4), o_nvs = take(o.nvs_slice && nvs, B * 4),
-               o_an = take(o.alloc_n && h->d.algo == 10, B * 4), o_au = take(o.alloc_ue && h->d.algo == 10, B * 2 * G * 2),
-               o_ar = take(o.alloc_rbg && h->d.algo == 10, B * 2 * G * 2);
+               o_an = take(o.alloc_n && h->d.algo == 10, B * 4), o_au = take(o.alloc_ue && h->d.algo == 10, B * h->d.grant_len * 2),
+               o_ar = take(o.alloc_rbg && h->d.algo == 10, B * h->d.grant_len * 2);
   const size_t total = off;
   if (h->mb_bytes < total) {
     CU(cudaStreamSynchronize(h->stream));
@@ -1614,8 +1628,8 @@ int rs_step_cell(rs_handle* h, const rs_cell_io* io) {
   if (so.slice_quota) memcpy(o.slice_quota, m + o_quo, B * S * 4);
   if (so.nvs_slice) memcpy(o.nvs_slice, m + o_nvs, B * 4);
   if (so.alloc_n) memcpy(o.alloc_n, m + o_an, B * 4);
-  if (so.alloc_ue) memcpy(o.alloc_ue, m + o_au, B * 2 * G * 2);
-  if (so.alloc_rbg) memcpy(o.alloc_rbg, m + o_ar, B * 2 * G * 2);
+  if (so.alloc_ue) memcpy(o.alloc_ue, m + o_au, B * h->d.grant_len * 2);
+  if (so.alloc_rbg) memcpy(o.alloc_rbg, m + o_ar, B * h->d.grant_len * 2);
   return RS_OK;
 }
 

@@ -194,6 +194,7 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
   int32_t* d_draws = nullptr;
   int16_t *d_rbg = nullptr, *d_gue = nullptr, *d_grbg = nullptr;   /* d_g*: id 10's grant list */
   int32_t* d_gn = nullptr;
+  size_t n_list = 0;   /* entries per cell of the grant list */
   int32_t *d_bits = nullptr, *d_tgt = nullptr, *d_quo = nullptr;
   uint8_t* d_fc = nullptr;
   const size_t row = G / 2;
@@ -215,12 +216,14 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
     cu(cudaMalloc(&d_tgt, sizeof(int32_t) * (size_t)TB * B * S), "cudaMalloc");
     cu(cudaMalloc(&d_quo, sizeof(int32_t) * (size_t)TB * B * S), "cudaMalloc");
     out.rbg_to_ue = d_rbg; out.tbs_bits = d_bits; out.final_cqi = d_fc; out.slice_target = d_tgt; out.slice_quota = d_quo;
-    if (a.algo == 10) {
+    if (a.algo == 10) {   /* the logged cell's every grant: up to S*G */
+      check(rs_set_grant_list_len(h, std::max(S * G, 2 * G)), "rs_set_grant_list_len");
+      n_list = rs_grant_list_len(h);
       cu(cudaMalloc(&d_gn, sizeof(int32_t) * (size_t)TB * B), "cudaMalloc");
-      cu(cudaMalloc(&d_gue, sizeof(int16_t) * (size_t)TB * B * 2 * G), "cudaMalloc");
-      cu(cudaMalloc(&d_grbg, sizeof(int16_t) * (size_t)TB * B * 2 * G), "cudaMalloc");
+      cu(cudaMalloc(&d_gue, sizeof(int16_t) * (size_t)TB * B * n_list), "cudaMalloc");
+      cu(cudaMalloc(&d_grbg, sizeof(int16_t) * (size_t)TB * B * n_list), "cudaMalloc");
       out.alloc_n = d_gn; out.alloc_ue = d_gue; out.alloc_rbg = d_grbg;
-      h_gue.resize(2 * (size_t)G); h_grbg.resize(2 * (size_t)G);
+      h_gue.resize(n_list); h_grbg.resize(n_list);
     }
     h_rbg.resize(G); h_bits.resize(U); h_fc.resize(U); h_tgt.resize(S); h_quo.resize(S); h_cqi.resize((size_t)U * row);
   }
@@ -266,8 +269,8 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
         if (a.algo == 10) {
           int32_t n_grants = 0;
           cu(cudaMemcpy(&n_grants, d_gn + tb, sizeof n_grants, cudaMemcpyDeviceToHost), "copy");
-          cu(cudaMemcpy(h_gue.data(), d_gue + tb * 2 * G, sizeof(int16_t) * 2 * G, cudaMemcpyDeviceToHost), "copy");
-          cu(cudaMemcpy(h_grbg.data(), d_grbg + tb * 2 * G, sizeof(int16_t) * 2 * G, cudaMemcpyDeviceToHost), "copy");
+          cu(cudaMemcpy(h_gue.data(), d_gue + tb * n_list, sizeof(int16_t) * n_list, cudaMemcpyDeviceToHost), "copy");
+          cu(cudaMemcpy(h_grbg.data(), d_grbg + tb * n_list, sizeof(int16_t) * n_list, cudaMemcpyDeviceToHost), "copy");
           check(rs_log_tti_grants(lg, ts, h_cqi.data(), n_grants, h_gue.data(), h_grbg.data(), h_bits.data(), h_fc.data(),
                                   h_tgt.data(), h_quo.data()), "rs_log_tti_grants");
         } else {

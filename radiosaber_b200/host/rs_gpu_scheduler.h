@@ -34,6 +34,7 @@
 #include <iostream>
 #include <list>
 #include <stdexcept>
+#include <algorithm>
 #include <chrono>
 #include <string>
 #include <vector>
@@ -207,6 +208,8 @@ class RsGpuScheduler : public PacketScheduler {
     cfg.tbs_row_m1 = row_m1;
     const char* dev = getenv("RS_DEVICE");
     Check(rs_create(&cfg, 1, dev ? atoi(dev) : 0, &h_), "rs_create");
+    /* UpperBound: every slice may take its own best RBGs, up to S * G grants; list them all */
+    if (id_ == 10) Check(rs_set_grant_list_len(h_, std::max(S * n_rbgs_, 2 * n_rbgs_)), "rs_set_grant_list_len");
     cqi_.assign((size_t)U * n_rbs_, 10); /* UserEquipmentRecord's initial CQI, ENodeB.cpp:207-217 */
     active_.assign(U, 0);
     queue_.assign(U, 0);
@@ -337,8 +340,8 @@ class RsGpuScheduler : public PacketScheduler {
     io.out.slice_quota = quota_.data();
     io.out.nvs_slice = &nvs_slice;
     if (id_ == 10) { /* UpperBound books an RBG to several slices: the grants come back as a list */
-      grant_ue_.assign(2 * (size_t)n_rbgs_, -1);
-      grant_rbg_.assign(2 * (size_t)n_rbgs_, -1);
+      grant_ue_.assign((size_t)rs_grant_list_len(h_), -1);
+      grant_rbg_.assign((size_t)rs_grant_list_len(h_), -1);
       io.out.alloc_n = &n_grants;
       io.out.alloc_ue = grant_ue_.data();
       io.out.alloc_rbg = grant_rbg_.data();
@@ -362,7 +365,6 @@ class RsGpuScheduler : public PacketScheduler {
     std::vector<UserToSchedule*> by_id(U, nullptr);
     for (auto it = users->begin(); it != users->end(); ++it) by_id[(*it)->GetUserID()] = *it;
     if (id_ == 10) {
-      if (n_grants > 2 * n_rbgs_) throw std::runtime_error("RsGpuScheduler: more grants than the list holds");
       for (int k = 0; k < n_grants; ++k) {   /* per user in grant order, like the reference fills the RB lists */
         const int ue = grant_ue_[k], g = grant_rbg_[k];
         if (ue < 0 || ue >= U || !by_id[ue]) continue;

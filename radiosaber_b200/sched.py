@@ -36,7 +36,7 @@ ABI_SYMBOLS = (
     "rs_log_stdout", "rs_log_stderr", "rs_log_clear", "rs_log_set_queues", "rs_log_set_app_ids",
     "rs_get_stream", "rs_host_alloc", "rs_host_free", "rs_step_cell", "rs_run_host_async", "rs_run_traces_host_async",
     "rs_wait", "rs_dims", "rs_fixed_shape", "rs_direct_metric",
-    "rs_create_profiles", "rs_set_cell_profiles", "rs_n_profiles",
+    "rs_create_profiles", "rs_set_cell_profiles", "rs_n_profiles", "rs_set_grant_list_len", "rs_grant_list_len",
 )
 
 
@@ -86,6 +86,9 @@ def lib():
         L.rs_set_cell_profiles.argtypes = [C.c_void_p, C.c_void_p]
         L.rs_n_profiles.argtypes = [C.c_void_p]
         L.rs_n_profiles.restype = C.c_int32
+        L.rs_set_grant_list_len.argtypes = [C.c_void_p, C.c_int32]
+        L.rs_grant_list_len.argtypes = [C.c_void_p]
+        L.rs_grant_list_len.restype = C.c_int32
         L.rs_destroy.argtypes = [C.c_void_p]
         L.rs_destroy.restype = None
         L.rs_set_stream.argtypes = [C.c_void_p, C.c_void_p]
@@ -264,6 +267,16 @@ class Scheduler:
             raise ValueError(f"cell_profile has {cp.shape[0]} entries for {self.B} cells")
         _check(lib().rs_set_cell_profiles(self._h, _ptr(cp)))
 
+    @property
+    def grant_list_len(self):
+        """Id 10: entries per cell of the alloc_ue / alloc_rbg outputs (0 for other ids)."""
+        return int(lib().rs_grant_list_len(self._h))
+
+    def set_grant_list_len(self, n):
+        """Id 10: list n grants per cell, 2G (the default) .. S*G (every grant; rs_set_grant_list_len).  The schedule
+        never depends on it: alloc_n counts every grant, the list holds the first n."""
+        _check(lib().rs_set_grant_list_len(self._h, int(n)))
+
     def close(self):
         if getattr(self, "_h", None) is not None and self._h:
             lib().rs_destroy(self._h)
@@ -312,8 +325,8 @@ class Scheduler:
             out["final_cqi"] = np.empty(lead + (U,), np.uint8)
             if self.algo == 10:
                 out["alloc_n"] = np.empty(lead, np.int32)
-                out["alloc_ue"] = np.empty(lead + (2 * G,), np.int16)
-                out["alloc_rbg"] = np.empty(lead + (2 * G,), np.int16)
+                out["alloc_ue"] = np.empty(lead + (self.grant_list_len,), np.int16)
+                out["alloc_rbg"] = np.empty(lead + (self.grant_list_len,), np.int16)
             if self.algo in (8, 9, 10, 101, 103):
                 out["slice_target"] = np.empty(lead + (S,), np.int32)
                 out["slice_quota"] = np.empty(lead + (S,), np.int32)
@@ -532,7 +545,8 @@ class LogWriter:
 
     def tti_grants(self, timestamp, cqi, n_grants, grant_ue, grant_rbg, tbs_bits, final_cqi, slice_target, slice_quota,
                    queue=None, hol=None):
-        """Id 10: one TTI from the grant list (rs_outputs.alloc_*) instead of the single-valued RBG->UE map."""
+        """Id 10: one TTI from the grant list (rs_outputs.alloc_*) instead of the single-valued RBG->UE map.  grant_ue /
+        grant_rbg hold n_grants entries: a handle's list of rs_grant_list_len >= alloc_n (S*G always is)."""
         if queue is not None or hol is not None:
             q = None if queue is None else np.ascontiguousarray(queue, dtype=np.int32)
             h = None if hol is None else np.ascontiguousarray(hol, dtype=np.float64)
@@ -541,7 +555,7 @@ class LogWriter:
              np.ascontiguousarray(tbs_bits, dtype=np.int32), np.ascontiguousarray(final_cqi, dtype=np.uint8),
              np.ascontiguousarray(slice_target, dtype=np.int32), np.ascontiguousarray(slice_quota, dtype=np.int32)]
         c = np.ascontiguousarray(cqi, dtype=np.uint8)
-        assert a[0].size >= min(int(n_grants), 2 * self.G) and a[1].size >= min(int(n_grants), 2 * self.G)
+        assert a[0].size >= int(n_grants) and a[1].size >= int(n_grants)   # every grant of the TTI
         _check(lib().rs_log_tti_grants(self._h, int(timestamp), _ptr(c), int(n_grants), *[_ptr(x) for x in a]))
 
     def set_counters(self, cum_bytes=None, cum_rbs=None):

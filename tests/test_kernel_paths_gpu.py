@@ -59,9 +59,11 @@ class Case:
     all-idle cell 0 and a cell 1 where only slice 1 has data, and optionally finite queues with head-of-line delays."""
 
     def __init__(self, algo, ups, B, T, seed, n_rbs=512, rbg=8, layout=0, trace=False, queue=False, nb=1, refresh=1,
-                 active=True):
+                 active=True, grant_len=None):
+        """grant_len: id 10's grant list length on both sides (None: the default 2G)."""
         rng = np.random.default_rng(seed)
         self.algo, self.B, self.T, self.layout, self.trace, self.nb, self.refresh = algo, B, T, layout, trace, nb, refresh
+        self.grant_len = grant_len
         self.R, self.rbg, self.G = n_rbs, rbg, n_rbs // rbg
         S = self.S = len(ups)
         self.u2s = np.repeat(np.arange(S), ups).astype(np.int32)
@@ -119,6 +121,8 @@ class Case:
         with _env(**env):
             g = sched.Scheduler(self.algo, self.w, self.p, self.u2s, self.B, cqi_per_rb=self.layout, **self.cfg())
         assert g.rand_stride == (self.stride if self.algo in TRANSPORT + (11,) else 0)
+        if self.grant_len is not None:
+            g.set_grant_list_len(self.grant_len)
         if self.trace:
             g.set_traces(self.traces, self.ue_trace)
         return g
@@ -126,7 +130,7 @@ class Case:
     def oracle(self, bounds):
         """Outputs of every TTI ([T][B][...]) and the state after the last TTI of every call."""
         o = OracleScheduler(self.algo, self.w, self.p, self.u2s, self.B, cqi_per_rb=1 if self.layout == 1 else 0,
-                            n_threads=8, **self.cfg())
+                            n_threads=8, grant_list_len=self.grant_len, **self.cfg())
         outs, states = [], []
         for t in range(self.T):
             kw = {} if self.queue is None else {"queue": self.queue[t], "hol": self.hol[t]}
@@ -173,8 +177,8 @@ class Case:
             out["nvs_slice"] = torch.empty((T, B), dtype=torch.int32)
         if self.algo == 10:
             out["alloc_n"] = torch.empty((T, B), dtype=torch.int32)
-            out["alloc_ue"] = torch.empty((T, B, 2 * G), dtype=torch.int16)
-            out["alloc_rbg"] = torch.empty((T, B, 2 * G), dtype=torch.int16)
+            out["alloc_ue"] = torch.empty((T, B, g.grant_list_len), dtype=torch.int16)
+            out["alloc_rbg"] = torch.empty((T, B, g.grant_list_len), dtype=torch.int16)
         out = {k: v.cuda() for k, v in out.items()}
         d_draws, d_act, d_q, d_h = dev(self.draws), dev(self.active), dev(self.queue), dev(self.hol)
         d_slabs = None if self.trace else dev(self.slabs)
@@ -203,10 +207,9 @@ class Case:
         outs, states = got
         w_outs, w_states = want
         for k, v in outs.items():
-            if k in ("alloc_ue", "alloc_rbg"):   # the grant list: alloc_n entries per cell-TTI
+            if k in ("alloc_ue", "alloc_rbg"):   # the grant list: the first alloc_n entries, -1 after them
                 for t, b in np.ndindex(self.T, self.B):
-                    n = int(w_outs["alloc_n"][t, b])
-                    assert np.array_equal(v[t, b, :n], w_outs[k][t, b, :n]), (tag, k, t, b)
+                    assert np.array_equal(v[t, b], w_outs[k][t, b]), (tag, k, t, b, int(w_outs["alloc_n"][t, b]))
                 continue
             bad = np.argwhere(v != w_outs[k])
             assert bad.size == 0, (tag, k, bad[:5].tolist())

@@ -2,10 +2,13 @@
 """Randomised differential run: CUDA path against the CPU oracle on random slice configurations, shapes,
 CQI layouts, idle bearers, finite queues and head-of-line delays, several hundred TTIs each so that the
 state (EWMA rates, offsets, credits) drifts far from its initial values.  Development / soak tool; the unit
-tests under tests/ are the contract.  Usage: python tools/fuzz_parity.py [--seconds 120] [--seed 1] [--wide]
+tests under tests/ are the contract.  Usage: python tools/fuzz_parity.py [--seconds 120] [--seed 1] [--wide] [--limits]
 
 --wide also draws the RBG count from the LTE-Sim bands, two bearers per UE, cells of up to ~600 UEs (512-thread
-CTAs) and the multi-TTI entries (rs_run_host / rs_run_traces_host with a random launch length) instead of rs_step."""
+CTAs) and the multi-TTI entries (rs_run_host / rs_run_traces_host with a random launch length) instead of rs_step.
+
+--limits draws near the limits rs_create accepts instead: every id, 24..64 slices, the bands, up to a few thousand UEs
+and id 10's whole grant list (up to S*G grants, rs_set_grant_list_len)."""
 import argparse
 import os
 import sys
@@ -23,9 +26,31 @@ from radiosaber_b200 import sched, workload  # noqa: E402
 BANDS = [(6, 1), (14, 2), (24, 2), (48, 3), (72, 4), (100, 4), (256, 8), (504, 8), (64, 1), (512, 8)]
 
 
-def one_case(rng, case, wide=False):
+def _limits_draws(rng):
+    """The configuration of a --limits case: (algo, S, u2s, w, p, layout, B, T, R, rbg)."""
+    algo = int(rng.choice([1, 7, 8, 9, 10, 11, 101, 103]))
+    S = int(rng.integers(24, 65))
+    ues = rng.integers(1, 13, S)
+    if rng.random() < 0.5:   # 480 .. 3000 UEs: 512 threads, per-thread UE loops
+        ues = np.maximum(1, np.round(ues * rng.integers(480, 3000) / ues.sum())).astype(np.int64)
+    u2s = np.repeat(np.arange(S), ues).astype(np.int32)
+    w = rng.dirichlet(np.ones(S) * rng.choice([0.3, 0.5, 1.0]))
+    p = np.zeros((S, 4), dtype=np.int32)
+    p[:, 0] = rng.integers(0, 2, S)
+    p[:, 1] = rng.integers(0, 2, S)
+    p[:, 2] = rng.choice([0, 1, 1, 1, 2], S)
+    p[:, 3] = rng.integers(0, 2, S)
+    R, rbg = BANDS[int(rng.integers(0, len(BANDS)))]
+    layout = int(rng.choice([0, 1, 2]))
+    if layout == 2 and (R // rbg) % 8:
+        layout = 0
+    return algo, S, u2s, w, p, layout, int(rng.integers(1, 5)), int(rng.integers(60, 121)), R, rbg
+
+
+def one_case(rng, case, wide=False, limits=False):
     """One random configuration; None or a description of the first mismatch.  wide=False draws exactly what it
-    always has (the seeds of tests/test_fuzz_gpu.py keep their cases); wide=True adds the draws of --wide after them."""
+    always has (the seeds of tests/test_fuzz_gpu.py keep their cases); wide=True adds the draws of --wide after them;
+    limits=True then replaces the configuration with one of --limits (the earlier draws are still made)."""
     algo = int(rng.choice([9, 9, 9, 8, 7, 1, 10, 11, 101, 103]))
     S = int(rng.integers(1, 33))
     ues = rng.integers(1, 9 if algo == 11 else 13, S)
@@ -61,9 +86,20 @@ def one_case(rng, case, wide=False):
             B, T = min(B, 4), min(T, 60)
         entry = str(rng.choice(["step", "host", "trace"]))
         tpl = int(rng.integers(1, 65))
+    grants = None
+    if limits:
+        algo, S, u2s, w, p, layout, B, T, R, rbg = _limits_draws(rng)
+        U, G, nb = len(u2s), R // rbg, 1
+        queue_aware = rng.random() < 0.5
+        with_active = rng.random() < 0.3
+        entry = str(rng.choice(["step", "host", "trace"]))
+        tpl = int(rng.integers(1, 65))
+        grants = max(S * G, 2 * G) if algo == 10 else None
     g = sched.Scheduler(algo, w, p, u2s, B, n_rbs=R, rbg_size=rbg, cqi_per_rb=layout, n_bearers=nb)
+    if grants:
+        g.set_grant_list_len(grants)
     o = OracleScheduler(algo, w, p, u2s, B, n_rbs=R, rbg_size=rbg, cqi_per_rb=1 if layout == 1 else 0, n_threads=8,
-                        n_bearers=nb)
+                        n_bearers=nb, grant_list_len=grants)
     _, dts = workload.tti_clock(T)
     seed = int(rng.integers(1, 1 << 30))
     refresh = int(rng.choice([1, 1, 7, 40]))
@@ -143,11 +179,12 @@ def main():
     ap.add_argument("--seconds", type=float, default=120)
     ap.add_argument("--seed", type=int, default=1)
     ap.add_argument("--wide", action="store_true", help="also draw bands, two bearers, wide cells and multi-TTI entries")
+    ap.add_argument("--limits", action="store_true", help="draw up to 64 slices, the bands and thousands of UEs")
     args = ap.parse_args()
     rng = np.random.default_rng(args.seed)
     t0, n, ttis = time.time(), 0, 0
     while time.time() - t0 < args.seconds:
-        err = one_case(rng, n, wide=args.wide)
+        err = one_case(rng, n, wide=args.wide, limits=args.limits)
         if err:
             print("MISMATCH", err)
             return 1
