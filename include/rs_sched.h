@@ -204,6 +204,61 @@ int rs_step_cell(rs_handle* h, const rs_cell_io* io);
  * HOST pointers for rs_step / rs_run_host / rs_run_traces_host, DEVICE pointers for the *_device calls. */
 int rs_set_queues(rs_handle* h, const int32_t* queue_bytes, const double* hol_delay);
 
+/* ---- per-bearer buffers kept on the device (closed-loop queues) ----------------------------------
+ * rs_set_queues feeds the queue-aware schedulers open loop: the caller says what every bearer holds at every TTI.
+ * With buffers the handle keeps, per bearer (cell b, UE u, slot i = priority i), a FIFO of at most K records
+ * (arrival time, bytes), the sum `queued` of their bytes and a `dropped` byte counter.  Arrivals are an input;
+ * departures are what the scheduler books.  At TTI t of a call, in this order:
+ *   1. arrival: a = arrivals[t][b][u][i] > 0 bytes are pushed as one record stamped arrival_time[t] (queued += a), or,
+ *      when the FIFO already holds K records, refused whole (dropped += a); a <= 0: nothing arrives;
+ *   2. what the scheduler sees, in place of rs_set_queues' values for the TTI: queue min(queued, INT32_MAX) (0 = the
+ *      bearer is not listed) and HoL delay now[t] - (arrival time of the head record), 0 when the FIFO is empty;
+ *   3. the TTI is scheduled exactly as with those values from rs_set_queues;
+ *   4. departure: the bytes booked to the bearer (the increment of its cum_bytes), clamped to queued, leave from the
+ *      head; emptied records are dropped, a record sent in part keeps its arrival time with its remaining bytes.
+ * A bearer flagged backlogged has no FIFO: it shows queue 100000000 (the infinite buffer) and HoL 0 every TTI.
+ * This is a byte FIFO: LTE-Sim's RLC segmentation and header bytes and its application models are not reproduced.
+ * rs_step_cell refuses a buffered handle (inside LTE-Sim the simulator owns the queues). */
+
+/* max_records = K, 1..RS_MAX_BUFFER_RECORDS, or 0 to switch the buffers off and free them.  backlogged: HOST uint8
+ * [B][U][nb] (nb = 2 with two bearers per UE), nonzero = no FIFO; NULL = none.  Enabling (again) empties every FIFO.
+ * Synchronous.  Memory: 24 + 12 K bytes of HBM per bearer. */
+#define RS_MAX_BUFFER_RECORDS 65536
+int rs_enable_buffers(rs_handle* h, int32_t max_records, const uint8_t* backlogged);
+
+/* Traffic for the NEXT run call on a buffered handle (consumed by it, like rs_set_queues, which a buffered handle
+ * refuses).  Every rs_step / rs_run_* call of a buffered handle needs one, with two bearers per UE too.
+ *   arrivals     [T][B][U][nb] int32, bytes arriving at each bearer at TTI t (<= 0: none)
+ *   now          HOST double [T], simulator time of TTI t; never decreases over the calls of the handle (rs_reset_state
+ *                forgets the last one)
+ *   arrival_time HOST double [T], the time stamped on the records TTI t pushes; <= now[t]
+ *   queue_out    [T][B][U][nb] int32 or NULL: the queue sizes step 2 showed the scheduler
+ *   hol_out      [T][B][U][nb] double or NULL: the head-of-line delays step 2 showed (never negative)
+ * arrivals / queue_out / hol_out are HOST pointers for rs_step / rs_run_host* / rs_run_traces_host*, DEVICE pointers
+ * for rs_run_device / rs_run_traces_device.  Bad times are RS_ERR_ARG before anything runs. */
+typedef struct rs_traffic {
+  const int32_t* arrivals;
+  const double* now;
+  const double* arrival_time;
+  int32_t* queue_out;
+  double* hol_out;
+} rs_traffic;
+int rs_set_traffic(rs_handle* h, const rs_traffic* traffic);
+
+/* The buffers' state, HOST arrays [B][U][nb], NULL = not wanted: bytes queued, records held, arrival time of the head
+ * record (0 when empty) and bytes dropped; a backlogged bearer reports 0 in each.  Synchronous: waits for the handle's
+ * work in flight. */
+int rs_get_buffers(rs_handle* h, int64_t* queued, int32_t* n_records, double* head_time, uint64_t* dropped);
+
+/* Synthetic arrivals into DEVICE int32 [n_ttis][B][U][nb] (bit-identical twin of radiosaber_b200/workload.py
+ * synth_arrivals): pkt_bytes and pkts_q16 are HOST int32 [P][S] (P = rs_n_profiles; cell b reads the row of its
+ * profile).  A bearer of slice s gets (q >> 16) + (draw16 < (q & 0xffff)) packets of pkt_bytes[s] bytes per TTI with
+ * q = pkts_q16[s] (packets per TTI in 16.16 fixed point), draw16 the top 16 bits of splitmix64 of a counter over
+ * (cell0 + b, tti0 + t, u, slot) built like rs_synth_cqi's.  pkt_bytes 0 = no arrivals.  Asynchronous on the handle's
+ * stream. */
+int rs_synth_arrivals(rs_handle* h, uint64_t seed, int64_t cell0, int64_t tti0, int32_t n_ttis, const int32_t* pkt_bytes,
+                      const int32_t* pkts_q16, int32_t* d_out);
+
 /* n_ttis consecutive TTIs with every input and output already in DEVICE memory.
  *   d_cqi   [ceil(T/cqi_refresh)][B][U][row]: TTI t reads slab t / cqi_refresh (the reference refreshes
  *           CQI every 40 TTIs, enb-mac-entity.cc:38; the headline workload every TTI);

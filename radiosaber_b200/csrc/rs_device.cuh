@@ -67,6 +67,14 @@ struct ConstTables {
 };
 static __constant__ ConstTables c_tab;   /* one copy per translation unit that holds kernels (rs_kernels.cu sets its own) */
 
+/* One bearer's byte FIFO (rs_enable_buffers): `n` records from ring slot `head` on, `queued` = the sum of their bytes;
+ * n = -1 = a backlogged bearer (no FIFO, the infinite buffer). */
+struct BufMeta {
+  long long queued;
+  unsigned long long dropped;   /* bytes of arrivals refused because the FIFO held its K records */
+  int head, n;
+};
+
 /* ---- per-handle description (lives in kernel parameter space) -------------------------------- */
 struct Layout {
   int avg, den, mtab, tx, mask, seg0, seg1, cnt, a, win, posl, posr,
@@ -143,6 +151,18 @@ struct RunArgs {
   short* rbg_to_ue; int* tbs_bits; uint8_t* mcs; uint8_t* final_cqi;
   int* slice_target; int* slice_quota; int* nvs_slice;
   int* alloc_n; short* alloc_ue; short* alloc_rbg;   /* id 10: [T][B], [T][B][grant_len], [T][B][grant_len] */
+  /* Per-bearer byte FIFOs (rs_enable_buffers), used by the queue-aware kernels only (the fields sit behind every other
+   * parameter, so the other kernels' parameter offsets are those of a handle without them).  buf_k records per bearer,
+   * 0 = off; buf_meta [B][U][nb], buf_time / buf_bytes [B][U][nb][buf_k] (a ring per bearer); arrivals [T][B][U][nb]
+   * bytes arriving at each bearer.  `queue` / `hol` are then written by the kernel (what each TTI shows the scheduler)
+   * before they are read. */
+  int buf_k;
+  BufMeta* buf_meta;
+  double* buf_time;
+  int* buf_bytes;
+  const int* arrivals;
+  double now[kMaxTtisPerLaunch];        /* simulator time of TTI t: HoL delay = now - arrival time of the head record */
+  double arr_time[kMaxTtisPerLaunch];   /* arrival time stamped on the records TTI t pushes */
 };
 
 /* ---- shared-memory layout (same function on host and device) --------------------------------- */
@@ -954,6 +974,49 @@ __device__ __forceinline__ void finalize_ue(const DevCfg& d, const Dims& dm, con
   if (o_fc) o_fc[u] = (uint8_t)fc;
 }
 
+/* Per-bearer byte FIFOs (rs_enable_buffers).  m / tm / by: the bearer's metadata and its ring of K records.  Inlined:
+ * out of line, the calls made the queue-aware kernels spill up to 72 B around them; inlined they stay within 32 B. */
+/* Start of a TTI: the arrival of `a` bytes stamped `at` (tail drop of the whole arrival when K records are held), then
+ * the queue size and head-of-line delay the scheduler sees, written to *q / *h. */
+static __device__ __forceinline__ void buf_arrive(BufMeta* m, double* tm, int* by, int K, int a, double at, double now, int* q,
+                                        double* h) {
+  BufMeta x = *m;
+  if (x.n < 0) { *q = 100000000; *h = 0.0; return; }   /* backlogged: the reference's infinite buffer */
+  if (a > 0) {
+    if (x.n == K) {
+      m->dropped = x.dropped + (unsigned long long)a;
+    } else {
+      const int i = x.head + x.n < K ? x.head + x.n : x.head + x.n - K;
+      tm[i] = at;
+      by[i] = a;
+      x.n++;
+      x.queued += a;
+      m->n = x.n;
+      m->queued = x.queued;
+    }
+  }
+  *q = (int)min(x.queued, (long long)0x7fffffff);
+  *h = x.n > 0 ? __dsub_rn(now, tm[x.head]) : 0.0;
+}
+/* End of a TTI: `sent` bytes booked to the bearer leave from the head, clamped to what is queued.  A record sent in
+ * part keeps its arrival time. */
+static __device__ __forceinline__ void buf_depart(BufMeta* m, int* by, int K, int sent) {
+  BufMeta x = *m;
+  if (sent <= 0 || x.n <= 0) return;
+  long long left = min((long long)sent, x.queued);
+  x.queued -= left;
+  while (left > 0) {
+    const int r = by[x.head];
+    if (r > left) { by[x.head] = r - (int)left; break; }
+    left -= r;
+    x.head = x.head + 1 == K ? 0 : x.head + 1;
+    x.n--;
+  }
+  m->queued = x.queued;
+  m->head = x.head;
+  m->n = x.n;
+}
+
 constexpr int kVogelTab = 16 * 17 + 16 * 17 + 2;   /* id 103: gap ranks [16][17] + acceptance thresholds [ranks + 1], int16 each */
 /* Scratch of ids 101 / 103 in the (dead) slot arrays of the sort; inter_scratch_bytes() of it
  * (make_layout's min_sort_n). */
@@ -1578,6 +1641,17 @@ __global__ void __launch_bounds__(kThreads, min_cells_per_sm<ALGO, TRACE, SH>())
     int* o_tgt = r.slice_target ? r.slice_target + tb * S : nullptr;
     int* o_quo = r.slice_quota ? r.slice_quota + tb * S : nullptr;
 
+    /* ---- buffered handles: arrivals, and the queue / HoL this TTI shows, from the bearers' FIFOs ---- */
+    if (QUEUE && r.buf_k > 0) {
+      const int* arr = r.arrivals + tb * U * nb;
+      for (int q = tid; q < U * nb; q += kThreads) {
+        const size_t i = (size_t)b * U * nb + q;
+        buf_arrive(r.buf_meta + i, r.buf_time + i * r.buf_k, r.buf_bytes + i * r.buf_k, r.buf_k, arr[q], r.arr_time[t],
+                   r.now[t], const_cast<int*>(qd) + q, const_cast<double*>(hl) + q);
+      }
+      __syncthreads();
+    }
+
     /* ---- NVS: SelectSliceToServe (nvs.cpp:94-142) runs before the EWMA update ---------------- */
     int served = -1;
     if (NVS) {
@@ -2191,8 +2265,16 @@ __global__ void __launch_bounds__(kThreads, min_cells_per_sm<ALGO, TRACE, SH>())
     /* ---- P6: link adaptation, accounting, outputs; reset per-TTI scratch ---------------------- */
     for (int u = tid; u < U; u += kThreads) {
       const unsigned m_lo = c.mask[2 * u], m_hi = c.mask[2 * u + 1];
+      const bool fifo = QUEUE && r.buf_k > 0;
+      int tx0 = 0, tx1 = 0;   /* the bytes finalize_ue books to each bearer are the increments of its tx counter */
+      if (fifo) { tx0 = c.tx[nb * u]; if (two) tx1 = c.tx[nb * u + 1]; }
       finalize_ue(d, dm, c, row_of(u), u, m_lo, m_hi, o_bits, o_mcs, o_fc, data_of(u), ALGO == 10 ? c.den : nullptr,
                   two ? qd : nullptr);
+      if (fifo)
+        for (int k = 0; k < nb; ++k) {
+          const size_t i = ((size_t)b * U + u) * nb + k;
+          buf_depart(r.buf_meta + i, r.buf_bytes + i * r.buf_k, r.buf_k, c.tx[nb * u + k] - (k ? tx1 : tx0));
+        }
       c.mask[2 * u] = 0;
       c.mask[2 * u + 1] = 0;
     }
@@ -2294,6 +2376,36 @@ __global__ void rs_synth_rand2_kernel(int* out, unsigned long long key, long lon
                                                : ((tti << 40) ^ (cell << 16) ^ which ^ 0x5EA4C4000000ull);
     out[i] = (int)((splitmix64(ctr ^ key) >> 11) % span);
   }
+}
+
+/* Synthetic arrivals (twin of workload.synth_arrivals): int32 [n_ttis][n_cells][U][nb].  spec [P][S][2] = (packet
+ * bytes, packets per TTI in 16.16 fixed point) of each profile's slices; a bearer gets (q >> 16) + (draw16 < (q & 0xffff))
+ * packets, draw16 the top 16 bits of one counter-based draw per (tti, cell, ue, slot). */
+__global__ void rs_synth_arrivals_kernel(int* out, unsigned long long key, long long cell0, long long tti0, int n_ttis,
+                                         const DevCfg d, const int* spec) {
+  const int nb = d.nb, U = d.U, S = d.S;
+  const size_t total = (size_t)n_ttis * d.n_cells * U * nb;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+    const unsigned long long slot = i % nb;
+    size_t r = i / nb;
+    const int u = (int)(r % U); r /= U;
+    const int b = (int)(r % d.n_cells);
+    const unsigned long long cell = cell0 + b;
+    const unsigned long long tti = tti0 + (long long)(r / d.n_cells);
+    const int pf = d.cell_profile ? d.cell_profile[b] : 0;
+    const int* sp = spec + 2 * ((size_t)pf * S + d.ue_to_slice[(size_t)pf * U + u]);
+    const unsigned long long ue = (unsigned long long)u;
+    const unsigned long long ctr = ((tti << 40) ^ (cell << 20) ^ (ue << 8) ^ slot) ^ ((ue >> 12) * 0xD6E8FEB86659FD93ull);
+    const unsigned draw16 = (unsigned)(splitmix64(ctr ^ key) >> 48);
+    const int q = sp[1];
+    out[i] = sp[0] * ((q >> 16) + (draw16 < (unsigned)(q & 0xffff) ? 1 : 0));
+  }
+}
+
+/* rs_get_buffers: the arrival time of every bearer's head record (0 when it holds none) */
+__global__ void rs_buf_heads_kernel(const BufMeta* meta, const double* tm, int K, size_t n, double* out) {
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
+    out[i] = meta[i].n > 0 ? tm[i * K + meta[i].head] : 0.0;
 }
 
 /* ---- per-slice totals: uint64 [P][4][S] += over cells (integers: order-independent) ----------- */

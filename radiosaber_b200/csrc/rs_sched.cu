@@ -261,6 +261,19 @@ struct rs_handle {
   const int32_t* q_next = nullptr;
   const double* hol_next = nullptr;
   DevBuf<unsigned char> holmul;
+  /* per-bearer FIFOs (rs_enable_buffers): buf_k records per bearer, 0 = off */
+  int buf_k = 0;
+  DevBuf<rs::BufMeta> buf_meta;
+  DevBuf<double> buf_time;
+  DevBuf<int> buf_bytes;
+  std::vector<unsigned char> buf_backlogged;   /* [B][U][nb], what rs_reset_state restores */
+  double last_now = -HUGE_VAL;                 /* `now` of the last TTI run on the buffers */
+  bool traffic_set = false;                    /* rs_set_traffic for the next run call, consumed by it */
+  rs_traffic traffic{};
+  DevBuf<int> shown_q;                         /* rs_run_device without queue_out / hol_out: what the TTIs show */
+  DevBuf<double> shown_hol;
+  DevBuf<int> synth_spec;                      /* rs_synth_arrivals' [P][S][2] */
+  DevBuf<unsigned char> buf_scratch;           /* rs_get_buffers */
   DevBuf<int> tbs1;
   DevBuf<short> vogel_tab;
   DevBuf<unsigned long long> stats;
@@ -273,7 +286,7 @@ struct rs_handle {
     DevBuf<uint8_t> cqi, active, mcs, final_cqi;
     DevBuf<int> rand2, tbs_bits, slice_target, slice_quota, nvs_slice;
     DevBuf<short> rbg_to_ue, alloc_ue, alloc_rbg;
-    DevBuf<int> alloc_n, queue;
+    DevBuf<int> alloc_n, queue, arrivals;
     DevBuf<double> hol;
     cudaEvent_t in_done = nullptr, k_done = nullptr, out_done = nullptr;
     cudaEvent_t k_done_x[3] = {};   /* kernel-done events of parts 1.. */
@@ -396,13 +409,14 @@ int upload(DevBuf<T>& b, const std::vector<T>& v) {
 }
 
 int alloc_slot(rs_handle* h, rs_handle::Slot& s, int T, const rs_outputs* out, bool want_active, bool want_cqi,
-               bool want_queue, bool want_hol) {
+               bool want_queue, bool want_hol, bool want_arrivals) {
   const size_t B = h->B, U = h->d.U, S = h->d.S, G = h->d.G, C = h->cqi_cols;
   if (want_cqi) CU(s.cqi.alloc((size_t)T * B * U * C));
   CU(s.rand2.alloc((size_t)T * B * std::max(h->d.rand_stride, 1)));
   if (want_active) CU(s.active.alloc((size_t)T * B * U));
   if (want_queue) CU(s.queue.alloc((size_t)T * B * U * h->d.nb));
   if (want_hol) CU(s.hol.alloc((size_t)T * B * U * h->d.nb));
+  if (want_arrivals) CU(s.arrivals.alloc((size_t)T * B * U * h->d.nb));
   if (out) {
     if (out->rbg_to_ue) CU(s.rbg_to_ue.alloc((size_t)T * B * G));
     if (out->tbs_bits) CU(s.tbs_bits.alloc((size_t)T * B * U));
@@ -448,6 +462,50 @@ int check_shared_fields(const rs_config* c, int P) {
   return RS_OK;
 }
 
+/* Every FIFO empty, the backlogged bearers flagged (n = -1), counters 0 and no `now` seen yet.  The caller has waited
+ * for the handle's work. */
+int buf_empty(rs_handle* h) {
+  h->last_now = -HUGE_VAL;
+  if (h->buf_k == 0) return RS_OK;
+  std::vector<rs::BufMeta> m(h->buf_backlogged.size());
+  for (size_t i = 0; i < m.size(); ++i) m[i] = rs::BufMeta{0, 0, 0, h->buf_backlogged[i] ? -1 : 0};
+  CU(cudaMemcpy(h->buf_meta.p, m.data(), m.size() * sizeof(rs::BufMeta), cudaMemcpyHostToDevice));
+  return RS_OK;
+}
+
+/* A buffered handle's traffic for a call of n TTIs (rs_set_traffic), consumed by the call; the times are checked here,
+ * before anything is enqueued. */
+int take_traffic(rs_handle* h, int n, rs_traffic* tr) {
+  const bool set = h->traffic_set;
+  *tr = h->traffic;
+  h->traffic_set = false;
+  if (h->buf_k == 0) return RS_OK;
+  if (!set) return fail(RS_ERR_ARG, "buffered handle: every run call needs rs_set_traffic");
+  if (n > 0 && (!tr->arrivals || !tr->now || !tr->arrival_time))
+    return fail(RS_ERR_ARG, "rs_set_traffic: arrivals, now and arrival_time are required");
+  double prev = h->last_now;
+  for (int t = 0; t < n; ++t) {
+    if (!(tr->now[t] >= prev))
+      return fail(RS_ERR_ARG, "rs_set_traffic: now[%d] = %.17g is before the previous TTI's %.17g", t, tr->now[t], prev);
+    if (!(tr->arrival_time[t] <= tr->now[t]))
+      return fail(RS_ERR_ARG, "rs_set_traffic: arrival_time[%d] = %.17g is after now[%d] = %.17g", t, tr->arrival_time[t], t,
+                  tr->now[t]);
+    prev = tr->now[t];
+  }
+  return RS_OK;
+}
+/* the FIFOs and the times of TTIs [t0, t0 + T) of a buffered call (the caller points a->arrivals at the launch's rows) */
+void fill_buffers(const rs_handle* h, rs::RunArgs* a, const rs_traffic& tr, int t0, int T) {
+  a->buf_k = h->buf_k;
+  a->buf_meta = h->buf_meta.p;
+  a->buf_time = h->buf_time.p;
+  a->buf_bytes = h->buf_bytes.p;
+  for (int t = 0; t < T; ++t) {
+    a->now[t] = tr.now[t0 + t];
+    a->arr_time[t] = tr.arrival_time[t0 + t];
+  }
+}
+
 bool wants(const rs_handle* h, int which) { /* outputs that exist for this scheduler id */
   const int a = h->d.algo;
   if (which == 0) return is_transport(a);   /* slice_target / slice_quota */
@@ -476,7 +534,7 @@ void rs_destroy(rs_handle* h) {
     s.cqi.release(); s.active.release(); s.mcs.release(); s.final_cqi.release(); s.rand2.release();
     s.tbs_bits.release(); s.slice_target.release(); s.slice_quota.release(); s.nvs_slice.release();
     s.rbg_to_ue.release(); s.alloc_ue.release(); s.alloc_rbg.release(); s.alloc_n.release();
-    s.queue.release(); s.hol.release();
+    s.queue.release(); s.hol.release(); s.arrivals.release();
     if (s.in_done) cudaEventDestroy(s.in_done);
     if (s.k_done) cudaEventDestroy(s.k_done);
     for (auto e : s.k_done_x) if (e) cudaEventDestroy(e);
@@ -492,6 +550,8 @@ void rs_destroy(rs_handle* h) {
   h->mb_dev.release();
   h->trace_tab.release(); h->ue_trace_off.release();
   h->holmul.release(); h->tbs1.release(); h->vogel_tab.release();
+  h->buf_meta.release(); h->buf_time.release(); h->buf_bytes.release(); h->shown_q.release(); h->shown_hol.release();
+  h->synth_spec.release(); h->buf_scratch.release();
   if (h->own_stream) cudaStreamDestroy(h->own_stream);
   if (h->copy_in) cudaStreamDestroy(h->copy_in);
   if (h->copy_out) cudaStreamDestroy(h->copy_out);
@@ -862,7 +922,7 @@ int rs_reset_state(rs_handle* h) {
   CU(cudaMemset(h->cum_rbs.p, 0, BU * 8));
   CU(cudaMemset(h->offset.p, 0, BS * 8));
   CU(cudaMemset(h->ewma.p, 0, BS * 8));
-  return RS_OK;
+  return buf_empty(h);
 }
 
 int rs_set_state(rs_handle* h, const double* avg_rate, const int32_t* tx_bytes, const uint64_t* cum_bytes,
@@ -971,17 +1031,28 @@ int run_device_impl(rs_handle* h, int32_t n_ttis, const uint8_t* d_cqi, int64_t 
   const double* d_hol = h->hol_next;
   h->q_next = nullptr;
   h->hol_next = nullptr;
+  rs_traffic tr;
+  if (const int rc = take_traffic(h, n_ttis, &tr); rc != RS_OK) return rc;
+  const bool buffered = h->buf_k > 0;
   if ((!d_cqi && !trace_row) || !dt || n_ttis < 0 || cqi_refresh < 1) return fail(RS_ERR_ARG, "rs_run_device: bad argument");
   if (h->d.rand_stride > 0 && !d_rand2) return fail(RS_ERR_ARG, "ids 8/9/11 need the rand() draws");
   if (!trace_row && (((uintptr_t)d_cqi & 3) || (cqi_tti_stride & 3))) return fail(RS_ERR_ARG, "cqi must be 4-byte aligned");
   if (trace_row && !h->trace_tab.p) return fail(RS_ERR_ARG, "no traces loaded: call rs_set_traces first");
-  if (h->d.nb == 2 && !d_queue) return fail(RS_ERR_ARG, "two bearers per UE: every run call needs rs_set_queues");
+  if (h->d.nb == 2 && !d_queue && !buffered) return fail(RS_ERR_ARG, "two bearers per UE: every run call needs rs_set_queues");
   if (n_ttis == 0) return RS_OK;
   CU(cudaSetDevice(h->device));
   if (trace_row) { const int rc = check_trace_rows(h, trace_row, n_ttis); if (rc != RS_OK) return rc; }
   if (ttis_per_launch <= 0) ttis_per_launch = 16;
   ttis_per_launch = std::min<int>(ttis_per_launch, rs::kMaxTtisPerLaunch);
   const size_t B = h->B, U = h->d.U;
+  /* buffered: the kernels write the queue / HoL each TTI shows into queue_out / hol_out, or into one launch's worth of
+   * scratch that every launch of the call reuses (launches of one part run in order; parts own disjoint cells) */
+  size_t q_tti = B * U * h->d.nb, h_tti = q_tti;
+  if (buffered) {
+    const size_t per_launch = (size_t)std::min(ttis_per_launch, n_ttis) * B * U * h->d.nb;
+    if (tr.queue_out) d_queue = tr.queue_out; else { CU(h->shown_q.alloc(per_launch)); d_queue = h->shown_q.p; q_tti = 0; }
+    if (tr.hol_out) d_hol = tr.hol_out; else { CU(h->shown_hol.alloc(per_launch)); d_hol = h->shown_hol.p; h_tti = 0; }
+  }
   /* more than one launch in this call and a big batch: the two halves of the batch go down two streams (forked
    * here, joined at the end of the call), so the tail of one launch overlaps the head of the next */
   const bool split = h->parts > 1 && n_ttis > ttis_per_launch;
@@ -1001,8 +1072,12 @@ int run_device_impl(rs_handle* h, int32_t n_ttis, const uint8_t* d_cqi, int64_t 
     a.active = d_active ? d_active + (size_t)t0 * active_tti_stride : nullptr;
     a.active_tti_stride = active_tti_stride;
     fill_scalars(h, &a, dt + t0, trace_row ? trace_row + t0 : nullptr, a.T);
-    a.queue = d_queue ? d_queue + (size_t)t0 * B * U * h->d.nb : nullptr;
-    a.hol = d_hol ? d_hol + (size_t)t0 * B * U * h->d.nb : nullptr;
+    a.queue = d_queue ? d_queue + (size_t)t0 * q_tti : nullptr;
+    a.hol = d_hol ? d_hol + (size_t)t0 * h_tti : nullptr;
+    if (buffered) {
+      a.arrivals = tr.arrivals + (size_t)t0 * B * U * h->d.nb;
+      fill_buffers(h, &a, tr, t0, a.T);
+    }
     a.stage = h->stage_ok && (trace_row || ((((uintptr_t)d_cqi) & 15) == 0 && (cqi_tti_stride & 15) == 0)) ? 1 : 0;
     point_outputs(h, &a, d_out, (size_t)t0);
     int rc = launch_ttis(h, a, trace_row != nullptr, nullptr, split ? 0 : -1);
@@ -1013,6 +1088,7 @@ int run_device_impl(rs_handle* h, int32_t n_ttis, const uint8_t* d_cqi, int64_t 
     CU(cudaEventRecord(h->join_evs[q - 1], h->xs[q - 1]));
     CU(cudaStreamWaitEvent(h->stream, h->join_evs[q - 1], 0));
   }
+  if (buffered) h->last_now = tr.now[n_ttis - 1];
   return RS_OK;
 }
 
@@ -1030,10 +1106,13 @@ int run_host_impl(rs_handle* h, int32_t n_ttis, const uint8_t* cqi, int32_t cqi_
   h->q_next = nullptr;
   h->hol_next = nullptr;
   if (ticket) *ticket = -1;
+  rs_traffic tr;
+  if (const int rc = take_traffic(h, n_ttis, &tr); rc != RS_OK) return rc;
+  const bool buffered = h->buf_k > 0;   /* the slot's queue / hol arrays are written by the kernel, not copied in */
   if ((!cqi && !trace_row) || !dt || n_ttis < 0 || cqi_refresh < 1) return fail(RS_ERR_ARG, "rs_run_host: bad argument");
   if (h->d.rand_stride > 0 && !rand2) return fail(RS_ERR_ARG, "ids 8/9/11 need the rand() draws");
   if (trace_row && !h->trace_tab.p) return fail(RS_ERR_ARG, "no traces loaded: call rs_set_traces first");
-  if (h->d.nb == 2 && !queue) return fail(RS_ERR_ARG, "two bearers per UE: every run call needs rs_set_queues");
+  if (h->d.nb == 2 && !queue && !buffered) return fail(RS_ERR_ARG, "two bearers per UE: every run call needs rs_set_queues");
   CU(cudaSetDevice(h->device));
   if (trace_row) { const int rc = check_trace_rows(h, trace_row, n_ttis); if (rc != RS_OK) return rc; }
   if (ttis_per_launch <= 0) ttis_per_launch = trace_row ? 16 : 8;
@@ -1048,7 +1127,8 @@ int run_host_impl(rs_handle* h, int32_t n_ttis, const uint8_t* cqi, int32_t cqi_
     for (int q = 1; q < P; ++q) CU(cudaStreamWaitEvent(h->xs[q - 1], h->fork_ev, 0));
   }
   for (auto& s : h->slot) {
-    const int rc = alloc_slot(h, s, TC, out, active != nullptr, !trace_row && !slabs, queue != nullptr, hol != nullptr);
+    const int rc = alloc_slot(h, s, TC, out, active != nullptr, !trace_row && !slabs, queue != nullptr || buffered,
+                              hol != nullptr || buffered, buffered);
     if (rc != RS_OK) { drain(h); return rc; }
   }
   if (slabs)
@@ -1096,6 +1176,7 @@ int run_host_impl(rs_handle* h, int32_t n_ttis, const uint8_t* cqi, int32_t cqi_
     if (active) CU_DRAIN(cudaMemcpyAsync(s.active.p, active + (size_t)t0 * B * U, (size_t)T * B * U, cudaMemcpyHostToDevice, h->copy_in));
     if (queue) CU_DRAIN(cudaMemcpyAsync(s.queue.p, queue + (size_t)t0 * B * U * NB, (size_t)T * B * U * NB * 4, cudaMemcpyHostToDevice, h->copy_in));
     if (hol) CU_DRAIN(cudaMemcpyAsync(s.hol.p, hol + (size_t)t0 * B * U * NB, (size_t)T * B * U * NB * 8, cudaMemcpyHostToDevice, h->copy_in));
+    if (buffered) CU_DRAIN(cudaMemcpyAsync(s.arrivals.p, tr.arrivals + (size_t)t0 * B * U * NB, (size_t)T * B * U * NB * 4, cudaMemcpyHostToDevice, h->copy_in));
     CU_DRAIN(cudaEventRecord(s.in_done, h->copy_in));
     /* kernel(s): inputs in, and the slot's previous outputs drained; a big batch runs as two half-batches, each half
      * chained on its own stream from chunk to chunk (the copies wait for both) */
@@ -1112,8 +1193,12 @@ int run_host_impl(rs_handle* h, int32_t n_ttis, const uint8_t* cqi, int32_t cqi_
     a.rand2 = (rand2 && RS) ? s.rand2.p : nullptr;
     a.active = active ? s.active.p : nullptr; a.active_tti_stride = (long long)(B * U);
     fill_scalars(h, &a, dt + t0, trace_row ? trace_row + t0 : nullptr, T);
-    a.queue = queue ? s.queue.p : nullptr;
-    a.hol = hol ? s.hol.p : nullptr;
+    a.queue = (queue || buffered) ? s.queue.p : nullptr;
+    a.hol = (hol || buffered) ? s.hol.p : nullptr;
+    if (buffered) {
+      a.arrivals = s.arrivals.p;
+      fill_buffers(h, &a, tr, t0, T);
+    }
     a.stage = h->stage_ok ? 1 : 0;   /* slot buffers come from cudaMalloc; B*U*C is a multiple of 16 when stage_ok */
     rs_outputs so{};
     if (out) {
@@ -1155,6 +1240,8 @@ int run_host_impl(rs_handle* h, int32_t n_ttis, const uint8_t* cqi, int32_t cqi_
       if (a.alloc_ue) CU_DRAIN(cudaMemcpyAsync(out->alloc_ue + (size_t)t0 * B * NL, s.alloc_ue.p, (size_t)T * B * NL * 2, cudaMemcpyDeviceToHost, h->copy_out));
       if (a.alloc_rbg) CU_DRAIN(cudaMemcpyAsync(out->alloc_rbg + (size_t)t0 * B * NL, s.alloc_rbg.p, (size_t)T * B * NL * 2, cudaMemcpyDeviceToHost, h->copy_out));
     }
+    if (tr.queue_out) CU_DRAIN(cudaMemcpyAsync(tr.queue_out + (size_t)t0 * B * U * NB, s.queue.p, (size_t)T * B * U * NB * 4, cudaMemcpyDeviceToHost, h->copy_out));
+    if (tr.hol_out) CU_DRAIN(cudaMemcpyAsync(tr.hol_out + (size_t)t0 * B * U * NB, s.hol.p, (size_t)T * B * U * NB * 8, cudaMemcpyDeviceToHost, h->copy_out));
     CU_DRAIN(cudaEventRecord(s.out_done, h->copy_out));
     s.out_rec = true;
     h->chunk_seq++;
@@ -1163,6 +1250,7 @@ int run_host_impl(rs_handle* h, int32_t n_ttis, const uint8_t* cqi, int32_t cqi_
     CU_DRAIN(cudaEventRecord(h->join_evs[q - 1], h->xs[q - 1]));
     CU_DRAIN(cudaStreamWaitEvent(h->stream, h->join_evs[q - 1], 0));
   }
+  if (buffered && n_ttis > 0) h->last_now = tr.now[n_ttis - 1];
   /* copy_out is behind every kernel of the call (it waited on each k_done), and every kernel is behind its inputs */
   const int64_t tk = h->calls++;
   CU_DRAIN(cudaEventRecord(h->call_done[tk % rs_handle::kTickets], h->copy_out));
@@ -1529,8 +1617,104 @@ int rs_log_get_counters(rs_log* lg, uint64_t* cum_bytes, uint64_t* cum_rbs) {
 int rs_set_queues(rs_handle* h, const int32_t* queue_bytes, const double* hol_delay) {
   if (!h) return fail(RS_ERR_ARG, "null handle");
   if (hol_delay && !queue_bytes) return fail(RS_ERR_ARG, "rs_set_queues: head-of-line delays without queue sizes");
+  if (h->buf_k > 0 && queue_bytes)
+    return fail(RS_ERR_ARG, "rs_set_queues: the handle keeps its own buffers (rs_enable_buffers); give it rs_set_traffic");
   h->q_next = queue_bytes;
   h->hol_next = hol_delay;
+  return RS_OK;
+}
+
+int rs_enable_buffers(rs_handle* h, int32_t max_records, const uint8_t* backlogged) {
+  if (!h) return fail(RS_ERR_ARG, "null handle");
+  if (max_records < 0 || max_records > RS_MAX_BUFFER_RECORDS)
+    return fail(RS_ERR_ARG, "rs_enable_buffers: max_records %d outside 0..%d", max_records, RS_MAX_BUFFER_RECORDS);
+  const int rc = rs_sync(h);   /* the launches in flight read the old buffers */
+  if (rc != RS_OK) return rc;
+  h->q_next = nullptr;
+  h->hol_next = nullptr;
+  h->traffic_set = false;
+  h->buf_k = 0;
+  h->buf_meta.release(); h->buf_time.release(); h->buf_bytes.release(); h->shown_q.release(); h->shown_hol.release();
+  h->buf_backlogged.clear();
+  h->last_now = -HUGE_VAL;
+  if (max_records == 0) return RS_OK;
+  const size_t n = (size_t)h->B * h->d.U * h->d.nb;
+  CU(h->buf_meta.alloc(n));
+  cudaError_t e = h->buf_time.alloc(n * (size_t)max_records);
+  if (e == cudaSuccess) e = h->buf_bytes.alloc(n * (size_t)max_records);
+  if (e != cudaSuccess) {
+    h->buf_meta.release(); h->buf_time.release(); h->buf_bytes.release();
+    return fail(RS_ERR_CUDA, "rs_enable_buffers: cudaMalloc of %zu bearers x %d records: %s", n, max_records, cudaGetErrorString(e));
+  }
+  if (backlogged) h->buf_backlogged.assign(backlogged, backlogged + n); else h->buf_backlogged.assign(n, 0);
+  h->buf_k = max_records;
+  return buf_empty(h);
+}
+
+int rs_set_traffic(rs_handle* h, const rs_traffic* traffic) {
+  if (!h || !traffic) return fail(RS_ERR_ARG, "rs_set_traffic: bad argument");
+  if (h->buf_k == 0) return fail(RS_ERR_ARG, "rs_set_traffic: the handle has no buffers (rs_enable_buffers)");
+  h->traffic = *traffic;
+  h->traffic_set = true;
+  return RS_OK;
+}
+
+int rs_get_buffers(rs_handle* h, int64_t* queued, int32_t* n_records, double* head_time, uint64_t* dropped) {
+  if (!h) return fail(RS_ERR_ARG, "null handle");
+  if (h->buf_k == 0) return fail(RS_ERR_ARG, "rs_get_buffers: the handle has no buffers (rs_enable_buffers)");
+  const int rc = rs_sync(h);
+  if (rc != RS_OK) return rc;
+  const size_t n = h->buf_backlogged.size();
+  std::vector<rs::BufMeta> m(n);
+  CU(cudaMemcpy(m.data(), h->buf_meta.p, n * sizeof(rs::BufMeta), cudaMemcpyDeviceToHost));
+  for (size_t i = 0; i < n; ++i) {
+    const bool fifo = m[i].n >= 0;
+    if (queued) queued[i] = fifo ? m[i].queued : 0;
+    if (n_records) n_records[i] = fifo ? m[i].n : 0;
+    if (dropped) dropped[i] = fifo ? m[i].dropped : 0;
+  }
+  if (head_time) {
+    CU(h->buf_scratch.alloc(n * sizeof(double)));
+    const int blocks = (int)std::min<size_t>((n + 255) / 256, 148 * 4);
+    rs::rs_buf_heads_kernel<<<blocks, 256, 0, h->stream>>>(h->buf_meta.p, h->buf_time.p, h->buf_k, n, (double*)h->buf_scratch.p);
+    CU(cudaGetLastError());
+    h->launches++;
+    CU(cudaMemcpyAsync(head_time, h->buf_scratch.p, n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+  }
+  return RS_OK;
+}
+
+int rs_synth_arrivals(rs_handle* h, uint64_t seed, int64_t cell0, int64_t tti0, int32_t n_ttis, const int32_t* pkt_bytes,
+                      const int32_t* pkts_q16, int32_t* d_out) {
+  if (!h || !pkt_bytes || !pkts_q16 || !d_out || n_ttis < 0) return fail(RS_ERR_ARG, "rs_synth_arrivals: bad argument");
+  const int P = h->P, S = h->d.S;
+  std::vector<int> spec((size_t)2 * P * S);
+  for (int i = 0; i < P * S; ++i) {
+    if (pkt_bytes[i] < 0 || pkts_q16[i] < 0)
+      return fail(RS_ERR_ARG, "rs_synth_arrivals: profile %d slice %d: negative packet size or rate", i / S, i % S);
+    if ((long long)pkt_bytes[i] * ((pkts_q16[i] >> 16) + 1) > 0x7fffffffLL)
+      return fail(RS_ERR_ARG, "rs_synth_arrivals: profile %d slice %d: a TTI's bytes overflow int32", i / S, i % S);
+    spec[2 * i] = pkt_bytes[i];
+    spec[2 * i + 1] = pkts_q16[i];
+  }
+  CU(cudaSetDevice(h->device));
+  CU(h->synth_spec.alloc(spec.size()));
+  /* pageable source: the copy is staged before the call returns; ordered with earlier kernels that read the table */
+  CU(cudaMemcpyAsync(h->synth_spec.p, spec.data(), spec.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+  auto sm64 = [](unsigned long long x) {
+    unsigned long long z = x + 0x9E3779B97F4A7C15ull;
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+  };
+  const unsigned long long key = sm64((seed & 0xFFFFFFFFull) | (0x41525200ull << 32));   /* "ARR\0" */
+  const size_t total_n = (size_t)n_ttis * h->B * h->d.U * h->d.nb;
+  if (total_n == 0) return RS_OK;
+  const int blocks = (int)std::min<size_t>((total_n + 255) / 256, 148 * 16);
+  rs::rs_synth_arrivals_kernel<<<blocks, 256, 0, h->stream>>>(d_out, key, cell0, tti0, n_ttis, h->d, h->synth_spec.p);
+  CU(cudaGetLastError());
+  h->launches++;
   return RS_OK;
 }
 
@@ -1546,6 +1730,9 @@ int rs_step_cell(rs_handle* h, const rs_cell_io* io) {
   if (!h || !io || !io->cqi) return fail(RS_ERR_ARG, "rs_step_cell: bad argument");
   h->q_next = nullptr;
   h->hol_next = nullptr;
+  h->traffic_set = false;
+  if (h->buf_k > 0)
+    return fail(RS_ERR_ARG, "rs_step_cell: the handle keeps its own buffers; inside a simulator the simulator owns the queues");
   if (io->hol_delay && !io->queue_bytes) return fail(RS_ERR_ARG, "rs_step_cell: head-of-line delays without queue sizes");
   if (h->d.rand_stride > 0 && !io->rand2) return fail(RS_ERR_ARG, "ids 8/9/11 need the rand() draws");
   if (h->d.nb == 2 && !io->queue_bytes) return fail(RS_ERR_ARG, "two bearers per UE: the call needs queue_bytes");

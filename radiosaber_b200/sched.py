@@ -37,6 +37,7 @@ ABI_SYMBOLS = (
     "rs_get_stream", "rs_host_alloc", "rs_host_free", "rs_step_cell", "rs_run_host_async", "rs_run_traces_host_async",
     "rs_wait", "rs_dims", "rs_fixed_shape", "rs_direct_metric",
     "rs_create_profiles", "rs_set_cell_profiles", "rs_n_profiles", "rs_set_grant_list_len", "rs_grant_list_len",
+    "rs_enable_buffers", "rs_set_traffic", "rs_get_buffers", "rs_synth_arrivals",
 )
 
 
@@ -67,6 +68,11 @@ class _CellIo(C.Structure):
         ("active", C.c_void_p), ("queue_bytes", C.c_void_p), ("hol_delay", C.c_void_p), ("dt", C.c_double),
         ("out", _Out),
     ]
+
+
+class _Traffic(C.Structure):
+    _fields_ = [("arrivals", C.c_void_p), ("now", C.c_void_p), ("arrival_time", C.c_void_p), ("queue_out", C.c_void_p),
+                ("hol_out", C.c_void_p)]
 
 
 def lib():
@@ -156,6 +162,11 @@ def lib():
         L.rs_fixed_shape.restype = C.c_int32
         L.rs_direct_metric.argtypes = [C.c_void_p]
         L.rs_direct_metric.restype = C.c_int32
+        L.rs_enable_buffers.argtypes = [C.c_void_p, C.c_int32, C.c_void_p]
+        L.rs_set_traffic.argtypes = [C.c_void_p, C.POINTER(_Traffic)]
+        L.rs_get_buffers.argtypes = [C.c_void_p] + [C.c_void_p] * 4
+        L.rs_synth_arrivals.argtypes = [C.c_void_p, C.c_uint64, C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p,
+                                        C.c_void_p]
         _lib = L
     return _lib
 
@@ -358,9 +369,66 @@ class Scheduler:
         _check(lib().rs_set_queues(self._h, _ptr(q), _ptr(h)))
         return q, h
 
-    def step(self, cqi, rand2=None, dt=0.001, active=None, want_aux=False, queue=None, hol=None):
+    # ---- per-bearer buffers on the device (closed-loop queues, rs_enable_buffers) -------------------
+    def enable_buffers(self, max_records, backlogged=None):
+        """Keep a byte FIFO of at most max_records records per bearer on the device (0 = off); backlogged: bool
+        [B][U] ([B][U][2] with two bearers) of bearers without a FIFO (the infinite buffer).  Empties every FIFO."""
+        bl = None if backlogged is None else np.ascontiguousarray(np.asarray(backlogged).reshape(self._per_bearer((self.B,))),
+                                                                  dtype=np.uint8)
+        _check(lib().rs_enable_buffers(self._h, int(max_records), _ptr(bl)))
+
+    def get_buffers(self):
+        """{queued int64, n_records int32, head_time float64, dropped uint64}, each [B][U] ([B][U][2])."""
+        shape = self._per_bearer((self.B,))
+        st = {"queued": np.empty(shape, np.int64), "n_records": np.empty(shape, np.int32),
+              "head_time": np.empty(shape, np.float64), "dropped": np.empty(shape, np.uint64)}
+        _check(lib().rs_get_buffers(self._h, *[_ptr(st[k]) for k in ("queued", "n_records", "head_time", "dropped")]))
+        return st
+
+    def synth_arrivals(self, seed, cell0, tti0, n_ttis, pkt_bytes, pkts_q16, d_out):
+        """rs_synth_arrivals: int32 [n_ttis][B][U][nb] into device memory; pkt_bytes / pkts_q16: int [P][S] (packet
+        size, packets per TTI in 16.16 fixed point) per slice of each profile.  Twin of workload.synth_arrivals."""
+        pb = np.ascontiguousarray(np.asarray(pkt_bytes).reshape(self.n_profiles, self.S), dtype=np.int32)
+        pq = np.ascontiguousarray(np.asarray(pkts_q16).reshape(self.n_profiles, self.S), dtype=np.int32)
+        _check(lib().rs_synth_arrivals(self._h, int(seed), int(cell0), int(tti0), int(n_ttis), _ptr(pb), _ptr(pq),
+                                       C.c_void_p(d_out)))
+
+    def _per_bearer(self, lead):
+        return lead + ((self.U,) if self.nb == 1 else (self.U, 2))
+
+    def _traffic(self, arrivals, now, arrival_time, T, out):
+        """Hand the next HOST run call of T TTIs its traffic (rs_set_traffic); the queue sizes and delays the TTIs show go
+        to out["queue_out"] / out["hol_out"].  Returns the arrays to keep alive."""
+        if arrivals is None:
+            return None
+        lead = (T, self.B) if T is not None else (self.B,)
+        n = 1 if T is None else T
+        a = np.ascontiguousarray(arrivals, dtype=np.int32).reshape(self._per_bearer(lead))
+        nw = np.ascontiguousarray(np.asarray(now, dtype=np.float64).reshape(n))
+        at = nw if arrival_time is None else np.ascontiguousarray(np.asarray(arrival_time, dtype=np.float64).reshape(n))
+        out["queue_out"] = np.empty(a.shape, np.int32)
+        out["hol_out"] = np.empty(a.shape, np.float64)
+        tr = _Traffic(_ptr(a), _ptr(nw), _ptr(at), _ptr(out["queue_out"]), _ptr(out["hol_out"]))
+        _check(lib().rs_set_traffic(self._h, C.byref(tr)))
+        return a, nw, at
+
+    def _device_traffic(self, n_ttis, d_arrivals, now, arrival_time, d_queue_out, d_hol_out):
+        """Hand the next DEVICE run call its traffic: arrivals / outputs are device pointers, now / arrival_time host
+        arrays [T].  Returns the arrays to keep alive."""
+        if not d_arrivals:
+            return None
+        nw = np.ascontiguousarray(np.asarray(now, dtype=np.float64).reshape(-1)[:n_ttis])
+        at = nw if arrival_time is None else np.ascontiguousarray(np.asarray(arrival_time, dtype=np.float64).reshape(-1)[:n_ttis])
+        tr = _Traffic(C.c_void_p(d_arrivals), _ptr(nw), _ptr(at), C.c_void_p(d_queue_out or None), C.c_void_p(d_hol_out or None))
+        _check(lib().rs_set_traffic(self._h, C.byref(tr)))
+        return nw, at
+
+    def step(self, cqi, rand2=None, dt=0.001, active=None, want_aux=False, queue=None, hol=None, arrivals=None, now=None,
+             arrival_time=None):
         """One TTI for every cell. cqi: uint8 [B][U][G] (or [B][U][R]); rand2: int32 [B][2]; queue / hol: the
-        bearers' dataToTransmit (int32 [B][U]) and head-of-line delays (float64 [B][U]), see rs_set_queues."""
+        bearers' dataToTransmit (int32 [B][U]) and head-of-line delays (float64 [B][U]), see rs_set_queues.  A buffered
+        handle takes arrivals (int32 [B][U]), now and arrival_time (default now) instead, and returns the queue sizes and
+        delays the TTI showed as out["queue_out"] / out["hol_out"] (rs_set_traffic)."""
         B, U = self.B, self.U
         keep = self._queues(queue, hol, (B,))
         cqi = np.ascontiguousarray(cqi, dtype=np.uint8)
@@ -368,6 +436,7 @@ class Scheduler:
         rand2 = self._draws(rand2, (B,))
         act = None if active is None else np.ascontiguousarray(active, dtype=np.uint8).reshape(B, U)
         out, o = self._host_outputs(None, want_aux)
+        keep_tr = self._traffic(arrivals, now, arrival_time, None, out)
         _check(lib().rs_step(self._h, _ptr(cqi), _ptr(rand2), _ptr(act), float(dt), C.byref(o)))
         return out
 
@@ -389,10 +458,17 @@ class Scheduler:
         _check(lib().rs_step_cell(self._h, C.byref(io)))
         return out
 
-    def run_host_async(self, cqi, rand2, dt, out, o, ttis_per_launch=0, cqi_refresh=1):
+    def run_host_async(self, cqi, rand2, dt, out, o, ttis_per_launch=0, cqi_refresh=1, traffic=None):
         """rs_run_host_async on caller-owned arrays (kept alive and untouched until wait(ticket)); out / o come from
-        _host_outputs().  Returns the ticket."""
+        _host_outputs().  traffic: (arrivals, now, arrival_time) of a buffered handle, whose arrays the caller keeps alive
+        as well (the shown queues and delays land in out["queue_out"] / out["hol_out"]).  Returns the ticket."""
         T = int(dt.shape[0])
+        if traffic is not None:
+            a, nw, at = traffic
+            out["queue_out"] = np.empty(a.shape, np.int32)
+            out["hol_out"] = np.empty(a.shape, np.float64)
+            tr = _Traffic(_ptr(a), _ptr(nw), _ptr(at), _ptr(out["queue_out"]), _ptr(out["hol_out"]))
+            _check(lib().rs_set_traffic(self._h, C.byref(tr)))
         ticket = C.c_int64(-1)
         _check(lib().rs_run_host_async(self._h, T, _ptr(cqi), int(cqi_refresh), _ptr(rand2), None, _ptr(dt),
                                        C.byref(o), int(ttis_per_launch), C.byref(ticket)))
@@ -402,9 +478,9 @@ class Scheduler:
         _check(lib().rs_wait(self._h, int(ticket)))
 
     def run_host(self, cqi, rand2, dt, active=None, want_aux=False, ttis_per_launch=0, cqi_refresh=1, queue=None,
-                 hol=None):
+                 hol=None, arrivals=None, now=None, arrival_time=None):
         """T TTIs with host arrays [T][B][...] (cqi: one slab per cqi_refresh TTIs); copies overlap
-        the kernels."""
+        the kernels.  arrivals [T][B][U] / now [T] / arrival_time [T]: as step() for a buffered handle."""
         B, U = self.B, self.U
         dt = np.ascontiguousarray(dt, dtype=np.float64)
         T = int(dt.shape[0])
@@ -414,6 +490,7 @@ class Scheduler:
         act = None if active is None else np.ascontiguousarray(active, dtype=np.uint8).reshape(T, B, U)
         out, o = self._host_outputs(T, want_aux)
         keep = self._queues(queue, hol, (T, B))
+        keep_tr = self._traffic(arrivals, now, arrival_time, T, out)
         _check(lib().rs_run_host(self._h, T, _ptr(cqi), int(cqi_refresh), _ptr(rand2), _ptr(act), _ptr(dt),
                                  C.byref(o), int(ttis_per_launch)))
         return out
@@ -425,10 +502,14 @@ class Scheduler:
             _check(lib().rs_set_queues(self._h, C.c_void_p(d_queue or None), C.c_void_p(d_hol or None)))
 
     def run_device(self, n_ttis, d_cqi, cqi_tti_stride, d_rand2, dt, d_out=None, d_active=0,
-                   active_tti_stride=0, ttis_per_launch=0, cqi_refresh=1, d_queue=0, d_hol=0):
+                   active_tti_stride=0, ttis_per_launch=0, cqi_refresh=1, d_queue=0, d_hol=0, d_arrivals=0, now=None,
+                   arrival_time=None, d_queue_out=0, d_hol_out=0):
+        """d_arrivals / d_queue_out / d_hol_out: device pointers of a buffered handle's traffic ([T][B][U][nb]); now /
+        arrival_time host arrays [T] (rs_set_traffic)."""
         dt = np.ascontiguousarray(dt, dtype=np.float64)
         assert dt.shape[0] >= n_ttis
         self._device_queues(d_queue, d_hol)
+        keep_tr = self._device_traffic(n_ttis, d_arrivals, now, arrival_time, d_queue_out, d_hol_out)
         o = _Out(*[(d_out or {}).get(k) for k in ("rbg_to_ue", "tbs_bits", "mcs", "final_cqi", "slice_target",
                                                     "slice_quota", "nvs_slice", "alloc_n", "alloc_ue", "alloc_rbg")])
         _check(lib().rs_run_device(self._h, int(n_ttis), C.c_void_p(d_cqi), int(cqi_tti_stride), int(cqi_refresh),
@@ -446,9 +527,9 @@ class Scheduler:
         self.trace_rows = int(traces.shape[1])
 
     def run_traces_host(self, trace_row, rand2, dt, active=None, want_aux=False, ttis_per_launch=0, queue=None,
-                        hol=None):
+                        hol=None, arrivals=None, now=None, arrival_time=None):
         """T TTIs with the CQI replayed from the loaded traces; trace_row: int32 [T] (-1 = no report yet); queue / hol
-        as run_host."""
+        and arrivals / now / arrival_time as run_host."""
         B, U = self.B, self.U
         dt = np.ascontiguousarray(dt, dtype=np.float64)
         T = int(dt.shape[0])
@@ -458,16 +539,19 @@ class Scheduler:
         act = None if active is None else np.ascontiguousarray(active, dtype=np.uint8).reshape(T, B, U)
         out, o = self._host_outputs(T, want_aux)
         keep = self._queues(queue, hol, (T, B))
+        keep_tr = self._traffic(arrivals, now, arrival_time, T, out)
         _check(lib().rs_run_traces_host(self._h, T, _ptr(trace_row), _ptr(rand2), _ptr(act), _ptr(dt), C.byref(o),
                                         int(ttis_per_launch)))
         return out
 
     def run_traces_device(self, n_ttis, trace_row, d_rand2, dt, d_out=None, d_active=0, active_tti_stride=0,
-                          ttis_per_launch=0, d_queue=0, d_hol=0):
+                          ttis_per_launch=0, d_queue=0, d_hol=0, d_arrivals=0, now=None, arrival_time=None, d_queue_out=0,
+                          d_hol_out=0):
         dt = np.ascontiguousarray(dt, dtype=np.float64)
         trace_row = np.ascontiguousarray(trace_row, dtype=np.int32)
         assert dt.shape[0] >= n_ttis and trace_row.shape[0] >= n_ttis
         self._device_queues(d_queue, d_hol)
+        keep_tr = self._device_traffic(n_ttis, d_arrivals, now, arrival_time, d_queue_out, d_hol_out)
         o = _Out(*[(d_out or {}).get(k) for k in ("rbg_to_ue", "tbs_bits", "mcs", "final_cqi", "slice_target",
                                                     "slice_quota", "nvs_slice", "alloc_n", "alloc_ue", "alloc_rbg")])
         _check(lib().rs_run_traces_device(self._h, int(n_ttis), _ptr(trace_row), C.c_void_p(d_rand2 or None),

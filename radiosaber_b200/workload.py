@@ -122,3 +122,38 @@ def tti_clock(n_ttis: int, start: float = 0.1):
         last = t
         t = t + 0.001
     return now, dt
+
+
+DOMAIN_ARRIVALS = 0x41525200  # "ARR\0"
+
+
+def synth_arrivals(seed: int, cell0: int, n_cells: int, tti0: int, n_ttis: int, ue_to_slice, pkt_bytes, pkts_q16,
+                   n_bearers: int = 1, cell_profile=None) -> np.ndarray:
+    """int32 [n_ttis][n_cells][U] ([..][U][2] with two bearers): bytes arriving at each bearer per TTI, for the
+    device-kept buffers (``rs_enable_buffers``; ``rs_synth_arrivals`` is the device twin).
+
+    ue_to_slice [U] or [P][U], pkt_bytes / pkts_q16 [S] or [P][S] (one row per slice profile; cell b reads row
+    cell_profile[b], row 0 without profiles).  A bearer of slice s gets ``(q >> 16) + (draw16 < (q & 0xffff))``
+    packets of ``pkt_bytes[s]`` bytes with ``q = pkts_q16[s]`` (packets per TTI in 16.16 fixed point); draw16 is the
+    top 16 bits of one splitmix64 draw of a counter over (cell, tti, ue, slot) built like :func:`synth_cqi`'s.
+    Integers only, so the two twins agree bit for bit."""
+    u2s = np.atleast_2d(np.asarray(ue_to_slice, dtype=np.int64))
+    pb = np.atleast_2d(np.asarray(pkt_bytes, dtype=np.int64))
+    pq = np.atleast_2d(np.asarray(pkts_q16, dtype=np.int64))
+    U = u2s.shape[1]
+    nb = 2 if int(n_bearers) == 2 else 1
+    cp = np.zeros(n_cells, dtype=np.int64) if cell_profile is None else np.asarray(cell_profile, dtype=np.int64)
+    key = _key(seed, DOMAIN_ARRIVALS)
+    tti = np.arange(tti0, tti0 + n_ttis, dtype=np.uint64)[:, None, None, None]
+    cell = np.arange(cell0, cell0 + n_cells, dtype=np.uint64)[None, :, None, None]
+    ue = np.arange(U, dtype=np.uint64)[None, None, :, None]
+    slot = np.arange(nb, dtype=np.uint64)[None, None, None, :]
+    with np.errstate(over="ignore"):
+        ctr = ((tti << np.uint64(40)) ^ (cell << np.uint64(20)) ^ (ue << np.uint64(8)) ^ slot)
+        ctr = ctr ^ ((ue >> np.uint64(12)) * np.uint64(0xD6E8FEB86659FD93))
+        draw16 = (splitmix64(ctr ^ key) >> np.uint64(48)).astype(np.int64)
+    s = u2s[cp]                                            # [B][U]: each cell's slices
+    size = np.take_along_axis(pb[cp], s, axis=1)[None, :, :, None]
+    q = np.take_along_axis(pq[cp], s, axis=1)[None, :, :, None]
+    out = (size * ((q >> 16) + (draw16 < (q & 0xffff)))).astype(np.int32)
+    return out if nb == 2 else out[..., 0]
