@@ -250,6 +250,15 @@ int rs_set_traffic(rs_handle* h, const rs_traffic* traffic);
  * work in flight. */
 int rs_get_buffers(rs_handle* h, int64_t* queued, int32_t* n_records, double* head_time, uint64_t* dropped);
 
+/* Per-slice totals of the buffers, uint64 [P][3][S] = { sum queued bytes, sum dropped bytes, sum records held } over
+ * the bearers with a FIFO (both slots with two bearers per UE; backlogged bearers add 0).  Row p sums the cells of
+ * profile p with its ue_to_slice, as rs_stats_device does; integers, so any reduction order gives the same bits.
+ * rs_buffer_stats_device writes DEVICE memory (P x 3 x S uint64; feed it to an NCCL reduce, rs_reduce_buffer_stats);
+ * rs_get_buffer_stats copies to HOST.  Both are ordered after the handle's earlier work on its stream, like
+ * rs_stats_device.  RS_ERR_ARG on a handle without buffers. */
+int rs_buffer_stats_device(rs_handle* h, uint64_t* d_stats);
+int rs_get_buffer_stats(rs_handle* h, uint64_t* stats);
+
 /* Synthetic arrivals into DEVICE int32 [n_ttis][B][U][nb] (bit-identical twin of radiosaber_b200/workload.py
  * synth_arrivals): pkt_bytes and pkts_q16 are HOST int32 [P][S] (P = rs_n_profiles; cell b reads the row of its
  * profile).  A bearer of slice s gets (q >> 16) + (draw16 < (q & 0xffff)) packets of pkt_bytes[s] bytes per TTI with
@@ -258,6 +267,12 @@ int rs_get_buffers(rs_handle* h, int64_t* queued, int32_t* n_records, double* he
  * stream. */
 int rs_synth_arrivals(rs_handle* h, uint64_t seed, int64_t cell0, int64_t tti0, int32_t n_ttis, const int32_t* pkt_bytes,
                       const int32_t* pkts_q16, int32_t* d_out);
+/* One slice's arrival spec for rs_synth_arrivals from a packet size and a mean rate in packets per TTI, as a traffic
+ * file gives them (host only, no GPU needed; rs_batch and radiosaber_b200/sched.py load_traffic_config both use it).
+ * *pkts_q16 = pkts_per_tti * 65536 rounded to the nearest integer (halves away from zero).  RS_ERR_ARG, with the
+ * reason in rs_last_error, unless pkt_bytes is an integer 0..INT32_MAX, pkts_per_tti is finite and >= 0, a positive
+ * rate is at least 1/65536 packet per TTI, and a TTI's most bytes, pkt_bytes x ((q >> 16) + 1), fit int32. */
+int rs_arrival_spec(double pkt_bytes, double pkts_per_tti, int32_t* pkt_bytes_out, int32_t* pkts_q16);
 
 /* n_ttis consecutive TTIs with every input and output already in DEVICE memory.
  *   d_cqi   [ceil(T/cqi_refresh)][B][U][row]: TTI t reads slab t / cqi_refresh (the reference refreshes

@@ -2438,6 +2438,36 @@ __global__ void rs_stats_kernel(const DevCfg d, unsigned long long* stats, int n
   }
 }
 
+/* ---- per-slice buffer totals: uint64 [P][3][S] += { queued, dropped, records } over the bearers with a FIFO ---- */
+/* Same row and shared-memory rules as rs_stats_kernel; meta [B][U][nb] (BufMeta::n < 0: backlogged, adds nothing). */
+__global__ void rs_buffer_stats_kernel(const BufMeta* meta, const DevCfg d, unsigned long long* stats, int n_profiles,
+                                       int in_smem) {
+  extern __shared__ unsigned long long s_acc[];   /* [P][3][S] */
+  const int S = d.S;
+  unsigned long long* acc = in_smem ? s_acc : stats;
+  if (in_smem) {
+    for (int i = threadIdx.x; i < 3 * S * n_profiles; i += blockDim.x) s_acc[i] = 0;
+    __syncthreads();
+  }
+  const size_t total = (size_t)d.n_cells * d.U * d.nb;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+    const BufMeta m = meta[i];
+    if (m.n < 0) continue;   /* backlogged: no FIFO */
+    const size_t cu = i / d.nb;
+    const int pf = d.cell_profile ? d.cell_profile[cu / d.U] : 0;
+    const int s = d.ue_to_slice[(size_t)pf * d.U + cu % d.U];
+    unsigned long long* row = acc + (size_t)pf * 3 * S;
+    if (m.queued) atomicAdd(&row[0 * S + s], (unsigned long long)m.queued);
+    if (m.dropped) atomicAdd(&row[1 * S + s], m.dropped);
+    if (m.n) atomicAdd(&row[2 * S + s], (unsigned long long)m.n);
+  }
+  if (in_smem) {
+    __syncthreads();
+    for (int i = threadIdx.x; i < 3 * S * n_profiles; i += blockDim.x)
+      if (s_acc[i]) atomicAdd(&stats[i], s_acc[i]);
+  }
+}
+
 #endif  /* RS_CORE_ONLY */
 
 }  // namespace RS_NS

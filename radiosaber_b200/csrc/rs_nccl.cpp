@@ -1,6 +1,7 @@
-/* rs_nccl.cpp -- include/rs_sched_nccl.h: the end-of-run NCCL reduce of the per-slice totals (SURVEY 8e).
+/* rs_nccl.cpp -- include/rs_sched_nccl.h: the end-of-run NCCL reduce of the per-slice totals (SURVEY 8e), and
+ * include/rs_sched_nccl_buffers.h: the same for the per-slice buffer totals.
  * Uses only the public ABI of librs_sched.so plus NCCL and the CUDA runtime. */
-#include "../../include/rs_sched_nccl.h"
+#include "../../include/rs_sched_nccl_buffers.h"
 
 #include <cuda_runtime.h>
 #include <nccl.h>
@@ -28,6 +29,34 @@ int nfail(const char* what, const char* why) {
     cudaError_t e_ = (call);                                                \
     if (e_ != cudaSuccess) return nfail(#call, cudaGetErrorString(e_));     \
   } while (0)
+
+/* fill(h, d) writes this rank's uint64 [P][rows][S] totals to device memory; one ncclReduce(sum) on the handle's stream
+ * adds them up on the root, which copies them to stats_out. */
+int reduce_totals(rs_handle* h, void* nccl_comm, int32_t root, uint64_t* stats_out, int rows,
+                  int (*fill)(rs_handle*, uint64_t*), const char* name, const char* fill_name) {
+  if (!h || !nccl_comm) return nfail(name, "bad argument");
+  ncclComm_t comm = (ncclComm_t)nccl_comm;
+  int32_t S = 0, dev = 0;
+  if (rs_dims(h, nullptr, &S, nullptr, nullptr, &dev) != RS_OK || S < 1) return nfail("rs_dims", rs_last_error());
+  const size_t n = (size_t)rows * S * rs_n_profiles(h);
+  int rank = -1;
+  NC(ncclCommUserRank(comm, &rank));
+  CUR(cudaSetDevice(dev));
+  cudaStream_t st = (cudaStream_t)rs_get_stream(h);
+  uint64_t* d = nullptr;
+  CUR(cudaMalloc((void**)&d, sizeof(uint64_t) * n));
+  int rc = fill(h, d);
+  if (rc != RS_OK) { cudaFree(d); return nfail(fill_name, rs_last_error()); }
+  ncclResult_t r = ncclReduce(d, d, n, ncclUint64, ncclSum, root, comm, st);
+  cudaError_t e = cudaSuccess;
+  if (r == ncclSuccess && rank == root && stats_out)
+    e = cudaMemcpyAsync(stats_out, d, sizeof(uint64_t) * n, cudaMemcpyDeviceToHost, st);
+  if (r == ncclSuccess && e == cudaSuccess) e = cudaStreamSynchronize(st);
+  cudaFree(d);
+  if (r != ncclSuccess) return nfail("ncclReduce", ncclGetErrorString(r));
+  if (e != cudaSuccess) return nfail(name, cudaGetErrorString(e));
+  return RS_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -67,28 +96,12 @@ void rs_comm_destroy(void* comm) {
 }
 
 int rs_reduce_stats(rs_handle* h, void* nccl_comm, int32_t root, uint64_t* stats_out) {
-  if (!h || !nccl_comm) return nfail("rs_reduce_stats", "bad argument");
-  ncclComm_t comm = (ncclComm_t)nccl_comm;
-  int32_t S = 0, dev = 0;
-  if (rs_dims(h, nullptr, &S, nullptr, nullptr, &dev) != RS_OK || S < 1) return nfail("rs_dims", rs_last_error());
-  const size_t n = (size_t)4 * S * rs_n_profiles(h);   /* [P][4][S] */
-  int rank = -1;
-  NC(ncclCommUserRank(comm, &rank));
-  CUR(cudaSetDevice(dev));
-  cudaStream_t st = (cudaStream_t)rs_get_stream(h);
-  uint64_t* d = nullptr;
-  CUR(cudaMalloc((void**)&d, sizeof(uint64_t) * n));
-  int rc = rs_stats_device(h, d);
-  if (rc != RS_OK) { cudaFree(d); return nfail("rs_stats_device", rs_last_error()); }
-  ncclResult_t r = ncclReduce(d, d, n, ncclUint64, ncclSum, root, comm, st);
-  cudaError_t e = cudaSuccess;
-  if (r == ncclSuccess && rank == root && stats_out)
-    e = cudaMemcpyAsync(stats_out, d, sizeof(uint64_t) * n, cudaMemcpyDeviceToHost, st);
-  if (r == ncclSuccess && e == cudaSuccess) e = cudaStreamSynchronize(st);
-  cudaFree(d);
-  if (r != ncclSuccess) return nfail("ncclReduce", ncclGetErrorString(r));
-  if (e != cudaSuccess) return nfail("rs_reduce_stats", cudaGetErrorString(e));
-  return RS_OK;
+  return reduce_totals(h, nccl_comm, root, stats_out, 4, rs_stats_device, "rs_reduce_stats", "rs_stats_device");
+}
+
+int rs_reduce_buffer_stats(rs_handle* h, void* nccl_comm, int32_t root, uint64_t* stats_out) {
+  return reduce_totals(h, nccl_comm, root, stats_out, 3, rs_buffer_stats_device, "rs_reduce_buffer_stats",
+                       "rs_buffer_stats_device");
 }
 
 }  /* extern "C" */

@@ -1718,6 +1718,24 @@ int rs_synth_arrivals(rs_handle* h, uint64_t seed, int64_t cell0, int64_t tti0, 
   return RS_OK;
 }
 
+int rs_arrival_spec(double pkt_bytes, double pkts_per_tti, int32_t* pkt_bytes_out, int32_t* pkts_q16) {
+  if (!pkt_bytes_out || !pkts_q16) return fail(RS_ERR_ARG, "rs_arrival_spec: bad argument");
+  if (!(pkt_bytes >= 0 && pkt_bytes <= 0x7fffffff) || pkt_bytes != std::floor(pkt_bytes))
+    return fail(RS_ERR_ARG, "pkt_bytes %g is not an integer 0..2147483647", pkt_bytes);
+  if (!std::isfinite(pkts_per_tti) || pkts_per_tti < 0)
+    return fail(RS_ERR_ARG, "pkts_per_tti %g is not a finite rate >= 0", pkts_per_tti);
+  const double q = std::round(pkts_per_tti * 65536.0);   /* the product is exact: a power-of-two scale */
+  if (q > 0x7fffffff) return fail(RS_ERR_ARG, "pkts_per_tti %g does not fit 16.16 fixed point (under 32768 packets per TTI)", pkts_per_tti);
+  if (pkts_per_tti > 0 && q == 0)
+    return fail(RS_ERR_ARG, "pkts_per_tti %g is below 1/65536 packet per TTI (16.16 fixed point)", pkts_per_tti);
+  const long long qi = (long long)q;
+  if ((long long)pkt_bytes * ((qi >> 16) + 1) > 0x7fffffffLL)
+    return fail(RS_ERR_ARG, "pkt_bytes %g at %g packets per TTI: a TTI's bytes overflow int32", pkt_bytes, pkts_per_tti);
+  *pkt_bytes_out = (int32_t)pkt_bytes;
+  *pkts_q16 = (int32_t)qi;
+  return RS_OK;
+}
+
 int rs_step(rs_handle* h, const uint8_t* cqi, const int32_t* rand2, const uint8_t* active, double dt,
             const rs_outputs* out) {
   return rs_run_host(h, 1, cqi, 1, rand2, active, &dt, out, 1);
@@ -1885,6 +1903,31 @@ int rs_stats_device(rs_handle* h, uint64_t* d_stats) {
       h->d, (unsigned long long*)d_stats, h->P, in_smem);
   CU(cudaGetLastError());
   h->launches++;
+  return RS_OK;
+}
+
+int rs_buffer_stats_device(rs_handle* h, uint64_t* d_stats) {
+  if (!h || !d_stats) return fail(RS_ERR_ARG, "rs_buffer_stats_device: bad argument");
+  if (h->buf_k == 0) return fail(RS_ERR_ARG, "rs_buffer_stats_device: the handle has no buffers (rs_enable_buffers)");
+  CU(cudaSetDevice(h->device));
+  const size_t words = (size_t)3 * h->d.S * h->P;   /* [P][3][S] */
+  CU(cudaMemsetAsync(d_stats, 0, sizeof(uint64_t) * words, h->stream));
+  const size_t total = (size_t)h->B * h->d.U * h->d.nb;
+  const int blocks = (int)std::min<size_t>((total + 255) / 256, 148 * 4);
+  const int in_smem = words * sizeof(unsigned long long) <= 48 * 1024 ? 1 : 0;   /* as rs_stats_device */
+  rs::rs_buffer_stats_kernel<<<blocks, 256, in_smem ? sizeof(unsigned long long) * words : 0, h->stream>>>(
+      h->buf_meta.p, h->d, (unsigned long long*)d_stats, h->P, in_smem);
+  CU(cudaGetLastError());
+  h->launches++;
+  return RS_OK;
+}
+
+int rs_get_buffer_stats(rs_handle* h, uint64_t* stats) {
+  if (!h || !stats) return fail(RS_ERR_ARG, "rs_get_buffer_stats: bad argument");
+  int rc = rs_buffer_stats_device(h, (uint64_t*)h->stats.p);   /* [P][3][S] fits the [P][4][S] scratch */
+  if (rc != RS_OK) return rc;
+  CU(cudaMemcpyAsync(stats, h->stats.p, sizeof(uint64_t) * 3 * h->d.S * h->P, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
   return RS_OK;
 }
 

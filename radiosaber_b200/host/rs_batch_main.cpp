@@ -19,6 +19,20 @@
  *                                               between GPUs inside a TTI; ONE ncclReduce of the per-slice totals at the
  *                                               end (SURVEY 8e; reference analogue: one process per seed + a sum in
  *                                               plot_throughput.py:26-56)
+ *            [--buffers K --traffic FILE ...]   closed loop: a byte FIFO of K records per bearer on the device
+ *                                               (rs_enable_buffers); arrivals drawn by rs_synth_arrivals from the traffic
+ *                                               file, which --traffic names once for every config or once per --config
+ *                                               (file p with config p); every line gains the per-slice queued_bytes,
+ *                                               dropped_bytes and records left at the end
+ *
+ * A traffic file, read with the slice config it goes with:
+ *     {"bearers": 2, "slices": [{"backlogged": 1}, {"pkt_bytes": 1500, "pkts_per_tti": 0.6}, ...]}
+ * "bearers" (1 or 2) becomes rs_config.n_bearers; "slices" has one entry per entry of the config's "slices", in the same
+ * order, and applies to each of its n_slices slices: every bearer of those slices is backlogged (no FIFO), or receives
+ * packets of pkt_bytes bytes at a mean of pkts_per_tti per TTI (rs_arrival_spec converts the rate to 16.16 fixed point).
+ * The config's own traffic fields (internet_flow, if_bitrate, video_*) are not read: LTE-Sim's application models and
+ * RLC header bytes behind them are not modelled here (DESIGN.md), and turning them into packet sizes and rates would
+ * pass an approximation off as the reference's traffic.
  *
  * Host logic only; every scheduling decision is made by the CUDA kernels behind the ABI (no CPU fallback).
  */
@@ -41,6 +55,7 @@
 
 #include "rs_sched.h"
 #include "rs_sched_nccl.h"
+#include "rs_sched_nccl_buffers.h"
 
 namespace {
 
@@ -118,19 +133,25 @@ void cu(cudaError_t e, const char* what) {
 struct Args {
   int algo = 9, cells = 4096, ttis = 1000, log_cell = -1, trace_rows = 475;   /* 475 lines: enb-mac-entity.cc:181 */
   int gpus = 1;
+  int buffers = -1;                  /* --buffers K; -1 = backlogged bearers only, as without the flag */
   uint64_t seed = 1;
-  std::vector<std::string> configs;
+  std::vector<std::string> configs, traffic;
   std::string traces, mapping, log_prefix;
 };
 
 struct Profile {   /* one slice config, expanded like the scheduler constructors do */
   std::vector<double> weight;
   std::vector<int32_t> params, u2s;
+  std::vector<int> groups;         /* n_slices of each entry of the config's "slices" */
+  /* from the traffic file (--buffers), [S] each */
+  std::vector<int32_t> pkt_bytes, pkts_q16;
+  std::vector<uint8_t> backlogged;
 };
 
 struct Setup {   /* what every shard shares */
   Args a;
   int S = 0, U = 0;
+  int nb = 1;                    /* bearers per UE (the traffic file's "bearers") */
   std::vector<Profile> prof;     /* [P]; cell b of the batch uses prof[b % P] */
   bool replay = false;
   int n_traces = 0;
@@ -142,8 +163,50 @@ struct Setup {   /* what every shard shares */
 struct ShardResult {
   double ms = 0;                 /* host clock around the synchronised scheduling calls */
   std::vector<uint64_t> stats;   /* [P][4][S] of this shard's cells (single GPU) or of ALL cells (root after the reduce) */
+  std::vector<uint64_t> buf_stats;   /* [P][3][S] (--buffers), the same way */
   std::string log_out, log_err, error;
 };
+
+std::string read_file(const std::string& path, const char* what) {
+  std::ifstream ifs(path);
+  if (!ifs.is_open()) throw std::runtime_error(std::string("Fail to open ") + what + " file " + path + ".");
+  std::stringstream ss;
+  ss << ifs.rdbuf();
+  return ss.str();
+}
+
+/* The traffic file `path` (format: header comment) for the slice config of `pr`; returns its "bearers". */
+int load_traffic(const std::string& path, Profile* pr) {
+  const std::string text = read_file(path, "traffic");
+  const Json t = Parser(text).value();
+  const std::string where = "traffic file " + path + ": ";
+  const Json& bearers = t["bearers"];
+  if (bearers.kind != Json::Num || (bearers.num != 1 && bearers.num != 2)) throw std::runtime_error(where + "\"bearers\" must be 1 or 2");
+  const Json& groups = t["slices"];
+  if (groups.kind != Json::Arr) throw std::runtime_error(where + "\"slices\" must be a list");
+  if (groups.arr.size() != pr->groups.size())
+    throw std::runtime_error(where + std::to_string(groups.arr.size()) + " entries in \"slices\", the slice config has " +
+                             std::to_string(pr->groups.size()) + " slice groups");
+  for (size_t g = 0; g < groups.arr.size(); ++g) {
+    const Json& e = groups.arr[g];
+    const std::string at = where + "slices[" + std::to_string(g) + "]: ";
+    int32_t pkt = 0, q16 = 0;
+    const bool backlogged = e.kind == Json::Obj && e.obj.size() == 1 && e["backlogged"].kind == Json::Num;
+    if (backlogged) {
+      if (e["backlogged"].num != 1) throw std::runtime_error(at + "\"backlogged\" must be 1");
+    } else {
+      if (e.kind != Json::Obj || e.obj.size() != 2 || e["pkt_bytes"].kind != Json::Num || e["pkts_per_tti"].kind != Json::Num)
+        throw std::runtime_error(at + "expected {\"backlogged\": 1} or {\"pkt_bytes\": n, \"pkts_per_tti\": x}");
+      if (rs_arrival_spec(e["pkt_bytes"].num, e["pkts_per_tti"].num, &pkt, &q16) != RS_OK) throw std::runtime_error(at + rs_last_error());
+    }
+    for (int j = 0; j < pr->groups[g]; ++j) {
+      pr->pkt_bytes.push_back(pkt);
+      pr->pkts_q16.push_back(q16);
+      pr->backlogged.push_back(backlogged ? 1 : 0);
+    }
+  }
+  return bearers.as_int();
+}
 
 constexpr int R = 512, RBG = 8, G = R / RBG;   /* 100 MHz: bandwidth-manager.cpp:98-102, eesm-effective-sinr.h:82-103 */
 
@@ -165,6 +228,7 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
     cfg.weight = su.prof[(size_t)p].weight.data();
     cfg.params = su.prof[(size_t)p].params.data();
     cfg.ue_to_slice = su.prof[(size_t)p].u2s.data();
+    if (a.buffers > 0) cfg.n_bearers = su.nb;
   }
   rs_handle* h = nullptr;
   if (P == 1) {
@@ -187,6 +251,22 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
       for (int u = 0; u < U; ++u) ue_trace[(size_t)b * U + u] = su.map[(size_t)(u + 7 * (int64_t)(cell0 + b)) % n_map];
     check(rs_set_traces(h, su.traces.data(), su.n_traces, n_rows, ue_trace.data()), "rs_set_traces");
   }
+  const bool buffered = a.buffers > 0;
+  const int slots = su.nb;   /* bearers per UE */
+  std::vector<int32_t> pkt_bytes, pkts_q16;   /* [P][S], rs_synth_arrivals' arrival spec */
+  if (buffered) {
+    std::vector<uint8_t> backlogged((size_t)B * U * slots);   /* cell cell0 + b: its config's slices */
+    for (int b = 0; b < B; ++b) {
+      const Profile& pr = su.prof[(size_t)((cell0 + b) % P)];
+      for (int u = 0; u < U; ++u)
+        for (int i = 0; i < slots; ++i) backlogged[((size_t)b * U + u) * slots + i] = pr.backlogged[(size_t)pr.u2s[(size_t)u]];
+    }
+    check(rs_enable_buffers(h, a.buffers, backlogged.data()), "rs_enable_buffers");
+    for (const Profile& pr : su.prof) {   /* profile p of the handle is config p */
+      pkt_bytes.insert(pkt_bytes.end(), pr.pkt_bytes.begin(), pr.pkt_bytes.end());
+      pkts_q16.insert(pkts_q16.end(), pr.pkts_q16.begin(), pr.pkts_q16.end());
+    }
+  }
 
   /* ---- run in blocks of TB TTIs with everything resident on the device ------------------------------- */
   const int TB = 16;
@@ -197,15 +277,19 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
   size_t n_list = 0;   /* entries per cell of the grant list */
   int32_t *d_bits = nullptr, *d_tgt = nullptr, *d_quo = nullptr;
   uint8_t* d_fc = nullptr;
-  const size_t row = G / 2;
+  int32_t *d_arr = nullptr, *d_qo = nullptr;   /* [TB][B][U][nb]: arrivals; the queues the TTIs showed (logged cell) */
+  double* d_ho = nullptr;                      /* [TB][B][U][nb]: the head-of-line delays they showed */
+  const size_t row = G / 2, per_tti = (size_t)B * U * slots;
   if (!replay) cu(cudaMalloc(&d_cqi, (size_t)TB * B * U * row), "cudaMalloc");
+  if (buffered) cu(cudaMalloc(&d_arr, sizeof(int32_t) * TB * per_tti), "cudaMalloc");
   if (n_draws > 0) cu(cudaMalloc(&d_draws, sizeof(int32_t) * (size_t)TB * B * n_draws), "cudaMalloc");
   const int lc = a.log_cell - cell0;   /* the logged cell, if it lives in this shard */
   const bool want_log = lc >= 0 && lc < B && !a.log_prefix.empty();
   rs_log* lg = nullptr;
   std::vector<int16_t> h_rbg, h_gue, h_grbg;
-  std::vector<int32_t> h_bits, h_tgt, h_quo;
+  std::vector<int32_t> h_bits, h_tgt, h_quo, h_q;
   std::vector<uint8_t> h_fc, h_cqi;
+  std::vector<double> h_hol;
   rs_outputs out;
   memset(&out, 0, sizeof out);
   if (want_log) {
@@ -226,12 +310,23 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
       h_gue.resize(n_list); h_grbg.resize(n_list);
     }
     h_rbg.resize(G); h_bits.resize(U); h_fc.resize(U); h_tgt.resize(S); h_quo.resize(S); h_cqi.resize((size_t)U * row);
+    if (buffered) {
+      cu(cudaMalloc(&d_qo, sizeof(int32_t) * TB * per_tti), "cudaMalloc");
+      cu(cudaMalloc(&d_ho, sizeof(double) * TB * per_tti), "cudaMalloc");
+      h_q.resize((size_t)U * slots); h_hol.resize((size_t)U * slots);
+    }
   }
   std::vector<int32_t> trow(TB);
   for (int t0 = 0; t0 < T; t0 += TB) {
     const int n = std::min(TB, T - t0);
     if (!replay) check(rs_synth_cqi(h, a.seed, cell0, t0, n, d_cqi), "rs_synth_cqi");
     if (n_draws > 0) check(rs_synth_rand2(h, a.seed, cell0, t0, n, d_draws), "rs_synth_rand2");
+    if (buffered) {
+      /* counter-based draws over global cells: N GPUs draw exactly the arrivals one GPU would */
+      check(rs_synth_arrivals(h, a.seed, cell0, t0, n, pkt_bytes.data(), pkts_q16.data(), d_arr), "rs_synth_arrivals");
+      const rs_traffic tr = {d_arr, su.now.data() + t0, su.now.data() + t0, d_qo, d_ho};
+      check(rs_set_traffic(h, &tr), "rs_set_traffic");
+    }
     check(rs_sync(h), "rs_sync");
     const auto w0 = std::chrono::steady_clock::now();
     if (replay) {
@@ -264,6 +359,11 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
         cu(cudaMemcpy(h_fc.data(), d_fc + tb * U, U, cudaMemcpyDeviceToHost), "copy");
         cu(cudaMemcpy(h_tgt.data(), d_tgt + tb * S, sizeof(int32_t) * S, cudaMemcpyDeviceToHost), "copy");
         cu(cudaMemcpy(h_quo.data(), d_quo + tb * S, sizeof(int32_t) * S, cudaMemcpyDeviceToHost), "copy");
+        if (buffered) {   /* what the TTI showed the scheduler: the logged dataToTransmit and hol_delay */
+          cu(cudaMemcpy(h_q.data(), d_qo + tb * U * slots, sizeof(int32_t) * U * slots, cudaMemcpyDeviceToHost), "copy");
+          cu(cudaMemcpy(h_hol.data(), d_ho + tb * U * slots, sizeof(double) * U * slots, cudaMemcpyDeviceToHost), "copy");
+          check(rs_log_set_queues(lg, h_q.data(), h_hol.data()), "rs_log_set_queues");
+        }
         /* PacketScheduler::m_ts counts TTIs since the eNB was created: 100 at the first TTI with bearers */
         const uint64_t ts = 100 + (uint64_t)(t0 + k);
         if (a.algo == 10) {
@@ -286,6 +386,15 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
   } else {
     check(rs_get_stats(h, res->stats.data()), "rs_get_stats");
   }
+  if (buffered) {
+    res->buf_stats.assign((size_t)3 * S * P, 0);
+    if (comm) {
+      if (rs_reduce_buffer_stats(h, comm, 0, res->buf_stats.data()) != RS_OK)
+        throw std::runtime_error(std::string("rs_reduce_buffer_stats: ") + rs_nccl_last_error());
+    } else {
+      check(rs_get_buffer_stats(h, res->buf_stats.data()), "rs_get_buffer_stats");
+    }
+  }
   (void)rank;
   if (lg) {
     res->log_out = rs_log_stdout(lg, nullptr);
@@ -294,6 +403,7 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
   }
   rs_destroy(h);
   cudaFree(d_cqi); cudaFree(d_draws); cudaFree(d_rbg); cudaFree(d_bits); cudaFree(d_fc); cudaFree(d_tgt); cudaFree(d_quo); cudaFree(d_gn); cudaFree(d_gue); cudaFree(d_grbg);
+  cudaFree(d_arr); cudaFree(d_qo); cudaFree(d_ho);
 }
 
 }  // namespace
@@ -316,13 +426,22 @@ int main(int argc, char** argv) {
       else if (k == "--log-cell") a.log_cell = atoi(next().c_str());
       else if (k == "--log-prefix") a.log_prefix = next();
       else if (k == "--gpus") a.gpus = atoi(next().c_str());
+      else if (k == "--buffers") a.buffers = atoi(next().c_str());
+      else if (k == "--traffic") a.traffic.push_back(next());
       else throw std::runtime_error("unknown argument " + k);
     }
     if (a.configs.empty() || a.cells < 1 || a.ttis < 1 || a.trace_rows < 1 || a.gpus < 1 || a.gpus > a.cells) {
       fprintf(stderr, "usage: rs_batch --algo ID --config cfg.json [--config cfg2.json ...] --cells B --ttis T [--seed s] [--gpus N] "
-                      "[--traces DIR --mapping FILE [--trace-rows N]] [--log-cell b --log-prefix P]\n");
+                      "[--traces DIR --mapping FILE [--trace-rows N]] [--log-cell b --log-prefix P] [--buffers K --traffic FILE ...]\n");
       return 2;
     }
+    if (a.buffers != -1 && (a.buffers < 1 || a.buffers > RS_MAX_BUFFER_RECORDS))
+      throw std::runtime_error("--buffers K: K records per bearer, 1.." + std::to_string(RS_MAX_BUFFER_RECORDS));
+    if (a.buffers > 0 && a.traffic.empty()) throw std::runtime_error("--buffers needs --traffic FILE");
+    if (a.buffers < 0 && !a.traffic.empty()) throw std::runtime_error("--traffic needs --buffers K");
+    if (!a.traffic.empty() && a.traffic.size() != 1 && a.traffic.size() != a.configs.size())
+      throw std::runtime_error(std::to_string(a.traffic.size()) + " --traffic files for " + std::to_string(a.configs.size()) +
+                               " --config files: give one for all or one per config");
     /* ---- the slice configs, expanded like the scheduler constructors do -------------------------------- */
     for (const std::string& path : a.configs) {
       std::ifstream ifs(path);
@@ -332,7 +451,8 @@ int main(int argc, char** argv) {
       const std::string text = ss.str();
       const Json cfgj = Parser(text).value();
       Profile pr;
-      for (const Json& grp : cfgj["slices"].arr)
+      for (const Json& grp : cfgj["slices"].arr) {
+        pr.groups.push_back(grp["n_slices"].as_int());
         for (int j = 0; j < grp["n_slices"].as_int(); ++j) {
           pr.weight.push_back(grp["weight"].num);
           pr.params.push_back(grp["algo_alpha"].as_int());
@@ -340,6 +460,7 @@ int main(int argc, char** argv) {
           pr.params.push_back(grp["algo_epsilon"].as_int());
           pr.params.push_back(grp["algo_psi"].as_int());
         }
+      }
       const std::vector<Json>& ups = cfgj["ues_per_slice"].arr;
       for (size_t s = 0; s < ups.size(); ++s)
         for (int j = 0; j < ups[s].as_int(); ++j) pr.u2s.push_back((int32_t)s);
@@ -350,6 +471,13 @@ int main(int argc, char** argv) {
                                  std::to_string(su.S) + " and " + std::to_string(su.U) + " (every config must have the same)");
       su.S = ps;
       su.U = pu;
+      if (a.buffers > 0) {
+        const int nb = load_traffic(a.traffic[a.traffic.size() == 1 ? 0 : su.prof.size()], &pr);
+        if (!su.prof.empty() && nb != su.nb)
+          throw std::runtime_error("traffic files with \"bearers\" " + std::to_string(su.nb) + " and " + std::to_string(nb) +
+                                   " (every config of a batch must have the same)");
+        su.nb = nb;
+      }
       su.prof.push_back(std::move(pr));
     }
     const int S = su.S, B = a.cells, T = a.ttis, P = (int)su.prof.size();
@@ -435,6 +563,14 @@ int main(int argc, char** argv) {
       for (int s = 0; s < S; ++s) printf("%s%llu", s ? ", " : "", (unsigned long long)stats[S + s]);
       printf("], \"slice_mbps_per_cell\": [");
       for (int s = 0; s < S; ++s) printf("%s%.3f", s ? ", " : "", (double)stats[s] * 8 / 1e6 / (T * 1e-3) / Bp);
+      if (a.buffers > 0) {   /* what the config's cells left in their buffers at the end */
+        const uint64_t* bs = res[0].buf_stats.data() + (size_t)p * 3 * S;
+        const char* names[3] = {"queued_bytes", "dropped_bytes", "records"};
+        for (int k = 0; k < 3; ++k) {
+          printf("], \"%s\": [", names[k]);
+          for (int s = 0; s < S; ++s) printf("%s%llu", s ? ", " : "", (unsigned long long)bs[(size_t)k * S + s]);
+        }
+      }
       printf("]}\n");
     }
     for (int r = 0; r < N; ++r) {

@@ -38,6 +38,7 @@ ABI_SYMBOLS = (
     "rs_wait", "rs_dims", "rs_fixed_shape", "rs_direct_metric",
     "rs_create_profiles", "rs_set_cell_profiles", "rs_n_profiles", "rs_set_grant_list_len", "rs_grant_list_len",
     "rs_enable_buffers", "rs_set_traffic", "rs_get_buffers", "rs_synth_arrivals",
+    "rs_buffer_stats_device", "rs_get_buffer_stats", "rs_arrival_spec",
 )
 
 
@@ -167,6 +168,9 @@ def lib():
         L.rs_get_buffers.argtypes = [C.c_void_p] + [C.c_void_p] * 4
         L.rs_synth_arrivals.argtypes = [C.c_void_p, C.c_uint64, C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p,
                                         C.c_void_p]
+        L.rs_buffer_stats_device.argtypes = [C.c_void_p, C.c_void_p]
+        L.rs_get_buffer_stats.argtypes = [C.c_void_p, C.c_void_p]
+        L.rs_arrival_spec.argtypes = [C.c_double, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
         _lib = L
     return _lib
 
@@ -202,6 +206,63 @@ def load_slice_config(path: str):
         raise ValueError("ues_per_slice does not match the number of slices")
     return (np.asarray(weight, dtype=np.float64), np.asarray(params, dtype=np.int32),
             np.asarray(ue_to_slice, dtype=np.int32))
+
+
+def arrival_spec(pkt_bytes, pkts_per_tti):
+    """(pkt_bytes, pkts_q16) of one slice for :meth:`Scheduler.synth_arrivals` / :func:`workload.synth_arrivals`:
+    the rate in 16.16 fixed point, rounded as ``rs_arrival_spec`` rounds it (host only).  ValueError on a value
+    the generator does not take."""
+    pb, q = C.c_int32(), C.c_int32()
+    if lib().rs_arrival_spec(float(pkt_bytes), float(pkts_per_tti), C.byref(pb), C.byref(q)) != 0:
+        raise ValueError(lib().rs_last_error().decode())
+    return int(pb.value), int(q.value)
+
+
+def load_traffic_config(path: str, config_path: str):
+    """Read a traffic file (the format of ``rs_batch --traffic``) for the slice config at ``config_path``.
+
+    ``{"bearers": 1 | 2, "slices": [...]}``: one entry of ``slices`` per entry of the config's ``slices``, in the same
+    order, applying to each of its ``n_slices`` slices: ``{"backlogged": 1}`` (no FIFO) or ``{"pkt_bytes": n,
+    "pkts_per_tti": x}``.  Returns (n_bearers, backlogged bool [U][nb], pkt_bytes int32 [S], pkts_q16 int32 [S]);
+    ValueError names what is wrong."""
+    with open(config_path) as f:
+        groups = [int(g["n_slices"]) for g in json.load(f)["slices"]]
+    _, _, u2s = load_slice_config(config_path)
+    with open(path) as f:
+        t = json.load(f)
+    where = f"traffic file {path}: "
+    if not isinstance(t, dict):
+        raise ValueError(where + "not a JSON object")
+    nb = t.get("bearers")
+    if isinstance(nb, bool) or nb not in (1, 2):
+        raise ValueError(where + '"bearers" must be 1 or 2')
+    entries = t.get("slices")
+    if not isinstance(entries, list):
+        raise ValueError(where + '"slices" must be a list')
+    if len(entries) != len(groups):
+        raise ValueError(where + f'{len(entries)} entries in "slices", the slice config has {len(groups)} slice groups')
+    pkt, q16, bl = [], [], []
+    num = (int, float)
+    for g, e in enumerate(entries):
+        at = where + f"slices[{g}]: "
+        p = q = 0
+        backlogged = isinstance(e, dict) and set(e) == {"backlogged"}
+        if backlogged:
+            if isinstance(e["backlogged"], bool) or e["backlogged"] != 1:
+                raise ValueError(at + '"backlogged" must be 1')
+        else:
+            if not (isinstance(e, dict) and set(e) == {"pkt_bytes", "pkts_per_tti"}
+                    and all(isinstance(e[k], num) and not isinstance(e[k], bool) for k in e)):
+                raise ValueError(at + 'expected {"backlogged": 1} or {"pkt_bytes": n, "pkts_per_tti": x}')
+            try:
+                p, q = arrival_spec(e["pkt_bytes"], e["pkts_per_tti"])
+            except ValueError as err:
+                raise ValueError(at + str(err)) from None
+        pkt += [p] * groups[g]
+        q16 += [q] * groups[g]
+        bl += [backlogged] * groups[g]
+    backlogged = np.repeat(np.asarray(bl, bool)[u2s][:, None], int(nb), axis=1)
+    return int(nb), backlogged, np.asarray(pkt, np.int32), np.asarray(q16, np.int32)
 
 
 class Scheduler:
@@ -384,6 +445,17 @@ class Scheduler:
               "head_time": np.empty(shape, np.float64), "dropped": np.empty(shape, np.uint64)}
         _check(lib().rs_get_buffers(self._h, *[_ptr(st[k]) for k in ("queued", "n_records", "head_time", "dropped")]))
         return st
+
+    def get_buffer_stats(self):
+        """uint64 [3][S]: per slice, the bytes queued, the bytes dropped and the records held over the bearers with a
+        FIFO; [P][3][S] with P > 1 slice profiles, row p over the cells of profile p (rs_get_buffer_stats)."""
+        st = np.empty((self.n_profiles, 3, self.S), dtype=np.uint64)
+        _check(lib().rs_get_buffer_stats(self._h, _ptr(st)))
+        return st[0] if self.n_profiles == 1 else st
+
+    def buffer_stats_device(self, d_stats):
+        """rs_buffer_stats_device into a DEVICE buffer of n_profiles * 3 * S uint64."""
+        _check(lib().rs_buffer_stats_device(self._h, C.c_void_p(d_stats)))
 
     def synth_arrivals(self, seed, cell0, tti0, n_ttis, pkt_bytes, pkts_q16, d_out):
         """rs_synth_arrivals: int32 [n_ttis][B][U][nb] into device memory; pkt_bytes / pkts_q16: int [P][S] (packet
