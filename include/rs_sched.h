@@ -274,6 +274,58 @@ int rs_synth_arrivals(rs_handle* h, uint64_t seed, int64_t cell0, int64_t tti0, 
  * rate is at least 1/65536 packet per TTI, and a TTI's most bytes, pkt_bytes x ((q >> 16) + 1), fit int32. */
 int rs_arrival_spec(double pkt_bytes, double pkts_per_tti, int32_t* pkt_bytes_out, int32_t* pkts_q16);
 
+/* ---- traffic sources drawn on the device -----------------------------------------------------------
+ * Generic traffic models, parameters given by the caller: periodic frames (video-like) and on-off packet sources
+ * (talk-spurt-like) next to rs_synth_arrivals' smooth rate.  They are NOT LTE-Sim's VoIP, TraceBased or InternetFlow
+ * applications, and the slice config's traffic fields are not read.
+ * A source is set per (profile, slice); every bearer of the slice (both slots with two bearers per UE) runs its own
+ * copy.  Global TTI tau = tti0 + t and global cell = cell0 + b, as in rs_synth_arrivals, so N GPUs drawing their shards
+ * of the cells draw exactly what one GPU draws.
+ *   per-TTI draw     one 64-bit draw per (tau, cell, ue, slot): rs_synth_arrivals' counter and key.  RATE uses its top
+ *                    16 bits, unchanged; ONOFF compares its low 32 bits with the leaving probability of its state.
+ *   per-bearer draw  one 64-bit draw per (cell, ue, slot) under its own key ("SRC\0"), no tau in the counter.  It gives
+ *                    the phase phi = (draw >> 32) % period_ttis (PERIODIC, ONOFF: the bearers of a cell do not all
+ *                    burst in the same TTI), the start frame f0 = low32 % n_frames (PERIODIC) and the initial ONOFF
+ *                    state: ON iff low32 < (uint64(leave_off_q32) << 32) / (leave_on_q32 + leave_off_q32), the
+ *                    stationary distribution in integers.
+ *   RATE             exactly rs_synth_arrivals: pkt_bytes x ((q >> 16) + (draw16 < (q & 0xffff))), q = pkts_q16.
+ *   PERIODIC         a frame arrives at tau iff (tau + phi) % period_ttis == 0, of frame_bytes[((tau + phi) /
+ *                    period_ttis + f0) % n_frames] bytes, pushed as one record (a buffer sends it in parts and keeps
+ *                    its arrival time, so its head-of-line delay is the frame's own).
+ *   ONOFF            at tau the chain steps first: it leaves its state iff low32 < leave_on_q32 (ON) / leave_off_q32
+ *                    (OFF); then, if ON and (tau + phi) % period_ttis == 0, pkt_bytes arrive.
+ * ONOFF is the only kind with state: one byte per bearer in HBM, owned by the handle.  rs_set_sources (again) resets
+ * every chain to its initial draw; the first rs_synth_traffic call after it may start at any tti0 >= 0, each later call
+ * must continue the chain: tti0 = the previous call's tti0 + n_ttis, with the same seed and cell0, else RS_ERR_ARG.
+ * So one 64-TTI call draws exactly what four 16-TTI calls draw. */
+#define RS_SRC_NONE 0      /* no arrivals (backlogged slices, or a silent slice) */
+#define RS_SRC_RATE 1      /* exactly rs_synth_arrivals: pkt_bytes x ((q >> 16) + (draw16 < (q & 0xffff))) */
+#define RS_SRC_PERIODIC 2  /* one frame every period_ttis TTIs; frame sizes cycle through frame_bytes[n_frames] */
+#define RS_SRC_ONOFF 3     /* two-state Markov chain; while ON one pkt_bytes packet every period_ttis TTIs */
+#define RS_MAX_FRAMES 1024
+typedef struct rs_source {
+  int32_t kind;
+  int32_t pkt_bytes;            /* RATE: 0..INT32_MAX; ONOFF: 1..INT32_MAX */
+  int32_t pkts_q16;             /* RATE: packets per TTI, 16.16 (rs_arrival_spec) */
+  int32_t period_ttis;          /* PERIODIC, ONOFF: >= 1 */
+  uint32_t leave_on_q32;        /* ONOFF: per-TTI probability of leaving ON, 0.32 fixed point (rs_onoff_spec), >= 1 */
+  uint32_t leave_off_q32;       /* ONOFF: per-TTI probability of leaving OFF, >= 1 */
+  int32_t n_frames;             /* PERIODIC: 1..RS_MAX_FRAMES */
+  const int32_t* frame_bytes;   /* PERIODIC: HOST [n_frames], each 1..INT32_MAX; copied by rs_set_sources */
+} rs_source;
+/* The handle's sources, src HOST [P][S] (P = rs_n_profiles; cell b uses the row of its profile).  Every entry is
+ * checked first (kind, sizes, period, frames, leaving probabilities, RATE's int32 rule of rs_synth_arrivals): RS_ERR_ARG
+ * names the profile and slice of the first bad one and nothing changes.  Fields a kind does not use are ignored.
+ * Ordered on the handle's stream like the generator; rs_synth_arrivals never touches these sources. */
+int rs_set_sources(rs_handle* h, const rs_source* src);
+/* Arrivals of the sources into DEVICE int32 [n_ttis][B][U][nb], exactly what rs_set_traffic takes.  Asynchronous on the
+ * handle's stream.  RS_ERR_ARG without rs_set_sources, for tti0 < 0, or for a call that does not continue the chain. */
+int rs_synth_traffic(rs_handle* h, uint64_t seed, int64_t cell0, int64_t tti0, int32_t n_ttis, int32_t* d_out);
+/* ONOFF leaving probabilities from mean ON and OFF run lengths in TTIs (host only, no GPU needed; rs_batch and
+ * radiosaber_b200/sched.py onoff_spec both use it): q = 2^32 / mean rounded to the nearest integer (halves away from
+ * zero).  RS_ERR_ARG, with the reason in rs_last_error, unless each mean is finite and in [2, 2^32]. */
+int rs_onoff_spec(double on_ttis, double off_ttis, uint32_t* leave_on_q32, uint32_t* leave_off_q32);
+
 /* n_ttis consecutive TTIs with every input and output already in DEVICE memory.
  *   d_cqi   [ceil(T/cqi_refresh)][B][U][row]: TTI t reads slab t / cqi_refresh (the reference refreshes
  *           CQI every 40 TTIs, enb-mac-entity.cc:38; the headline workload every TTI);

@@ -2378,28 +2378,73 @@ __global__ void rs_synth_rand2_kernel(int* out, unsigned long long key, long lon
   }
 }
 
-/* Synthetic arrivals (twin of workload.synth_arrivals): int32 [n_ttis][n_cells][U][nb].  spec [P][S][2] = (packet
- * bytes, packets per TTI in 16.16 fixed point) of each profile's slices; a bearer gets (q >> 16) + (draw16 < (q & 0xffff))
- * packets, draw16 the top 16 bits of one counter-based draw per (tti, cell, ue, slot). */
-__global__ void rs_synth_arrivals_kernel(int* out, unsigned long long key, long long cell0, long long tti0, int n_ttis,
-                                         const DevCfg d, const int* spec) {
-  const int nb = d.nb, U = d.U, S = d.S;
-  const size_t total = (size_t)n_ttis * d.n_cells * U * nb;
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
-    const unsigned long long slot = i % nb;
-    size_t r = i / nb;
-    const int u = (int)(r % U); r /= U;
-    const int b = (int)(r % d.n_cells);
-    const unsigned long long cell = cell0 + b;
-    const unsigned long long tti = tti0 + (long long)(r / d.n_cells);
-    const int pf = d.cell_profile ? d.cell_profile[b] : 0;
-    const int* sp = spec + 2 * ((size_t)pf * S + d.ue_to_slice[(size_t)pf * U + u]);
-    const unsigned long long ue = (unsigned long long)u;
-    const unsigned long long ctr = ((tti << 40) ^ (cell << 20) ^ (ue << 8) ^ slot) ^ ((ue >> 12) * 0xD6E8FEB86659FD93ull);
-    const unsigned draw16 = (unsigned)(splitmix64(ctr ^ key) >> 48);
-    const int q = sp[1];
-    out[i] = sp[0] * ((q >> 16) + (draw16 < (unsigned)(q & 0xffff) ? 1 : 0));
+/* One traffic source (rs_source of include/rs_sched.h) as the generator reads it; frames live in a separate table at
+ * frame_off.  on0 = the initial-state threshold of an ONOFF chain, (leave_off << 32) / (leave_on + leave_off). */
+struct SrcRow {
+  int kind, pkt_bytes, pkts_q16, period;
+  unsigned leave_on, leave_off, on0;
+  int n_frames, frame_off;
+};
+enum { kSrcNone = 0, kSrcRate = 1, kSrcPeriodic = 2, kSrcOnOff = 3 };
+
+/* Synthetic traffic (twin of workload.synth_traffic): int32 [n_ttis][n_cells][U][nb], one thread per bearer walking the
+ * call's TTIs, so the stores of each TTI are coalesced across bearers.  src [P][S] is the source of each profile's
+ * slices.  Per (tti, cell, ue, slot) one draw under key_arr, the counter of rs_synth_cqi (RATE: top 16 bits; ONOFF: low
+ * 32); per (cell, ue, slot) one draw under key_src without the TTI (phase, start frame, initial ONOFF state).  state
+ * [n_cells][U][nb]: the ONOFF chains between calls (null: no chain kept, rs_synth_arrivals); init = start them from the
+ * initial draw instead of reading them. */
+__global__ void __launch_bounds__(256) rs_synth_traffic_kernel(int* out, unsigned long long key_arr,
+                                                               unsigned long long key_src, long long cell0,
+                                                               long long tti0, int n_ttis, const DevCfg d,
+                                                               const SrcRow* src, const int* frames,
+                                                               unsigned char* state, int init) {
+  const int nb = d.nb, U = d.U;
+  const size_t n = (size_t)d.n_cells * U * nb;
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const unsigned long long slot = i % nb;
+  const size_t r = i / nb;
+  const int u = (int)(r % U), b = (int)(r / U);
+  const int pf = d.cell_profile ? d.cell_profile[b] : 0;
+  const SrcRow s = src[(size_t)pf * d.S + d.ue_to_slice[(size_t)pf * U + u]];
+  const unsigned long long ue = (unsigned long long)u, cell = (unsigned long long)(cell0 + b);
+  const unsigned long long ctr = (cell << 20) ^ (ue << 8) ^ slot ^ ((ue >> 12) * 0xD6E8FEB86659FD93ull);
+  unsigned long long tti = (unsigned long long)tti0;
+  int* o = out + i;
+  if (s.kind == kSrcRate) {
+    for (int t = 0; t < n_ttis; ++t, ++tti, o += n) {
+      const unsigned draw16 = (unsigned)(splitmix64((tti << 40) ^ ctr ^ key_arr) >> 48);
+      *o = s.pkt_bytes * ((s.pkts_q16 >> 16) + (draw16 < (unsigned)(s.pkts_q16 & 0xffff) ? 1 : 0));
+    }
+    return;
   }
+  if (s.kind != kSrcPeriodic && s.kind != kSrcOnOff) {
+    for (int t = 0; t < n_ttis; ++t, o += n) *o = 0;
+    return;
+  }
+  /* phase: (tti + phi) % period, kept as a counter from here on; fi = the frame the next phase-0 TTI sends */
+  const unsigned long long hb = splitmix64(ctr ^ key_src);
+  const unsigned lo = (unsigned)hb, period = (unsigned)s.period;
+  const unsigned long long x = tti + (hb >> 32) % period;
+  unsigned ph = (unsigned)(x % period);
+  if (s.kind == kSrcPeriodic) {
+    const unsigned nf = (unsigned)s.n_frames;
+    unsigned fi = (unsigned)(((x / period) % nf + lo % nf) % nf);
+    const int* fr = frames + s.frame_off;
+    for (int t = 0; t < n_ttis; ++t, o += n) {
+      *o = ph == 0 ? fr[fi] : 0;
+      if (++ph == period) { ph = 0; if (++fi == nf) fi = 0; }
+    }
+    return;
+  }
+  bool on = init ? lo < s.on0 : state[i] != 0;
+  for (int t = 0; t < n_ttis; ++t, ++tti, o += n) {
+    const unsigned draw = (unsigned)splitmix64((tti << 40) ^ ctr ^ key_arr);
+    if (draw < (on ? s.leave_on : s.leave_off)) on = !on;
+    *o = on && ph == 0 ? s.pkt_bytes : 0;
+    if (++ph == period) ph = 0;
+  }
+  if (state) state[i] = on ? 1 : 0;
 }
 
 /* rs_get_buffers: the arrival time of every bearer's head record (0 when it holds none) */

@@ -272,7 +272,16 @@ struct rs_handle {
   rs_traffic traffic{};
   DevBuf<int> shown_q;                         /* rs_run_device without queue_out / hol_out: what the TTIs show */
   DevBuf<double> shown_hol;
-  DevBuf<int> synth_spec;                      /* rs_synth_arrivals' [P][S][2] */
+  DevBuf<rs::SrcRow> synth_spec;               /* rs_synth_arrivals' RATE sources [P][S], rebuilt per call */
+  /* traffic sources (rs_set_sources) and the ONOFF chains of rs_synth_traffic */
+  DevBuf<rs::SrcRow> src_tab;                  /* [P][S] */
+  DevBuf<int> src_frames;                      /* the PERIODIC sources' frame sizes, back to back */
+  DevBuf<unsigned char> src_state;             /* [B][U][nb]: 1 = ON */
+  bool src_set = false;                        /* rs_set_sources has been called */
+  bool src_fresh = true;                       /* no launch since rs_set_sources: the chains start from their initial draw */
+  bool src_started = false;                    /* a call since rs_set_sources fixed seed, cell0 and the next TTI */
+  uint64_t src_seed = 0;
+  int64_t src_cell0 = 0, src_next = 0;
   DevBuf<unsigned char> buf_scratch;           /* rs_get_buffers */
   DevBuf<int> tbs1;
   DevBuf<short> vogel_tab;
@@ -552,6 +561,7 @@ void rs_destroy(rs_handle* h) {
   h->holmul.release(); h->tbs1.release(); h->vogel_tab.release();
   h->buf_meta.release(); h->buf_time.release(); h->buf_bytes.release(); h->shown_q.release(); h->shown_hol.release();
   h->synth_spec.release(); h->buf_scratch.release();
+  h->src_tab.release(); h->src_frames.release(); h->src_state.release();
   if (h->own_stream) cudaStreamDestroy(h->own_stream);
   if (h->copy_in) cudaStreamDestroy(h->copy_in);
   if (h->copy_out) cudaStreamDestroy(h->copy_out);
@@ -1685,36 +1695,137 @@ int rs_get_buffers(rs_handle* h, int64_t* queued, int32_t* n_records, double* he
   return RS_OK;
 }
 
+namespace {
+unsigned long long host_splitmix64(unsigned long long x) {
+  unsigned long long z = x + 0x9E3779B97F4A7C15ull;
+  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+  return z ^ (z >> 31);
+}
+/* rs_synth_traffic_kernel over the handle's bearers; keys as workload._key(seed, "ARR\0") / (seed, "SRC\0") */
+int launch_traffic(rs_handle* h, uint64_t seed, int64_t cell0, int64_t tti0, int32_t n_ttis, const rs::SrcRow* src,
+                   const int* frames, unsigned char* state, bool init, int32_t* d_out) {
+  const size_t n = (size_t)h->B * h->d.U * h->d.nb;
+  if (n_ttis == 0 || n == 0) return RS_OK;
+  const unsigned long long key_arr = host_splitmix64((seed & 0xFFFFFFFFull) | (0x41525200ull << 32));
+  const unsigned long long key_src = host_splitmix64((seed & 0xFFFFFFFFull) | (0x53524300ull << 32));
+  rs::rs_synth_traffic_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(d_out, key_arr, key_src, cell0, tti0, n_ttis,
+                                                                                  h->d, src, frames, state, init ? 1 : 0);
+  CU(cudaGetLastError());
+  h->launches++;
+  return RS_OK;
+}
+}  // namespace
+
 int rs_synth_arrivals(rs_handle* h, uint64_t seed, int64_t cell0, int64_t tti0, int32_t n_ttis, const int32_t* pkt_bytes,
                       const int32_t* pkts_q16, int32_t* d_out) {
   if (!h || !pkt_bytes || !pkts_q16 || !d_out || n_ttis < 0) return fail(RS_ERR_ARG, "rs_synth_arrivals: bad argument");
   const int P = h->P, S = h->d.S;
-  std::vector<int> spec((size_t)2 * P * S);
+  std::vector<rs::SrcRow> spec((size_t)P * S);
   for (int i = 0; i < P * S; ++i) {
     if (pkt_bytes[i] < 0 || pkts_q16[i] < 0)
       return fail(RS_ERR_ARG, "rs_synth_arrivals: profile %d slice %d: negative packet size or rate", i / S, i % S);
     if ((long long)pkt_bytes[i] * ((pkts_q16[i] >> 16) + 1) > 0x7fffffffLL)
       return fail(RS_ERR_ARG, "rs_synth_arrivals: profile %d slice %d: a TTI's bytes overflow int32", i / S, i % S);
-    spec[2 * i] = pkt_bytes[i];
-    spec[2 * i + 1] = pkts_q16[i];
+    spec[i] = rs::SrcRow{RS_SRC_RATE, pkt_bytes[i], pkts_q16[i], 1, 0, 0, 0, 0, 0};
   }
   CU(cudaSetDevice(h->device));
   CU(h->synth_spec.alloc(spec.size()));
   /* pageable source: the copy is staged before the call returns; ordered with earlier kernels that read the table */
-  CU(cudaMemcpyAsync(h->synth_spec.p, spec.data(), spec.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
-  auto sm64 = [](unsigned long long x) {
-    unsigned long long z = x + 0x9E3779B97F4A7C15ull;
-    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-    return z ^ (z >> 31);
-  };
-  const unsigned long long key = sm64((seed & 0xFFFFFFFFull) | (0x41525200ull << 32));   /* "ARR\0" */
-  const size_t total_n = (size_t)n_ttis * h->B * h->d.U * h->d.nb;
-  if (total_n == 0) return RS_OK;
-  const int blocks = (int)std::min<size_t>((total_n + 255) / 256, 148 * 16);
-  rs::rs_synth_arrivals_kernel<<<blocks, 256, 0, h->stream>>>(d_out, key, cell0, tti0, n_ttis, h->d, h->synth_spec.p);
-  CU(cudaGetLastError());
-  h->launches++;
+  CU(cudaMemcpyAsync(h->synth_spec.p, spec.data(), spec.size() * sizeof(rs::SrcRow), cudaMemcpyHostToDevice, h->stream));
+  return launch_traffic(h, seed, cell0, tti0, n_ttis, h->synth_spec.p, nullptr, nullptr, false, d_out);
+}
+
+int rs_set_sources(rs_handle* h, const rs_source* src) {
+  if (!h || !src) return fail(RS_ERR_ARG, "rs_set_sources: bad argument");
+  const int P = h->P, S = h->d.S;
+  std::vector<rs::SrcRow> rows((size_t)P * S);
+  std::vector<int> frames;
+  for (int i = 0; i < P * S; ++i) {
+    const rs_source& e = src[i];
+    rs::SrcRow& r = rows[(size_t)i];
+    r = rs::SrcRow{e.kind, 0, 0, 1, 0, 0, 0, 0, 0};
+    const int p = i / S, s = i % S;
+    if (e.kind == RS_SRC_RATE) {
+      if (e.pkt_bytes < 0 || e.pkts_q16 < 0)
+        return fail(RS_ERR_ARG, "rs_set_sources: profile %d slice %d: negative packet size or rate", p, s);
+      if ((long long)e.pkt_bytes * ((e.pkts_q16 >> 16) + 1) > 0x7fffffffLL)
+        return fail(RS_ERR_ARG, "rs_set_sources: profile %d slice %d: a TTI's bytes overflow int32", p, s);
+      r.pkt_bytes = e.pkt_bytes;
+      r.pkts_q16 = e.pkts_q16;
+    } else if (e.kind == RS_SRC_PERIODIC || e.kind == RS_SRC_ONOFF) {
+      if (e.period_ttis < 1) return fail(RS_ERR_ARG, "rs_set_sources: profile %d slice %d: period_ttis %d < 1", p, s, e.period_ttis);
+      r.period = e.period_ttis;
+      if (e.kind == RS_SRC_PERIODIC) {
+        if (e.n_frames < 1 || e.n_frames > RS_MAX_FRAMES || !e.frame_bytes)
+          return fail(RS_ERR_ARG, "rs_set_sources: profile %d slice %d: n_frames %d outside 1..%d (or no frame_bytes)", p, s,
+                      e.n_frames, RS_MAX_FRAMES);
+        for (int k = 0; k < e.n_frames; ++k)
+          if (e.frame_bytes[k] < 1)
+            return fail(RS_ERR_ARG, "rs_set_sources: profile %d slice %d: frame_bytes[%d] = %d is not 1..2147483647", p, s, k,
+                        e.frame_bytes[k]);
+        r.n_frames = e.n_frames;
+        r.frame_off = (int)frames.size();
+        frames.insert(frames.end(), e.frame_bytes, e.frame_bytes + e.n_frames);
+      } else {
+        if (e.pkt_bytes < 1) return fail(RS_ERR_ARG, "rs_set_sources: profile %d slice %d: pkt_bytes %d < 1", p, s, e.pkt_bytes);
+        if (e.leave_on_q32 < 1 || e.leave_off_q32 < 1)
+          return fail(RS_ERR_ARG, "rs_set_sources: profile %d slice %d: a leaving probability of 0 (rs_onoff_spec)", p, s);
+        r.pkt_bytes = e.pkt_bytes;
+        r.leave_on = e.leave_on_q32;
+        r.leave_off = e.leave_off_q32;
+        r.on0 = (unsigned)(((unsigned long long)e.leave_off_q32 << 32) /
+                           ((unsigned long long)e.leave_on_q32 + e.leave_off_q32));
+      }
+    } else if (e.kind != RS_SRC_NONE) {
+      return fail(RS_ERR_ARG, "rs_set_sources: profile %d slice %d: kind %d is not RS_SRC_NONE..RS_SRC_ONOFF", p, s, e.kind);
+    }
+  }
+  CU(cudaSetDevice(h->device));
+  CU(h->src_tab.alloc(rows.size()));
+  CU(h->src_frames.alloc(frames.size()));
+  CU(h->src_state.alloc((size_t)h->B * h->d.U * h->d.nb));
+  /* pageable sources: staged before the call returns, ordered after the launches that read the old tables */
+  CU(cudaMemcpyAsync(h->src_tab.p, rows.data(), rows.size() * sizeof(rs::SrcRow), cudaMemcpyHostToDevice, h->stream));
+  if (!frames.empty())
+    CU(cudaMemcpyAsync(h->src_frames.p, frames.data(), frames.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+  h->src_set = true;
+  h->src_fresh = true;
+  h->src_started = false;
+  return RS_OK;
+}
+
+int rs_synth_traffic(rs_handle* h, uint64_t seed, int64_t cell0, int64_t tti0, int32_t n_ttis, int32_t* d_out) {
+  if (!h || !d_out || n_ttis < 0 || tti0 < 0) return fail(RS_ERR_ARG, "rs_synth_traffic: bad argument");
+  if (!h->src_set) return fail(RS_ERR_ARG, "rs_synth_traffic: no sources (rs_set_sources)");
+  if (h->src_started && (tti0 != h->src_next || seed != h->src_seed || cell0 != h->src_cell0))
+    return fail(RS_ERR_ARG, "rs_synth_traffic: the on-off chains continue at tti0 %lld with seed %llu and cell0 %lld "
+                "(called with %lld, %llu, %lld); rs_set_sources restarts them", (long long)h->src_next,
+                (unsigned long long)h->src_seed, (long long)h->src_cell0, (long long)tti0, (unsigned long long)seed,
+                (long long)cell0);
+  CU(cudaSetDevice(h->device));
+  const int rc = launch_traffic(h, seed, cell0, tti0, n_ttis, h->src_tab.p, h->src_frames.p, h->src_state.p, h->src_fresh, d_out);
+  if (rc != RS_OK) return rc;
+  if (n_ttis > 0) h->src_fresh = false;
+  h->src_started = true;
+  h->src_seed = seed;
+  h->src_cell0 = cell0;
+  h->src_next = tti0 + n_ttis;
+  return RS_OK;
+}
+
+int rs_onoff_spec(double on_ttis, double off_ttis, uint32_t* leave_on_q32, uint32_t* leave_off_q32) {
+  if (!leave_on_q32 || !leave_off_q32) return fail(RS_ERR_ARG, "rs_onoff_spec: bad argument");
+  const double mean[2] = {on_ttis, off_ttis};
+  const char* name[2] = {"on_ttis", "off_ttis"};
+  uint32_t q[2];
+  for (int k = 0; k < 2; ++k) {
+    if (!(mean[k] >= 2.0 && mean[k] <= 4294967296.0))   /* NaN fails too */
+      return fail(RS_ERR_ARG, "%s %g is not a finite mean in [2, 2^32] TTIs", name[k], mean[k]);
+    q[k] = (uint32_t)std::round(4294967296.0 / mean[k]);   /* 1 .. 2^31 */
+  }
+  *leave_on_q32 = q[0];
+  *leave_off_q32 = q[1];
   return RS_OK;
 }
 

@@ -20,22 +20,32 @@
  *                                               end (SURVEY 8e; reference analogue: one process per seed + a sum in
  *                                               plot_throughput.py:26-56)
  *            [--buffers K --traffic FILE ...]   closed loop: a byte FIFO of K records per bearer on the device
- *                                               (rs_enable_buffers); arrivals drawn by rs_synth_arrivals from the traffic
- *                                               file, which --traffic names once for every config or once per --config
+ *                                               (rs_enable_buffers); arrivals drawn on the device by the traffic file's
+ *                                               sources (rs_set_sources, rs_synth_traffic), the file named by --traffic
+ *                                               once for every config or once per --config
  *                                               (file p with config p); every line gains the per-slice queued_bytes,
  *                                               dropped_bytes and records left at the end
  *
  * A traffic file, read with the slice config it goes with:
  *     {"bearers": 2, "slices": [{"backlogged": 1}, {"pkt_bytes": 1500, "pkts_per_tti": 0.6}, ...]}
  * "bearers" (1 or 2) becomes rs_config.n_bearers; "slices" has one entry per entry of the config's "slices", in the same
- * order, and applies to each of its n_slices slices: every bearer of those slices is backlogged (no FIFO), or receives
- * packets of pkt_bytes bytes at a mean of pkts_per_tti per TTI (rs_arrival_spec converts the rate to 16.16 fixed point).
- * The config's own traffic fields (internet_flow, if_bitrate, video_*) are not read: LTE-Sim's application models and
+ * order, and applies to each of its n_slices slices.  Every bearer of those slices
+ *   {"backlogged": 1}                                   is backlogged (no FIFO);
+ *   {"pkt_bytes": n, "pkts_per_tti": x}                 receives packets of n bytes at a mean of x per TTI (RS_SRC_RATE;
+ *                                                       rs_arrival_spec converts the rate to 16.16 fixed point);
+ *   {"period_ttis": n, "frame_bytes": [f0, f1, ...]}    receives one frame every n TTIs, sizes cycling through the list
+ *                                                       (RS_SRC_PERIODIC);
+ *   {"pkt_bytes": n, "period_ttis": p,                  runs an on-off chain with mean ON / OFF runs of x / y TTIs
+ *    "on_ttis": x, "off_ttis": y}                       (rs_onoff_spec) and receives n bytes every p TTIs while ON
+ *                                                       (RS_SRC_ONOFF).
+ * These are generic traffic models, not LTE-Sim's VoIP, TraceBased or InternetFlow applications.  The config's own
+ * traffic fields (internet_flow, if_bitrate, video_*) are not read: LTE-Sim's application models and
  * RLC header bytes behind them are not modelled here (DESIGN.md), and turning them into packet sizes and rates would
  * pass an approximation off as the reference's traffic.
  *
  * Host logic only; every scheduling decision is made by the CUDA kernels behind the ABI (no CPU fallback).
  */
+#include <algorithm>
 #include <cctype>
 #include <chrono>
 #include <cmath>
@@ -143,9 +153,10 @@ struct Profile {   /* one slice config, expanded like the scheduler constructors
   std::vector<double> weight;
   std::vector<int32_t> params, u2s;
   std::vector<int> groups;         /* n_slices of each entry of the config's "slices" */
-  /* from the traffic file (--buffers), [S] each */
-  std::vector<int32_t> pkt_bytes, pkts_q16;
+  /* from the traffic file (--buffers): src and backlogged [S]; frames [groups], a PERIODIC entry's frame sizes */
+  std::vector<rs_source> src;
   std::vector<uint8_t> backlogged;
+  std::vector<std::vector<int32_t>> frames;
 };
 
 struct Setup {   /* what every shard shares */
@@ -175,6 +186,51 @@ std::string read_file(const std::string& path, const char* what) {
   return ss.str();
 }
 
+/* x as an integer lo..INT32_MAX, else the reason (the words of sched.py's load_traffic) */
+int32_t int_in(double x, double lo, const char* name) {
+  if (!(x >= lo && x <= 2147483647.0) || x != std::floor(x)) {
+    char buf[128];
+    snprintf(buf, sizeof buf, "%s %g is not an integer %g..2147483647", name, x, lo);
+    throw std::invalid_argument(buf);
+  }
+  return (int32_t)x;
+}
+
+/* One entry of "slices" -> its source (kind RS_SRC_NONE = backlogged); frames receives a PERIODIC entry's sizes. */
+rs_source parse_source(const Json& e, std::vector<int32_t>* frames) {
+  rs_source src;
+  memset(&src, 0, sizeof src);
+  const size_t nk = e.kind == Json::Obj ? e.obj.size() : 0;
+  auto num = [&](const char* k) { return e[k].kind == Json::Num; };
+  if (nk == 1 && num("backlogged")) {
+    if (e["backlogged"].num != 1) throw std::invalid_argument("\"backlogged\" must be 1");
+    src.kind = RS_SRC_NONE;
+  } else if (nk == 2 && num("pkt_bytes") && num("pkts_per_tti")) {
+    src.kind = RS_SRC_RATE;
+    if (rs_arrival_spec(e["pkt_bytes"].num, e["pkts_per_tti"].num, &src.pkt_bytes, &src.pkts_q16) != RS_OK)
+      throw std::invalid_argument(rs_last_error());
+  } else if (nk == 2 && num("period_ttis") && e["frame_bytes"].kind == Json::Arr &&
+             std::all_of(e["frame_bytes"].arr.begin(), e["frame_bytes"].arr.end(), [](const Json& v) { return v.kind == Json::Num; })) {
+    src.kind = RS_SRC_PERIODIC;
+    src.period_ttis = int_in(e["period_ttis"].num, 1, "period_ttis");
+    const std::vector<Json>& f = e["frame_bytes"].arr;
+    if (f.empty() || f.size() > RS_MAX_FRAMES)
+      throw std::invalid_argument(std::to_string(f.size()) + " frame_bytes, expected 1.." + std::to_string(RS_MAX_FRAMES));
+    for (const Json& v : f) frames->push_back(int_in(v.num, 1, "frame_bytes"));
+    src.n_frames = (int32_t)f.size();
+  } else if (nk == 4 && num("pkt_bytes") && num("period_ttis") && num("on_ttis") && num("off_ttis")) {
+    src.kind = RS_SRC_ONOFF;
+    src.pkt_bytes = int_in(e["pkt_bytes"].num, 1, "pkt_bytes");
+    src.period_ttis = int_in(e["period_ttis"].num, 1, "period_ttis");
+    if (rs_onoff_spec(e["on_ttis"].num, e["off_ttis"].num, &src.leave_on_q32, &src.leave_off_q32) != RS_OK)
+      throw std::invalid_argument(rs_last_error());
+  } else {
+    throw std::invalid_argument("expected {\"backlogged\": 1}, {\"pkt_bytes\": n, \"pkts_per_tti\": x}, {\"period_ttis\": n, "
+                                "\"frame_bytes\": [n, ...]} or {\"pkt_bytes\": n, \"period_ttis\": n, \"on_ttis\": x, \"off_ttis\": x}");
+  }
+  return src;
+}
+
 /* The traffic file `path` (format: header comment) for the slice config of `pr`; returns its "bearers". */
 int load_traffic(const std::string& path, Profile* pr) {
   const std::string text = read_file(path, "traffic");
@@ -187,22 +243,17 @@ int load_traffic(const std::string& path, Profile* pr) {
   if (groups.arr.size() != pr->groups.size())
     throw std::runtime_error(where + std::to_string(groups.arr.size()) + " entries in \"slices\", the slice config has " +
                              std::to_string(pr->groups.size()) + " slice groups");
+  pr->frames.resize(groups.arr.size());
   for (size_t g = 0; g < groups.arr.size(); ++g) {
-    const Json& e = groups.arr[g];
-    const std::string at = where + "slices[" + std::to_string(g) + "]: ";
-    int32_t pkt = 0, q16 = 0;
-    const bool backlogged = e.kind == Json::Obj && e.obj.size() == 1 && e["backlogged"].kind == Json::Num;
-    if (backlogged) {
-      if (e["backlogged"].num != 1) throw std::runtime_error(at + "\"backlogged\" must be 1");
-    } else {
-      if (e.kind != Json::Obj || e.obj.size() != 2 || e["pkt_bytes"].kind != Json::Num || e["pkts_per_tti"].kind != Json::Num)
-        throw std::runtime_error(at + "expected {\"backlogged\": 1} or {\"pkt_bytes\": n, \"pkts_per_tti\": x}");
-      if (rs_arrival_spec(e["pkt_bytes"].num, e["pkts_per_tti"].num, &pkt, &q16) != RS_OK) throw std::runtime_error(at + rs_last_error());
+    rs_source src;
+    try {
+      src = parse_source(groups.arr[g], &pr->frames[g]);
+    } catch (const std::invalid_argument& e) {
+      throw std::runtime_error(where + "slices[" + std::to_string(g) + "]: " + e.what());
     }
     for (int j = 0; j < pr->groups[g]; ++j) {
-      pr->pkt_bytes.push_back(pkt);
-      pr->pkts_q16.push_back(q16);
-      pr->backlogged.push_back(backlogged ? 1 : 0);
+      pr->src.push_back(src);
+      pr->backlogged.push_back(src.kind == RS_SRC_NONE ? 1 : 0);
     }
   }
   return bearers.as_int();
@@ -253,7 +304,6 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
   }
   const bool buffered = a.buffers > 0;
   const int slots = su.nb;   /* bearers per UE */
-  std::vector<int32_t> pkt_bytes, pkts_q16;   /* [P][S], rs_synth_arrivals' arrival spec */
   if (buffered) {
     std::vector<uint8_t> backlogged((size_t)B * U * slots);   /* cell cell0 + b: its config's slices */
     for (int b = 0; b < B; ++b) {
@@ -262,10 +312,14 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
         for (int i = 0; i < slots; ++i) backlogged[((size_t)b * U + u) * slots + i] = pr.backlogged[(size_t)pr.u2s[(size_t)u]];
     }
     check(rs_enable_buffers(h, a.buffers, backlogged.data()), "rs_enable_buffers");
-    for (const Profile& pr : su.prof) {   /* profile p of the handle is config p */
-      pkt_bytes.insert(pkt_bytes.end(), pr.pkt_bytes.begin(), pr.pkt_bytes.end());
-      pkts_q16.insert(pkts_q16.end(), pr.pkts_q16.begin(), pr.pkts_q16.end());
-    }
+    std::vector<rs_source> src;   /* [P][S]: profile p of the handle is config p */
+    for (const Profile& pr : su.prof)
+      for (size_t g = 0, s = 0; g < pr.groups.size(); ++g)
+        for (int j = 0; j < pr.groups[g]; ++j, ++s) {
+          src.push_back(pr.src[s]);
+          if (src.back().kind == RS_SRC_PERIODIC) src.back().frame_bytes = pr.frames[g].data();
+        }
+    check(rs_set_sources(h, src.data()), "rs_set_sources");
   }
 
   /* ---- run in blocks of TB TTIs with everything resident on the device ------------------------------- */
@@ -323,7 +377,7 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
     if (n_draws > 0) check(rs_synth_rand2(h, a.seed, cell0, t0, n, d_draws), "rs_synth_rand2");
     if (buffered) {
       /* counter-based draws over global cells: N GPUs draw exactly the arrivals one GPU would */
-      check(rs_synth_arrivals(h, a.seed, cell0, t0, n, pkt_bytes.data(), pkts_q16.data(), d_arr), "rs_synth_arrivals");
+      check(rs_synth_traffic(h, a.seed, cell0, t0, n, d_arr), "rs_synth_traffic");
       const rs_traffic tr = {d_arr, su.now.data() + t0, su.now.data() + t0, d_qo, d_ho};
       check(rs_set_traffic(h, &tr), "rs_set_traffic");
     }

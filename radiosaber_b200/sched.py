@@ -39,6 +39,7 @@ ABI_SYMBOLS = (
     "rs_create_profiles", "rs_set_cell_profiles", "rs_n_profiles", "rs_set_grant_list_len", "rs_grant_list_len",
     "rs_enable_buffers", "rs_set_traffic", "rs_get_buffers", "rs_synth_arrivals",
     "rs_buffer_stats_device", "rs_get_buffer_stats", "rs_arrival_spec",
+    "rs_set_sources", "rs_synth_traffic", "rs_onoff_spec",
 )
 
 
@@ -74,6 +75,17 @@ class _CellIo(C.Structure):
 class _Traffic(C.Structure):
     _fields_ = [("arrivals", C.c_void_p), ("now", C.c_void_p), ("arrival_time", C.c_void_p), ("queue_out", C.c_void_p),
                 ("hol_out", C.c_void_p)]
+
+
+class _Source(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("pkt_bytes", C.c_int32), ("pkts_q16", C.c_int32), ("period_ttis", C.c_int32),
+                ("leave_on_q32", C.c_uint32), ("leave_off_q32", C.c_uint32), ("n_frames", C.c_int32),
+                ("frame_bytes", C.c_void_p)]
+
+
+SRC_NONE, SRC_RATE, SRC_PERIODIC, SRC_ONOFF = 0, 1, 2, 3   # rs_source.kind (RS_SRC_*)
+MAX_FRAMES = 1024                                          # RS_MAX_FRAMES
+INT32_MAX = 2147483647
 
 
 def lib():
@@ -171,6 +183,9 @@ def lib():
         L.rs_buffer_stats_device.argtypes = [C.c_void_p, C.c_void_p]
         L.rs_get_buffer_stats.argtypes = [C.c_void_p, C.c_void_p]
         L.rs_arrival_spec.argtypes = [C.c_double, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
+        L.rs_set_sources.argtypes = [C.c_void_p, C.POINTER(_Source)]
+        L.rs_synth_traffic.argtypes = [C.c_void_p, C.c_uint64, C.c_int64, C.c_int64, C.c_int32, C.c_void_p]
+        L.rs_onoff_spec.argtypes = [C.c_double, C.c_double, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]
         _lib = L
     return _lib
 
@@ -218,13 +233,61 @@ def arrival_spec(pkt_bytes, pkts_per_tti):
     return int(pb.value), int(q.value)
 
 
-def load_traffic_config(path: str, config_path: str):
+def onoff_spec(on_ttis, off_ttis):
+    """(leave_on_q32, leave_off_q32) of an on-off source from its mean ON and OFF run lengths in TTIs: 2^32 / mean,
+    rounded as ``rs_onoff_spec`` rounds it (host only).  ValueError unless each mean is finite and in [2, 2^32]."""
+    on, off = C.c_uint32(), C.c_uint32()
+    if lib().rs_onoff_spec(float(on_ttis), float(off_ttis), C.byref(on), C.byref(off)) != 0:
+        raise ValueError(lib().rs_last_error().decode())
+    return int(on.value), int(off.value)
+
+
+_ENTRY_FORMS = ('{"backlogged": 1}, {"pkt_bytes": n, "pkts_per_tti": x}, {"period_ttis": n, "frame_bytes": [n, ...]} '
+                'or {"pkt_bytes": n, "period_ttis": n, "on_ttis": x, "off_ttis": x}')
+
+
+def _int_in(x, lo, name):
+    """x as an int if it is an integer lo..INT32_MAX, else ValueError in the words rs_batch uses."""
+    if not (lo <= x <= INT32_MAX) or x != int(x):
+        raise ValueError(f"{name} {float(x):g} is not an integer {lo}..{INT32_MAX}")
+    return int(x)
+
+
+def _source(e):
+    """One entry of a traffic file's "slices" -> (backlogged, source dict of rs_source's fields); ValueError."""
+    num = lambda v: isinstance(v, (int, float)) and not isinstance(v, bool)   # noqa: E731
+    keys = set(e) if isinstance(e, dict) else None
+    if keys == {"backlogged"}:
+        if isinstance(e["backlogged"], bool) or e["backlogged"] != 1:
+            raise ValueError('"backlogged" must be 1')
+        return True, {"kind": SRC_NONE}
+    if keys == {"pkt_bytes", "pkts_per_tti"} and all(num(v) for v in e.values()):
+        p, q = arrival_spec(e["pkt_bytes"], e["pkts_per_tti"])
+        return False, {"kind": SRC_RATE, "pkt_bytes": p, "pkts_q16": q}
+    if (keys == {"period_ttis", "frame_bytes"} and num(e["period_ttis"]) and isinstance(e["frame_bytes"], list)
+            and all(num(v) for v in e["frame_bytes"])):
+        period = _int_in(e["period_ttis"], 1, "period_ttis")
+        if not 1 <= len(e["frame_bytes"]) <= MAX_FRAMES:
+            raise ValueError(f"{len(e['frame_bytes'])} frame_bytes, expected 1..{MAX_FRAMES}")
+        frames = [_int_in(v, 1, "frame_bytes") for v in e["frame_bytes"]]
+        return False, {"kind": SRC_PERIODIC, "period_ttis": period, "frame_bytes": frames}
+    if keys == {"pkt_bytes", "period_ttis", "on_ttis", "off_ttis"} and all(num(v) for v in e.values()):
+        pkt = _int_in(e["pkt_bytes"], 1, "pkt_bytes")
+        period = _int_in(e["period_ttis"], 1, "period_ttis")
+        on, off = onoff_spec(e["on_ttis"], e["off_ttis"])
+        return False, {"kind": SRC_ONOFF, "pkt_bytes": pkt, "period_ttis": period, "leave_on_q32": on, "leave_off_q32": off}
+    raise ValueError("expected " + _ENTRY_FORMS)
+
+
+def load_traffic(path: str, config_path: str):
     """Read a traffic file (the format of ``rs_batch --traffic``) for the slice config at ``config_path``.
 
     ``{"bearers": 1 | 2, "slices": [...]}``: one entry of ``slices`` per entry of the config's ``slices``, in the same
-    order, applying to each of its ``n_slices`` slices: ``{"backlogged": 1}`` (no FIFO) or ``{"pkt_bytes": n,
-    "pkts_per_tti": x}``.  Returns (n_bearers, backlogged bool [U][nb], pkt_bytes int32 [S], pkts_q16 int32 [S]);
-    ValueError names what is wrong."""
+    order, applying to each of its ``n_slices`` slices: ``{"backlogged": 1}`` (no FIFO), ``{"pkt_bytes": n,
+    "pkts_per_tti": x}`` (RATE), ``{"period_ttis": n, "frame_bytes": [n, ...]}`` (PERIODIC) or ``{"pkt_bytes": n,
+    "period_ttis": n, "on_ttis": x, "off_ttis": x}`` (ONOFF, mean run lengths in TTIs).  Returns (n_bearers, backlogged
+    bool [U][nb], sources: [S] dicts for :meth:`Scheduler.set_sources` / :func:`workload.synth_traffic`); ValueError
+    names what is wrong."""
     with open(config_path) as f:
         groups = [int(g["n_slices"]) for g in json.load(f)["slices"]]
     _, _, u2s = load_slice_config(config_path)
@@ -241,28 +304,28 @@ def load_traffic_config(path: str, config_path: str):
         raise ValueError(where + '"slices" must be a list')
     if len(entries) != len(groups):
         raise ValueError(where + f'{len(entries)} entries in "slices", the slice config has {len(groups)} slice groups')
-    pkt, q16, bl = [], [], []
-    num = (int, float)
+    sources, bl = [], []
     for g, e in enumerate(entries):
-        at = where + f"slices[{g}]: "
-        p = q = 0
-        backlogged = isinstance(e, dict) and set(e) == {"backlogged"}
-        if backlogged:
-            if isinstance(e["backlogged"], bool) or e["backlogged"] != 1:
-                raise ValueError(at + '"backlogged" must be 1')
-        else:
-            if not (isinstance(e, dict) and set(e) == {"pkt_bytes", "pkts_per_tti"}
-                    and all(isinstance(e[k], num) and not isinstance(e[k], bool) for k in e)):
-                raise ValueError(at + 'expected {"backlogged": 1} or {"pkt_bytes": n, "pkts_per_tti": x}')
-            try:
-                p, q = arrival_spec(e["pkt_bytes"], e["pkts_per_tti"])
-            except ValueError as err:
-                raise ValueError(at + str(err)) from None
-        pkt += [p] * groups[g]
-        q16 += [q] * groups[g]
+        try:
+            backlogged, src = _source(e)
+        except ValueError as err:
+            raise ValueError(where + f"slices[{g}]: " + str(err)) from None
+        sources += [src] * groups[g]
         bl += [backlogged] * groups[g]
     backlogged = np.repeat(np.asarray(bl, bool)[u2s][:, None], int(nb), axis=1)
-    return int(nb), backlogged, np.asarray(pkt, np.int32), np.asarray(q16, np.int32)
+    return int(nb), backlogged, sources
+
+
+def load_traffic_config(path: str, config_path: str):
+    """:func:`load_traffic` for a file of backlogged and rate entries only, in the arrays of
+    :func:`workload.synth_arrivals`: (n_bearers, backlogged bool [U][nb], pkt_bytes int32 [S], pkts_q16 int32 [S]).
+    ValueError names what is wrong, and asks for load_traffic on a file with periodic or on-off entries."""
+    nb, backlogged, sources = load_traffic(path, config_path)
+    if any(s["kind"] not in (SRC_NONE, SRC_RATE) for s in sources):
+        raise ValueError(f"traffic file {path}: periodic or on-off entries: read it with load_traffic")
+    pkt = [s.get("pkt_bytes", 0) for s in sources]
+    q16 = [s.get("pkts_q16", 0) for s in sources]
+    return nb, backlogged, np.asarray(pkt, np.int32), np.asarray(q16, np.int32)
 
 
 class Scheduler:
@@ -464,6 +527,28 @@ class Scheduler:
         pq = np.ascontiguousarray(np.asarray(pkts_q16).reshape(self.n_profiles, self.S), dtype=np.int32)
         _check(lib().rs_synth_arrivals(self._h, int(seed), int(cell0), int(tti0), int(n_ttis), _ptr(pb), _ptr(pq),
                                        C.c_void_p(d_out)))
+
+    def set_sources(self, sources):
+        """rs_set_sources: the traffic source of every slice, [S] dicts or [P][S] (one list per profile), with the fields
+        of rs_source (see :func:`workload.synth_traffic`; :func:`load_traffic` returns them).  Restarts the on-off
+        chains."""
+        rows = [list(sources)] if isinstance(sources[0], dict) else [list(p) for p in sources]
+        if len(rows) != self.n_profiles or any(len(r) != self.S for r in rows):
+            raise ValueError(f"sources: expected [{self.n_profiles}][{self.S}]")
+        arr = (_Source * (self.n_profiles * self.S))()
+        keep = []
+        for i, e in enumerate(x for r in rows for x in r):
+            fr = np.ascontiguousarray(e.get("frame_bytes", []), dtype=np.int32)
+            keep.append(fr)
+            arr[i] = _Source(int(e["kind"]), int(e.get("pkt_bytes", 0)), int(e.get("pkts_q16", 0)),
+                             int(e.get("period_ttis", 0)), int(e.get("leave_on_q32", 0)), int(e.get("leave_off_q32", 0)),
+                             int(fr.shape[0]), _ptr(fr) if fr.shape[0] else None)
+        _check(lib().rs_set_sources(self._h, arr))
+
+    def synth_traffic(self, seed, cell0, tti0, n_ttis, d_out):
+        """rs_synth_traffic: int32 [n_ttis][B][U][nb] of the sources into device memory; a call continues the on-off
+        chains of the previous one (tti0 = its tti0 + n_ttis).  Twin of workload.synth_traffic."""
+        _check(lib().rs_synth_traffic(self._h, int(seed), int(cell0), int(tti0), int(n_ttis), C.c_void_p(d_out)))
 
     def _per_bearer(self, lead):
         return lead + ((self.U,) if self.nb == 1 else (self.U, 2))

@@ -157,3 +157,86 @@ def synth_arrivals(seed: int, cell0: int, n_cells: int, tti0: int, n_ttis: int, 
     q = np.take_along_axis(pq[cp], s, axis=1)[None, :, :, None]
     out = (size * ((q >> 16) + (draw16 < (q & 0xffff)))).astype(np.int32)
     return out if nb == 2 else out[..., 0]
+
+
+DOMAIN_SOURCES = 0x53524300  # "SRC\0"
+SRC_NONE, SRC_RATE, SRC_PERIODIC, SRC_ONOFF = 0, 1, 2, 3
+
+
+def synth_traffic(seed: int, cell0: int, n_cells: int, tti0: int, n_ttis: int, ue_to_slice, sources, n_bearers: int = 1,
+                  cell_profile=None, state=None):
+    """(arrivals, state): int32 [n_ttis][n_cells][U] ([..][U][2] with two bearers) bytes arriving at each bearer from the
+    traffic sources, and the on-off chains after the last TTI (uint8, shaped like one TTI of arrivals, 1 = ON; 0 for
+    bearers of other kinds).  ``rs_set_sources`` + ``rs_synth_traffic`` is the device twin, bit for bit.
+
+    sources: one dict per slice ([S]), or one list per slice profile ([P][S]), with the fields of ``rs_source``:
+    ``kind`` (SRC_NONE / SRC_RATE / SRC_PERIODIC / SRC_ONOFF) and ``pkt_bytes``, ``pkts_q16``, ``period_ttis``,
+    ``frame_bytes`` (a list), ``leave_on_q32``, ``leave_off_q32`` as the kind needs them.  state: what an earlier call
+    returned, for a call that continues at its tti0 + n_ttis; None = the chains start from their initial draw.  The rules
+    are those of include/rs_sched.h: global TTI tau = tti0 + t, global cell = cell0 + b; one draw per (tau, cell, ue, slot)
+    (:func:`synth_arrivals`' counter and key: RATE is :func:`synth_arrivals` itself, ONOFF takes the low 32 bits) and one
+    per (cell, ue, slot) under key "SRC" without tau (phase, start frame, initial on-off state)."""
+    src = [list(sources)] if isinstance(sources[0], dict) else [list(p) for p in sources]
+    u2s = np.atleast_2d(np.asarray(ue_to_slice, dtype=np.int64))
+    P, S, U = len(src), len(src[0]), u2s.shape[1]
+    nb = 2 if int(n_bearers) == 2 else 1
+    cp = np.zeros(n_cells, dtype=np.int64) if cell_profile is None else np.asarray(cell_profile, dtype=np.int64)
+
+    def field(name, default=0):
+        return np.array([[int(e.get(name, default)) for e in row] for row in src], dtype=np.int64)   # [P][S]
+
+    kind = field("kind")
+    rate = kind == SRC_RATE
+    arr = synth_arrivals(seed, cell0, n_cells, tti0, n_ttis, u2s, np.where(rate, field("pkt_bytes"), 0),
+                         np.where(rate, field("pkts_q16"), 0), n_bearers=nb, cell_profile=cp)
+    arr = arr.reshape(n_ttis, n_cells, U, nb).astype(np.int64)
+
+    def per_bearer(a):   # [P][S] -> [B][U][1]
+        return np.take_along_axis(a[cp], u2s[cp], axis=1)[:, :, None]
+
+    k = per_bearer(kind)
+    period = per_bearer(np.maximum(field("period_ttis", 1), 1))
+    key = _key(seed, DOMAIN_SOURCES)
+    cell = np.arange(cell0, cell0 + n_cells, dtype=np.uint64)[:, None, None]
+    ue = np.arange(U, dtype=np.uint64)[None, :, None]
+    slot = np.arange(nb, dtype=np.uint64)[None, None, :]
+    with np.errstate(over="ignore"):
+        ctr = (cell << np.uint64(20)) ^ (ue << np.uint64(8)) ^ slot ^ ((ue >> np.uint64(12)) * np.uint64(0xD6E8FEB86659FD93))
+        hb = splitmix64(ctr ^ key)
+    lo = (hb & np.uint64(0xFFFFFFFF)).astype(np.int64)                    # [B][U][nb]
+    phi = ((hb >> np.uint64(32)) % period.astype(np.uint64)).astype(np.int64)
+    tau = np.arange(tti0, tti0 + n_ttis, dtype=np.int64)[:, None, None, None]
+    x = tau + phi                                                          # [T][B][U][nb]
+    aligned = x % period == 0
+
+    periodic = k == SRC_PERIODIC
+    if periodic.any():
+        frames = [np.asarray(e.get("frame_bytes", [1]), dtype=np.int64) if e["kind"] == SRC_PERIODIC else np.ones(1, np.int64)
+                  for row in src for e in row]
+        n_frames = np.array([len(f) for f in frames], dtype=np.int64).reshape(P, S)
+        offset = np.concatenate([[0], np.cumsum(n_frames.reshape(-1))[:-1]]).reshape(P, S)
+        nf, off = per_bearer(n_frames), per_bearer(offset)
+        fi = (x // period + lo % nf) % nf
+        size = np.concatenate(frames)[off + fi]
+        arr = np.where(periodic & aligned, size, arr)
+
+    on = np.zeros((n_cells, U, nb), dtype=bool)
+    onoff = k == SRC_ONOFF
+    if onoff.any():
+        leave_on, leave_off = per_bearer(field("leave_on_q32")), per_bearer(field("leave_off_q32"))
+        if state is None:
+            # the stationary ON probability leave_off / (leave_on + leave_off) in 0.32 fixed point, rounded down
+            thr = (leave_off.astype(np.uint64) << np.uint64(32)) // np.maximum(leave_on + leave_off, 1).astype(np.uint64)
+            on = lo < thr.astype(np.int64)
+        else:
+            on = np.asarray(state).reshape(n_cells, U, nb) != 0
+        on &= onoff
+        pkt = per_bearer(field("pkt_bytes"))
+        akey = _key(seed, DOMAIN_ARRIVALS)
+        with np.errstate(over="ignore"):
+            for t in range(n_ttis):
+                draw = (splitmix64((np.uint64(tti0 + t) << np.uint64(40)) ^ ctr ^ akey) & np.uint64(0xFFFFFFFF)).astype(np.int64)
+                on ^= onoff & (draw < np.where(on, leave_on, leave_off))
+                arr[t] = np.where(onoff, np.where(on & aligned[t], pkt, 0), arr[t])
+    out, st = arr.astype(np.int32), on.astype(np.uint8)
+    return (out, st) if nb == 2 else (out[..., 0], st[..., 0])
