@@ -410,6 +410,54 @@ int rs_synth_cqi(rs_handle* h, uint64_t seed, int64_t cell0, int64_t epoch0, int
 /* d_out: int32 [n_ttis][B][n], n = max(2, rs_rand_draws_per_cell_tti()), values in [0, INT32_MAX - S]. */
 int rs_synth_rand2(rs_handle* h, uint64_t seed, int64_t cell0, int64_t tti0, int32_t n_ttis, int32_t* d_out);
 
+/* ---- synthetic channel drawn on the device ---------------------------------------------------------
+ * CQI with the structure rs_synth_cqi lacks: a per-UE level (cell-centre or cell-edge UEs) and an offset that is
+ * correlated across RBGs and across epochs.  A generic model with caller-given parameters, set per (profile, slice);
+ * every UE of the slice runs its own realisation.  Global cell = cell0 + b and epoch e = epoch0 + j, as in
+ * rs_synth_cqi: slab j holds epoch epoch0 + j, and the consumer's cqi_refresh maps TTIs to slabs.  Stateless in the
+ * epoch: any (cell range, epoch range) can be drawn on its own, in any chunking, on any GPU.
+ *   RS_CH_IID     exactly rs_synth_cqi's value for that (cell, epoch, UE, RBG): same key, counter and thresholds, so a
+ *                 handle whose channels are all IID writes byte for byte what rs_synth_cqi writes.
+ *   RS_CH_FADING  cqi = clamp(L + offset(g, e), 1, 15) at RBG g of epoch e, integers only:
+ *     draws       per (cell, UE) 17 splitmix64 draws under the key ("CHN\0"), counter (cell << 20) ^ (ue << 8) ^ i ^
+ *                 ((ue >> 12) * 0xD6E8FEB86659FD93), i = 0..16;  hi(i) / lo(i) = the draw's top / low 32 bits.
+ *     level       L = 1 + #{k : hi(0) >= level_thr[k]}, fixed for the run.
+ *     paths       K = 8; path k has phase theta_k = hi(1 + k), RBG slope omega_k = slope(lo(1 + k), W_f) and epoch
+ *                 slope nu_k = slope(hi(9 + k), W_t), in phase units (2^32 = one turn), where slope(r, W) =
+ *                 uint32((uint64(r) * (2W + 1)) >> 32) - W is uniform over [-W, W], W_f = floor(2^31 / coherence_rbgs),
+ *                 W_t = floor(2^31 / coherence_epochs), and a coherence of 0 gives W = 0: flat across RBGs, or frozen.
+ *     offset      x = sum_k cos_q14[(theta_k + g * omega_k + uint32(e) * nu_k) >> 22] (uint32 arithmetic; cos_q14 =
+ *                 include/rs_cos_q14.inc, round(16384 cos(2 pi i / 1024))); offset = (x * depth_q8 + 2^22) >> 23
+ *                 (arithmetic shift).  x has standard deviation 2^15, so the offset's is depth_q8 / 256 CQI steps.
+ *     correlation Before rounding and clamping the offset's autocorrelation is sinc(pi dg / coherence_rbgs) x sinc(pi de /
+ *                 coherence_epochs) (sinc(y) = sin(y) / y): offsets one coherence length apart are uncorrelated.
+ * Not a 3GPP TDL/CDL model nor LTE-Sim's path-loss / shadowing / fast-fading tables; L does not move with mobility. */
+#define RS_CH_IID 0
+#define RS_CH_FADING 1
+typedef struct rs_channel {
+  int32_t kind;
+  uint32_t level_thr[14];     /* FADING: non-decreasing thresholds on a 32-bit draw (rs_channel_spec) */
+  int32_t depth_q8;           /* FADING: offset standard deviation in CQI steps, 8.8 fixed point, 0..15 x 256 */
+  int32_t coherence_rbgs;     /* FADING: >= 0, 0 = flat across RBGs */
+  int32_t coherence_epochs;   /* FADING: >= 0, 0 = frozen in time */
+} rs_channel;
+/* The handle's channels, ch HOST [P][S] (P = rs_n_profiles; cell b uses the row of its profile).  Every entry is checked
+ * first (kind, thresholds, depth, coherences): RS_ERR_ARG names the profile and slice of the first bad one and nothing
+ * changes.  Fields IID does not use are ignored.  Ordered on the handle's stream like rs_set_sources. */
+int rs_set_channels(rs_handle* h, const rs_channel* ch);
+/* n_slabs slabs [B][U][row] of the channels' CQI into DEVICE d_out, in the handle's CQI layout (0, or 2: 4-bit packed;
+ * layout 1 is RS_ERR_UNSUPPORTED as in rs_synth_cqi).  Asynchronous on the handle's stream.  RS_ERR_ARG without
+ * rs_set_channels. */
+int rs_synth_channel(rs_handle* h, uint64_t seed, int64_t cell0, int64_t epoch0, int32_t n_slabs, uint8_t* d_out);
+/* A FADING channel from a level histogram and the offset's spread and coherences (host only, no GPU needed; rs_batch and
+ * radiosaber_b200/sched.py channel_spec both use it).  level_counts [15]: integer counts of levels 1..15, total 1..2^32-1;
+ * level_thr[k] = min((cum_k << 32) / total, 2^32 - 1) with cum_k = the counts of levels 1..k+1 (so a level above the
+ * last counted one has probability at most 2^-32).  depth_q8 = depth_cqi x 256 rounded to the nearest integer (halves
+ * away from zero), depth_cqi in [0, 15]; each coherence 0 or in [1, INT32_MAX], rounded the same way.  RS_ERR_ARG, with
+ * the reason in rs_last_error, otherwise (non-integer or negative counts, non-finite values). */
+int rs_channel_spec(const double* level_counts, double depth_cqi, double coherence_rbgs, double coherence_epochs,
+                    rs_channel* out);
+
 /* Per-slice totals over every cell of this handle (what the reference's plotters sum from the
  * stderr log, NSDI23-radiosaber-experiments/exp-customization/plot_throughput.py:26-56).
  * stats: uint64 [P][4][S] = { sum cumulative bytes, sum cumulative RBs, sum q, sum q*q } with

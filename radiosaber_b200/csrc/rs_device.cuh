@@ -2447,6 +2447,100 @@ __global__ void __launch_bounds__(256) rs_synth_traffic_kernel(int* out, unsigne
   if (state) state[i] = on ? 1 : 0;
 }
 
+/* One channel (rs_channel of include/rs_sched.h) as the generator reads it; wf / wt = floor(2^31 / coherence), the
+ * bound of the per-RBG / per-epoch phase slopes (0 for coherence 0). */
+struct ChanRow {
+  int kind, depth_q8;
+  unsigned wf, wt;
+  unsigned thr[14];
+};
+enum { kChIid = 0, kChFading = 1 };
+
+/* a 32-bit draw -> a phase slope uniform over [-w, w] (mod 2^32) */
+__device__ __forceinline__ unsigned chan_slope(unsigned raw, unsigned w) {
+  return (unsigned)(((unsigned long long)raw * (2ull * w + 1)) >> 32) - w;
+}
+
+/* Stores one slab of a (cell, UE) row: lane l holds the CQI of RBGs l (v0) and l + 32 (v1).  Packed: a shuffle pairs
+ * neighbouring RBGs, so lanes 0..G/2-1 store the row's bytes contiguously. */
+__device__ __forceinline__ void chan_store(uint8_t* o, int lane, int G, int packed, int v0, int v1) {
+  if (packed) {
+    /* even lane a: byte (RBG a, a + 1) in bits 0..7, byte (RBG a + 32, a + 33) in bits 8..15 */
+    const unsigned v = (unsigned)v0 | ((unsigned)v1 << 8);
+    const unsigned p = v | (__shfl_down_sync(0xffffffffu, v, 1) << 4);
+    const unsigned q = __shfl_sync(0xffffffffu, p, (2 * lane) & 31);
+    if (lane < G / 2) o[lane] = (uint8_t)(lane < 16 ? q : q >> 8);
+  } else {
+    if (lane < G) o[lane] = (uint8_t)v0;
+    if (lane + 32 < G) o[lane + 32] = (uint8_t)v1;
+  }
+}
+
+/* Synthetic channel (twin of workload.synth_channel): n_slabs slabs [n_cells][U][G] (packed = 0) or [..][G/2] (packed
+ * = 1, RBG 2k in the low nibble), slab j = epoch epoch0 + j.  One warp per (cell, UE) row: lane l owns RBGs l and l + 32
+ * in every slab.  FADING rows: lanes 0..16 make the row's draws under key_chn (counter index 0: level; 1..8: phase and
+ * RBG slope of paths 0..7; 9..16: their epoch slope) and shuffles broadcast them; each sample then sums eight cos_q14
+ * lookups from shared memory, the phases stepping by the epoch slope from slab to slab.  IID rows draw rs_synth_cqi's
+ * values (key_cqi, cdf). */
+__global__ void __launch_bounds__(256) rs_synth_channel_kernel(uint8_t* out, unsigned long long key_cqi,
+                                                               unsigned long long key_chn, long long cell0,
+                                                               long long epoch0, int n_slabs, const DevCfg d,
+                                                               const ChanRow* tab, const short* cos_q14, int packed,
+                                                               CdfTable cdf) {
+  __shared__ short s_cos[1024];
+  for (int i = threadIdx.x; i < 1024; i += blockDim.x) s_cos[i] = cos_q14[i];
+  __syncthreads();
+  const int lane = threadIdx.x & 31, G = d.G, U = d.U;
+  const size_t n_rows = (size_t)d.n_cells * U, row_bytes = packed ? G / 2 : G, slab = n_rows * row_bytes;
+  for (size_t r = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < n_rows;
+       r += ((size_t)gridDim.x * blockDim.x) >> 5) {
+    const int u = (int)(r % U), b = (int)(r / U);
+    const int pf = d.cell_profile ? d.cell_profile[b] : 0;
+    const ChanRow* c = tab + (size_t)pf * d.S + d.ue_to_slice[(size_t)pf * U + u];
+    const unsigned long long ue = (unsigned long long)u, cell = (unsigned long long)(cell0 + b);
+    uint8_t* o = out + r * row_bytes;
+    if (c->kind != kChFading) {   /* the same for the whole warp */
+      for (int j = 0; j < n_slabs; ++j, o += slab) {
+        const unsigned long long e = (unsigned long long)(epoch0 + j);
+        const int v0 = synth_one(key_cqi, e, cell, ue, lane, cdf);
+        const int v1 = lane + 32 < G ? synth_one(key_cqi, e, cell, ue, lane + 32, cdf) : 0;
+        chan_store(o, lane, G, packed, v0, v1);
+      }
+      continue;
+    }
+    const unsigned long long ctr = (cell << 20) ^ (ue << 8) ^ ((ue >> 12) * 0xD6E8FEB86659FD93ull);
+    const unsigned long long hd = splitmix64(ctr ^ (unsigned long long)lane ^ key_chn);
+    const unsigned hi = (unsigned)(hd >> 32);
+    const unsigned sl = lane >= 9 ? chan_slope(hi, c->wt) : chan_slope((unsigned)hd, c->wf);
+    const unsigned lv = __shfl_sync(0xffffffffu, hi, 0);
+    int level = 1;
+#pragma unroll
+    for (int k = 0; k < 14; ++k) level += lv >= c->thr[k];
+    const int depth = c->depth_q8;
+    const unsigned e0 = (unsigned)epoch0;
+    unsigned ph0[8], ph1[8], nu[8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+      const unsigned th = __shfl_sync(0xffffffffu, hi, 1 + k), om = __shfl_sync(0xffffffffu, sl, 1 + k);
+      nu[k] = __shfl_sync(0xffffffffu, sl, 9 + k);
+      ph0[k] = th + (unsigned)lane * om + e0 * nu[k];
+      ph1[k] = ph0[k] + 32u * om;
+    }
+    for (int j = 0; j < n_slabs; ++j, o += slab) {
+      int x0 = 0, x1 = 0;
+#pragma unroll
+      for (int k = 0; k < 8; ++k) {
+        x0 += s_cos[ph0[k] >> 22];
+        x1 += s_cos[ph1[k] >> 22];
+        ph0[k] += nu[k];
+        ph1[k] += nu[k];
+      }
+      chan_store(o, lane, G, packed, min(max(level + ((x0 * depth + (1 << 22)) >> 23), 1), 15),
+                 min(max(level + ((x1 * depth + (1 << 22)) >> 23), 1), 15));
+    }
+  }
+}
+
 /* rs_get_buffers: the arrival time of every bearer's head record (0 when it holds none) */
 __global__ void rs_buf_heads_kernel(const BufMeta* meta, const double* tm, int K, size_t n, double* out) {
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)

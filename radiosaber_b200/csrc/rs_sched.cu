@@ -73,6 +73,9 @@ const int kMcsToItbs[29] = {0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 9, 10, 11, 12, 13, 14,
 const int kTbs[110 * 27] = {
 #include "../../include/rs_tbs_36213.inc"
 };
+const short kCosQ14[1024] = {
+#include "../../include/rs_cos_q14.inc"
+};
 inline int mcs_from_cqi(int cqi) { return 2 * (cqi - 1); }          /* MapCQIToMCS */
 inline int tbs_row(int row, int itbs, const int32_t* row_m1) {
   return row < 0 ? row_m1[itbs] : kTbs[row * 27 + itbs];
@@ -282,6 +285,10 @@ struct rs_handle {
   bool src_started = false;                    /* a call since rs_set_sources fixed seed, cell0 and the next TTI */
   uint64_t src_seed = 0;
   int64_t src_cell0 = 0, src_next = 0;
+  /* synthetic channels (rs_set_channels) */
+  DevBuf<rs::ChanRow> chn_tab;                 /* [P][S] */
+  DevBuf<short> cos_q14;                       /* include/rs_cos_q14.inc */
+  bool chn_set = false;
   DevBuf<unsigned char> buf_scratch;           /* rs_get_buffers */
   DevBuf<int> tbs1;
   DevBuf<short> vogel_tab;
@@ -562,6 +569,7 @@ void rs_destroy(rs_handle* h) {
   h->buf_meta.release(); h->buf_time.release(); h->buf_bytes.release(); h->shown_q.release(); h->shown_hol.release();
   h->synth_spec.release(); h->buf_scratch.release();
   h->src_tab.release(); h->src_frames.release(); h->src_state.release();
+  h->chn_tab.release(); h->cos_q14.release();
   if (h->own_stream) cudaStreamDestroy(h->own_stream);
   if (h->copy_in) cudaStreamDestroy(h->copy_in);
   if (h->copy_out) cudaStreamDestroy(h->copy_out);
@@ -1702,6 +1710,19 @@ unsigned long long host_splitmix64(unsigned long long x) {
   z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
   return z ^ (z >> 31);
 }
+/* rs_synth_cqi's thresholds: the histogram of cqi-traces-noise0 (SURVEY 8d), as in radiosaber_b200/workload.py */
+rs::CdfTable cqi_cdf() {
+  static const unsigned long long hist[15] = {19075, 7082, 33860, 261099, 438688, 199446, 518174, 661977,
+                                              237928, 861279, 596358, 355319, 447453, 12000, 153462};
+  unsigned long long total = 0, cum = 0;
+  for (int i = 0; i < 15; ++i) total += hist[i];
+  rs::CdfTable cdf;
+  for (int i = 0; i < 14; ++i) {
+    cum += hist[i];
+    cdf.thr[i] = (unsigned)(unsigned long long)(((double)cum / (double)total) * 4294967296.0);
+  }
+  return cdf;
+}
 /* rs_synth_traffic_kernel over the handle's bearers; keys as workload._key(seed, "ARR\0") / (seed, "SRC\0") */
 int launch_traffic(rs_handle* h, uint64_t seed, int64_t cell0, int64_t tti0, int32_t n_ttis, const rs::SrcRow* src,
                    const int* frames, unsigned char* state, bool init, int32_t* d_out) {
@@ -1953,23 +1974,8 @@ int rs_synth_cqi(rs_handle* h, uint64_t seed, int64_t cell0, int64_t epoch0, int
   if (!h || !d_out || n_slabs < 0) return fail(RS_ERR_ARG, "rs_synth_cqi: bad argument");
   if (h->d.cqi_per_rb == 1) return fail(RS_ERR_UNSUPPORTED, "synthetic CQI is one value per RBG");
   CU(cudaSetDevice(h->device));
-  /* histogram of cqi-traces-noise0 (SURVEY 8d); thresholds as in radiosaber_b200/workload.py */
-  static const unsigned long long hist[15] = {19075, 7082, 33860, 261099, 438688, 199446, 518174, 661977,
-                                              237928, 861279, 596358, 355319, 447453, 12000, 153462};
-  unsigned long long total = 0, cum = 0;
-  for (int i = 0; i < 15; ++i) total += hist[i];
-  rs::CdfTable cdf;
-  for (int i = 0; i < 14; ++i) {
-    cum += hist[i];
-    cdf.thr[i] = (unsigned)(unsigned long long)(((double)cum / (double)total) * 4294967296.0);
-  }
-  auto sm64 = [](unsigned long long x) {
-    unsigned long long z = x + 0x9E3779B97F4A7C15ull;
-    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-    return z ^ (z >> 31);
-  };
-  const unsigned long long key = sm64((seed & 0xFFFFFFFFull) | (0x43514900ull << 32));
+  const rs::CdfTable cdf = cqi_cdf();
+  const unsigned long long key = host_splitmix64((seed & 0xFFFFFFFFull) | (0x43514900ull << 32));
   const size_t total_n = (size_t)n_slabs * h->B * h->d.U * h->cqi_cols;
   if (total_n == 0) return RS_OK;
   const int blocks = (int)std::min<size_t>((total_n + 255) / 256, 148 * 16);
@@ -2128,3 +2134,94 @@ int rs_test_sort_timed(int32_t device, const uint8_t* keys, int32_t n_arrays, in
 }
 
 }  /* extern "C" */
+
+int rs_set_channels(rs_handle* h, const rs_channel* ch) {
+  if (!h || !ch) return fail(RS_ERR_ARG, "rs_set_channels: bad argument");
+  const int P = h->P, S = h->d.S;
+  std::vector<rs::ChanRow> rows((size_t)P * S);
+  for (int i = 0; i < P * S; ++i) {
+    const rs_channel& e = ch[i];
+    rs::ChanRow& r = rows[(size_t)i];
+    memset(&r, 0, sizeof r);
+    r.kind = e.kind;
+    const int p = i / S, s = i % S;
+    if (e.kind == RS_CH_FADING) {
+      if (e.depth_q8 < 0 || e.depth_q8 > 15 * 256)
+        return fail(RS_ERR_ARG, "rs_set_channels: profile %d slice %d: depth_q8 %d is not 0..3840", p, s, e.depth_q8);
+      if (e.coherence_rbgs < 0)
+        return fail(RS_ERR_ARG, "rs_set_channels: profile %d slice %d: coherence_rbgs %d is below 0", p, s, e.coherence_rbgs);
+      if (e.coherence_epochs < 0)
+        return fail(RS_ERR_ARG, "rs_set_channels: profile %d slice %d: coherence_epochs %d is below 0", p, s, e.coherence_epochs);
+      for (int k = 1; k < 14; ++k)
+        if (e.level_thr[k] < e.level_thr[k - 1])
+          return fail(RS_ERR_ARG, "rs_set_channels: profile %d slice %d: level_thr[%d] < level_thr[%d] (thresholds must not "
+                      "decrease)", p, s, k, k - 1);
+      memcpy(r.thr, e.level_thr, sizeof r.thr);
+      r.depth_q8 = e.depth_q8;
+      r.wf = e.coherence_rbgs ? (unsigned)(2147483648u / (unsigned)e.coherence_rbgs) : 0u;
+      r.wt = e.coherence_epochs ? (unsigned)(2147483648u / (unsigned)e.coherence_epochs) : 0u;
+    } else if (e.kind != RS_CH_IID) {
+      return fail(RS_ERR_ARG, "rs_set_channels: profile %d slice %d: kind %d is not RS_CH_IID or RS_CH_FADING", p, s, e.kind);
+    }
+  }
+  CU(cudaSetDevice(h->device));
+  CU(h->chn_tab.alloc(rows.size()));
+  /* pageable sources: staged before the call returns, ordered after the launches that read the old table */
+  CU(cudaMemcpyAsync(h->chn_tab.p, rows.data(), rows.size() * sizeof(rs::ChanRow), cudaMemcpyHostToDevice, h->stream));
+  if (!h->cos_q14.p) {
+    CU(h->cos_q14.alloc(1024));
+    CU(cudaMemcpyAsync(h->cos_q14.p, kCosQ14, sizeof kCosQ14, cudaMemcpyHostToDevice, h->stream));
+  }
+  h->chn_set = true;
+  return RS_OK;
+}
+
+int rs_synth_channel(rs_handle* h, uint64_t seed, int64_t cell0, int64_t epoch0, int32_t n_slabs, uint8_t* d_out) {
+  if (!h || !d_out || n_slabs < 0) return fail(RS_ERR_ARG, "rs_synth_channel: bad argument");
+  if (h->d.cqi_per_rb == 1) return fail(RS_ERR_UNSUPPORTED, "synthetic CQI is one value per RBG");
+  if (!h->chn_set) return fail(RS_ERR_ARG, "rs_synth_channel: no channels (rs_set_channels)");
+  CU(cudaSetDevice(h->device));
+  const size_t rows = (size_t)h->B * h->d.U;
+  if (n_slabs == 0 || rows == 0) return RS_OK;
+  const unsigned long long key_cqi = host_splitmix64((seed & 0xFFFFFFFFull) | (0x43514900ull << 32));   /* "CQI\0" */
+  const unsigned long long key_chn = host_splitmix64((seed & 0xFFFFFFFFull) | (0x43484E00ull << 32));   /* "CHN\0" */
+  const int blocks = (int)std::min<size_t>((rows + 7) / 8, 148 * 16);   /* one warp per (cell, UE) row */
+  rs::rs_synth_channel_kernel<<<blocks, 256, 0, h->stream>>>(d_out, key_cqi, key_chn, cell0, epoch0, n_slabs, h->d,
+                                                             h->chn_tab.p, h->cos_q14.p, h->d.cqi_per_rb == 2 ? 1 : 0,
+                                                             cqi_cdf());
+  CU(cudaGetLastError());
+  h->launches++;
+  return RS_OK;
+}
+
+int rs_channel_spec(const double* level_counts, double depth_cqi, double coherence_rbgs, double coherence_epochs,
+                    rs_channel* out) {
+  if (!level_counts || !out) return fail(RS_ERR_ARG, "rs_channel_spec: bad argument");
+  unsigned long long count[15], total = 0;
+  for (int k = 0; k < 15; ++k) {
+    const double c = level_counts[k];
+    if (!(c >= 0.0 && c <= 4294967295.0) || c != std::floor(c))   /* NaN fails too */
+      return fail(RS_ERR_ARG, "level_counts[%d] = %g is not an integer 0..4294967295", k, c);
+    count[k] = (unsigned long long)c;
+    total += count[k];
+  }
+  if (total == 0 || total > 0xFFFFFFFFull)
+    return fail(RS_ERR_ARG, "level_counts sum to %llu, expected 1..4294967295", total);
+  if (!(depth_cqi >= 0.0 && depth_cqi <= 15.0)) return fail(RS_ERR_ARG, "depth_cqi %g is not in [0, 15]", depth_cqi);
+  const double coh[2] = {coherence_rbgs, coherence_epochs};
+  const char* name[2] = {"coherence_rbgs", "coherence_epochs"};
+  for (int k = 0; k < 2; ++k)
+    if (coh[k] != 0.0 && !(coh[k] >= 1.0 && coh[k] <= 2147483647.0))
+      return fail(RS_ERR_ARG, "%s %g is not 0 or in [1, 2147483647]", name[k], coh[k]);
+  memset(out, 0, sizeof *out);
+  out->kind = RS_CH_FADING;
+  unsigned long long cum = 0;
+  for (int k = 0; k < 14; ++k) {
+    cum += count[k];
+    out->level_thr[k] = (uint32_t)std::min<unsigned long long>((cum << 32) / total, 0xFFFFFFFFull);
+  }
+  out->depth_q8 = (int32_t)std::round(depth_cqi * 256.0);
+  out->coherence_rbgs = (int32_t)std::round(coherence_rbgs);
+  out->coherence_epochs = (int32_t)std::round(coherence_epochs);
+  return RS_OK;
+}

@@ -25,6 +25,9 @@
  *                                               once for every config or once per --config
  *                                               (file p with config p); every line gains the per-slice queued_bytes,
  *                                               dropped_bytes and records left at the end
+ *            [--channel FILE ...]               synthetic channel CQI drawn on the device (rs_set_channels,
+ *                                               rs_synth_channel) in place of rs_synth_cqi's i.i.d. draws, the file named
+ *                                               once for every config or once per --config; not with --traces
  *
  * A traffic file, read with the slice config it goes with:
  *     {"bearers": 2, "slices": [{"backlogged": 1}, {"pkt_bytes": 1500, "pkts_per_tti": 0.6}, ...]}
@@ -42,6 +45,19 @@
  * traffic fields (internet_flow, if_bitrate, video_*) are not read: LTE-Sim's application models and
  * RLC header bytes behind them are not modelled here (DESIGN.md), and turning them into packet sizes and rates would
  * pass an approximation off as the reference's traffic.
+ *
+ * A channel file, read with the slice config it goes with:
+ *     {"report_ttis": 40, "slices": [{"iid": 1}, {"level_counts": [15 counts], "depth_cqi": 1.5, "coherence_rbgs": 8,
+ *                                                 "coherence_reports": 4}, ...]}
+ * CQI reports fall on the global TTIs that are multiples of "report_ttis" (default 1; 40 is the reference's
+ * CQI_INTERVAL), as in the trace replay path, and report e is epoch e of the channel.  "slices" has one entry per entry
+ * of the config's "slices", applying to each of its n_slices slices:
+ *   {"iid": 1}                                          rs_synth_cqi's i.i.d. draws (RS_CH_IID);
+ *   {"level_counts": [...], "depth_cqi": d,             a per-UE level drawn from the 15 counts and an offset of standard
+ *    "coherence_rbgs": f, "coherence_reports": t}       deviation d CQI steps, coherent over f RBGs and t reports
+ *                                                       (RS_CH_FADING, rs_channel_spec).
+ * Other keys (a "note") are not read.  A file of {"iid": 1} entries with report_ttis 1 gives the output of a run
+ * without --channel, byte for byte.
  *
  * Host logic only; every scheduling decision is made by the CUDA kernels behind the ABI (no CPU fallback).
  */
@@ -122,6 +138,8 @@ struct Parser {
     } else if (s[i] == '"') {
       v.kind = Json::Str;
       str();
+    } else if (s.compare(i, 4, "null") == 0) {   /* read like an absent key, as Python's dict.get reads None */
+      i += 4;
     } else {
       char* end = nullptr;
       v.kind = Json::Num;
@@ -145,7 +163,7 @@ struct Args {
   int gpus = 1;
   int buffers = -1;                  /* --buffers K; -1 = backlogged bearers only, as without the flag */
   uint64_t seed = 1;
-  std::vector<std::string> configs, traffic;
+  std::vector<std::string> configs, traffic, channel;
   std::string traces, mapping, log_prefix;
 };
 
@@ -157,12 +175,14 @@ struct Profile {   /* one slice config, expanded like the scheduler constructors
   std::vector<rs_source> src;
   std::vector<uint8_t> backlogged;
   std::vector<std::vector<int32_t>> frames;
+  std::vector<rs_channel> chn;     /* [S], from the channel file (--channel) */
 };
 
 struct Setup {   /* what every shard shares */
   Args a;
   int S = 0, U = 0;
   int nb = 1;                    /* bearers per UE (the traffic file's "bearers") */
+  int report = 1;                /* TTIs per CQI report: the channel file's "report_ttis" (1 without --channel) */
   std::vector<Profile> prof;     /* [P]; cell b of the batch uses prof[b % P] */
   bool replay = false;
   int n_traces = 0;
@@ -259,6 +279,59 @@ int load_traffic(const std::string& path, Profile* pr) {
   return bearers.as_int();
 }
 
+/* One entry of a channel file's "slices" -> its channel. */
+rs_channel parse_channel(const Json& e) {
+  rs_channel ch;
+  memset(&ch, 0, sizeof ch);
+  const size_t nk = e.kind == Json::Obj ? e.obj.size() : 0;
+  auto num = [&](const char* k) { return e[k].kind == Json::Num; };
+  const Json& lc = e["level_counts"];
+  if (nk == 1 && num("iid")) {
+    if (e["iid"].num != 1) throw std::invalid_argument("\"iid\" must be 1");
+    ch.kind = RS_CH_IID;
+  } else if (nk == 4 && lc.kind == Json::Arr && lc.arr.size() == 15 &&
+             std::all_of(lc.arr.begin(), lc.arr.end(), [](const Json& v) { return v.kind == Json::Num; }) &&
+             num("depth_cqi") && num("coherence_rbgs") && num("coherence_reports")) {
+    double counts[15];
+    for (int k = 0; k < 15; ++k) counts[k] = lc.arr[(size_t)k].num;
+    if (rs_channel_spec(counts, e["depth_cqi"].num, e["coherence_rbgs"].num, e["coherence_reports"].num, &ch) != RS_OK)
+      throw std::invalid_argument(rs_last_error());
+  } else {
+    throw std::invalid_argument("expected {\"iid\": 1} or {\"level_counts\": [15 counts], \"depth_cqi\": x, "
+                                "\"coherence_rbgs\": x, \"coherence_reports\": x}");
+  }
+  return ch;
+}
+
+/* The channel file `path` (format: header comment) for the slice config of `pr`; returns its "report_ttis". */
+int load_channel(const std::string& path, Profile* pr) {
+  const std::string text = read_file(path, "channel");
+  const Json t = Parser(text).value();
+  const std::string where = "channel file " + path + ": ";
+  const Json& groups = t["slices"];
+  if (groups.kind != Json::Arr) throw std::runtime_error(where + "\"slices\" must be a list");
+  const Json& rep = t["report_ttis"];
+  int report = 1;
+  if (rep.kind != Json::Null) {
+    if (rep.kind != Json::Num || !(rep.num >= 1 && rep.num <= 2147483647.0) || rep.num != std::floor(rep.num))
+      throw std::runtime_error(where + "\"report_ttis\" must be an integer 1..2147483647");
+    report = (int)rep.num;
+  }
+  if (groups.arr.size() != pr->groups.size())
+    throw std::runtime_error(where + std::to_string(groups.arr.size()) + " entries in \"slices\", the slice config has " +
+                             std::to_string(pr->groups.size()) + " slice groups");
+  for (size_t g = 0; g < groups.arr.size(); ++g) {
+    rs_channel ch;
+    try {
+      ch = parse_channel(groups.arr[g]);
+    } catch (const std::invalid_argument& e) {
+      throw std::runtime_error(where + "slices[" + std::to_string(g) + "]: " + e.what());
+    }
+    pr->chn.insert(pr->chn.end(), (size_t)pr->groups[g], ch);
+  }
+  return report;
+}
+
 constexpr int R = 512, RBG = 8, G = R / RBG;   /* 100 MHz: bandwidth-manager.cpp:98-102, eesm-effective-sinr.h:82-103 */
 
 /* Cells [cell0, cell0 + nb) of the batch on GPU `gpu`.  comm != NULL: join the end-of-run reduce (root = rank 0). */
@@ -321,6 +394,13 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
         }
     check(rs_set_sources(h, src.data()), "rs_set_sources");
   }
+  const bool channel = !a.channel.empty();
+  if (channel) {
+    std::vector<rs_channel> chn;   /* [P][S]: profile p of the handle is config p */
+    for (const Profile& pr : su.prof) chn.insert(chn.end(), pr.chn.begin(), pr.chn.end());
+    check(rs_set_channels(h, chn.data()), "rs_set_channels");
+  }
+  const int rep = su.report;
 
   /* ---- run in blocks of TB TTIs with everything resident on the device ------------------------------- */
   const int TB = 16;
@@ -371,9 +451,17 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
     }
   }
   std::vector<int32_t> trow(TB);
-  for (int t0 = 0; t0 < T; t0 += TB) {
-    const int n = std::min(TB, T - t0);
-    if (!replay) check(rs_synth_cqi(h, a.seed, cell0, t0, n, d_cqi), "rs_synth_cqi");
+  for (int t0 = 0, n = 0; t0 < T; t0 += n) {
+    n = std::min(TB, T - t0);
+    /* rs_run_device reads slab t / rep from the start of the call: a chunk that starts between two reports ends at the
+     * next one, so every chunk starts on a report or lies within one */
+    if (t0 % rep) n = std::min(n, rep - t0 % rep);
+    if (channel) {
+      /* the reports of TTIs t0 .. t0 + n - 1, one slab each */
+      check(rs_synth_channel(h, a.seed, cell0, t0 / rep, (t0 + n - 1) / rep - t0 / rep + 1, d_cqi), "rs_synth_channel");
+    } else if (!replay) {
+      check(rs_synth_cqi(h, a.seed, cell0, t0, n, d_cqi), "rs_synth_cqi");
+    }
     if (n_draws > 0) check(rs_synth_rand2(h, a.seed, cell0, t0, n, d_draws), "rs_synth_rand2");
     if (buffered) {
       /* counter-based draws over global cells: N GPUs draw exactly the arrivals one GPU would */
@@ -388,7 +476,7 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
       for (int k = 0; k < n; ++k) trow[k] = rs_trace_row(su.now[(t0 + k) - (t0 + k) % 40], n_rows);
       check(rs_run_traces_device(h, n, trow.data(), d_draws, nullptr, 0, su.dt.data() + t0, want_log ? &out : nullptr, TB), "rs_run_traces_device");
     } else {
-      check(rs_run_device(h, n, d_cqi, (int64_t)B * U * row, 1, d_draws, nullptr, 0, su.dt.data() + t0, want_log ? &out : nullptr, TB), "rs_run_device");
+      check(rs_run_device(h, n, d_cqi, (int64_t)B * U * row, rep, d_draws, nullptr, 0, su.dt.data() + t0, want_log ? &out : nullptr, TB), "rs_run_device");
     }
     check(rs_sync(h), "rs_sync");
     res->ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - w0).count();
@@ -406,7 +494,9 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
             }
           }
         } else {
-          cu(cudaMemcpy(h_cqi.data(), d_cqi + tb * U * row, (size_t)U * row, cudaMemcpyDeviceToHost), "copy");
+          /* the slab TTI t0 + k read */
+          const size_t sb = (size_t)((t0 + k) / rep - t0 / rep) * B + lc;
+          cu(cudaMemcpy(h_cqi.data(), d_cqi + sb * U * row, (size_t)U * row, cudaMemcpyDeviceToHost), "copy");
         }
         cu(cudaMemcpy(h_rbg.data(), d_rbg + tb * G, sizeof(int16_t) * G, cudaMemcpyDeviceToHost), "copy");
         cu(cudaMemcpy(h_bits.data(), d_bits + tb * U, sizeof(int32_t) * U, cudaMemcpyDeviceToHost), "copy");
@@ -482,11 +572,13 @@ int main(int argc, char** argv) {
       else if (k == "--gpus") a.gpus = atoi(next().c_str());
       else if (k == "--buffers") a.buffers = atoi(next().c_str());
       else if (k == "--traffic") a.traffic.push_back(next());
+      else if (k == "--channel") a.channel.push_back(next());
       else throw std::runtime_error("unknown argument " + k);
     }
     if (a.configs.empty() || a.cells < 1 || a.ttis < 1 || a.trace_rows < 1 || a.gpus < 1 || a.gpus > a.cells) {
       fprintf(stderr, "usage: rs_batch --algo ID --config cfg.json [--config cfg2.json ...] --cells B --ttis T [--seed s] [--gpus N] "
-                      "[--traces DIR --mapping FILE [--trace-rows N]] [--log-cell b --log-prefix P] [--buffers K --traffic FILE ...]\n");
+                      "[--traces DIR --mapping FILE [--trace-rows N]] [--log-cell b --log-prefix P] [--buffers K --traffic FILE ...] "
+                      "[--channel FILE ...]\n");
       return 2;
     }
     if (a.buffers != -1 && (a.buffers < 1 || a.buffers > RS_MAX_BUFFER_RECORDS))
@@ -495,6 +587,10 @@ int main(int argc, char** argv) {
     if (a.buffers < 0 && !a.traffic.empty()) throw std::runtime_error("--traffic needs --buffers K");
     if (!a.traffic.empty() && a.traffic.size() != 1 && a.traffic.size() != a.configs.size())
       throw std::runtime_error(std::to_string(a.traffic.size()) + " --traffic files for " + std::to_string(a.configs.size()) +
+                               " --config files: give one for all or one per config");
+    if (!a.channel.empty() && !a.traces.empty()) throw std::runtime_error("--channel and --traces both give the CQI: use one");
+    if (!a.channel.empty() && a.channel.size() != 1 && a.channel.size() != a.configs.size())
+      throw std::runtime_error(std::to_string(a.channel.size()) + " --channel files for " + std::to_string(a.configs.size()) +
                                " --config files: give one for all or one per config");
     /* ---- the slice configs, expanded like the scheduler constructors do -------------------------------- */
     for (const std::string& path : a.configs) {
@@ -531,6 +627,13 @@ int main(int argc, char** argv) {
           throw std::runtime_error("traffic files with \"bearers\" " + std::to_string(su.nb) + " and " + std::to_string(nb) +
                                    " (every config of a batch must have the same)");
         su.nb = nb;
+      }
+      if (!a.channel.empty()) {
+        const int report = load_channel(a.channel[a.channel.size() == 1 ? 0 : su.prof.size()], &pr);
+        if (!su.prof.empty() && report != su.report)
+          throw std::runtime_error("channel files with \"report_ttis\" " + std::to_string(su.report) + " and " +
+                                   std::to_string(report) + " (every config of a batch must have the same)");
+        su.report = report;
       }
       su.prof.push_back(std::move(pr));
     }

@@ -40,6 +40,7 @@ ABI_SYMBOLS = (
     "rs_enable_buffers", "rs_set_traffic", "rs_get_buffers", "rs_synth_arrivals",
     "rs_buffer_stats_device", "rs_get_buffer_stats", "rs_arrival_spec",
     "rs_set_sources", "rs_synth_traffic", "rs_onoff_spec",
+    "rs_set_channels", "rs_synth_channel", "rs_channel_spec",
 )
 
 
@@ -83,7 +84,13 @@ class _Source(C.Structure):
                 ("frame_bytes", C.c_void_p)]
 
 
+class _Channel(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("level_thr", C.c_uint32 * 14), ("depth_q8", C.c_int32),
+                ("coherence_rbgs", C.c_int32), ("coherence_epochs", C.c_int32)]
+
+
 SRC_NONE, SRC_RATE, SRC_PERIODIC, SRC_ONOFF = 0, 1, 2, 3   # rs_source.kind (RS_SRC_*)
+CH_IID, CH_FADING = 0, 1                                   # rs_channel.kind (RS_CH_*)
 MAX_FRAMES = 1024                                          # RS_MAX_FRAMES
 INT32_MAX = 2147483647
 
@@ -186,6 +193,9 @@ def lib():
         L.rs_set_sources.argtypes = [C.c_void_p, C.POINTER(_Source)]
         L.rs_synth_traffic.argtypes = [C.c_void_p, C.c_uint64, C.c_int64, C.c_int64, C.c_int32, C.c_void_p]
         L.rs_onoff_spec.argtypes = [C.c_double, C.c_double, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]
+        L.rs_set_channels.argtypes = [C.c_void_p, C.POINTER(_Channel)]
+        L.rs_synth_channel.argtypes = [C.c_void_p, C.c_uint64, C.c_int64, C.c_int64, C.c_int32, C.c_void_p]
+        L.rs_channel_spec.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_double, C.POINTER(_Channel)]
         _lib = L
     return _lib
 
@@ -326,6 +336,76 @@ def load_traffic_config(path: str, config_path: str):
     pkt = [s.get("pkt_bytes", 0) for s in sources]
     q16 = [s.get("pkts_q16", 0) for s in sources]
     return nb, backlogged, np.asarray(pkt, np.int32), np.asarray(q16, np.int32)
+
+
+def channel_spec(level_counts, depth_cqi, coherence_rbgs, coherence_epochs):
+    """A FADING channel dict for :meth:`Scheduler.set_channels` / :func:`workload.synth_channel` from the counts of
+    levels 1..15, the offset's standard deviation in CQI steps and its coherence lengths in RBGs and epochs (0 = flat /
+    frozen), converted as ``rs_channel_spec`` converts them (host only).  ValueError on a value it refuses."""
+    counts = np.ascontiguousarray(level_counts, dtype=np.float64)
+    if counts.shape != (15,):
+        raise ValueError(f"level_counts: {counts.size} values, expected 15")
+    ch = _Channel()
+    if lib().rs_channel_spec(_ptr(counts), float(depth_cqi), float(coherence_rbgs), float(coherence_epochs),
+                             C.byref(ch)) != 0:
+        raise ValueError(lib().rs_last_error().decode())
+    return {"kind": CH_FADING, "level_thr": [int(v) for v in ch.level_thr], "depth_q8": int(ch.depth_q8),
+            "coherence_rbgs": int(ch.coherence_rbgs), "coherence_epochs": int(ch.coherence_epochs)}
+
+
+_CHANNEL_FORMS = ('{"iid": 1} or {"level_counts": [15 counts], "depth_cqi": x, "coherence_rbgs": x, '
+                  '"coherence_reports": x}')
+
+
+def _channel(e):
+    """One entry of a channel file's "slices" -> a channel dict; ValueError in the words rs_batch uses."""
+    num = lambda v: isinstance(v, (int, float)) and not isinstance(v, bool)   # noqa: E731
+    keys = set(e) if isinstance(e, dict) else None
+    if keys == {"iid"} and num(e["iid"]):
+        if e["iid"] != 1:
+            raise ValueError('"iid" must be 1')
+        return {"kind": CH_IID}
+    if (keys == {"level_counts", "depth_cqi", "coherence_rbgs", "coherence_reports"}
+            and isinstance(e["level_counts"], list) and len(e["level_counts"]) == 15
+            and all(num(v) for v in e["level_counts"])
+            and all(num(e[k]) for k in ("depth_cqi", "coherence_rbgs", "coherence_reports"))):
+        return channel_spec(e["level_counts"], e["depth_cqi"], e["coherence_rbgs"], e["coherence_reports"])
+    raise ValueError("expected " + _CHANNEL_FORMS)
+
+
+def load_channel(path: str, config_path: str):
+    """Read a channel file (the format of ``rs_batch --channel``) for the slice config at ``config_path``.
+
+    ``{"report_ttis": R, "slices": [...]}``: CQI reports fall on the TTIs that are multiples of R (default 1; 40 is the
+    reference's CQI_INTERVAL), and epoch e of the channel is the report at TTI e * R.  ``slices`` has one entry per entry
+    of the config's ``slices``, in the same order, applying to each of its ``n_slices`` slices: ``{"iid": 1}`` (exactly
+    :func:`workload.synth_cqi`) or ``{"level_counts": [15 counts], "depth_cqi": x, "coherence_rbgs": x,
+    "coherence_reports": x}`` (FADING, :func:`channel_spec`; the time coherence is counted in reports).  Other keys
+    (such as ``"note"``) are not read.  Returns (report_ttis, channels: [S] dicts for :meth:`Scheduler.set_channels` /
+    :func:`workload.synth_channel`); ValueError names what is wrong, in the words of rs_batch."""
+    with open(config_path) as f:
+        groups = [int(g["n_slices"]) for g in json.load(f)["slices"]]
+    with open(path) as f:
+        t = json.load(f)
+    where = f"channel file {path}: "
+    entries = t.get("slices") if isinstance(t, dict) else None
+    if not isinstance(entries, list):
+        raise ValueError(where + '"slices" must be a list')
+    rep = t.get("report_ttis")
+    if rep is None:   # absent or null: one report per TTI, as rs_batch reads it
+        rep = 1
+    if isinstance(rep, bool) or not isinstance(rep, (int, float)) or not (1 <= rep <= INT32_MAX) or rep != int(rep):
+        raise ValueError(where + f'"report_ttis" must be an integer 1..{INT32_MAX}')
+    if len(entries) != len(groups):
+        raise ValueError(where + f'{len(entries)} entries in "slices", the slice config has {len(groups)} slice groups')
+    channels = []
+    for g, e in enumerate(entries):
+        try:
+            ch = _channel(e)
+        except ValueError as err:
+            raise ValueError(where + f"slices[{g}]: " + str(err)) from None
+        channels += [ch] * groups[g]
+    return int(rep), channels
 
 
 class Scheduler:
@@ -549,6 +629,24 @@ class Scheduler:
         """rs_synth_traffic: int32 [n_ttis][B][U][nb] of the sources into device memory; a call continues the on-off
         chains of the previous one (tti0 = its tti0 + n_ttis).  Twin of workload.synth_traffic."""
         _check(lib().rs_synth_traffic(self._h, int(seed), int(cell0), int(tti0), int(n_ttis), C.c_void_p(d_out)))
+
+    def set_channels(self, channels):
+        """rs_set_channels: the synthetic channel of every slice, [S] dicts or [P][S] (one list per profile), with the
+        fields of rs_channel (see :func:`workload.synth_channel`; :func:`channel_spec` and :func:`load_channel` make
+        them)."""
+        rows = [list(channels)] if isinstance(channels[0], dict) else [list(p) for p in channels]
+        if len(rows) != self.n_profiles or any(len(r) != self.S for r in rows):
+            raise ValueError(f"channels: expected [{self.n_profiles}][{self.S}]")
+        arr = (_Channel * (self.n_profiles * self.S))()
+        for i, e in enumerate(x for r in rows for x in r):
+            arr[i] = _Channel(int(e["kind"]), (C.c_uint32 * 14)(*[int(v) for v in e.get("level_thr", [0] * 14)]),
+                              int(e.get("depth_q8", 0)), int(e.get("coherence_rbgs", 0)), int(e.get("coherence_epochs", 0)))
+        _check(lib().rs_set_channels(self._h, arr))
+
+    def synth_channel(self, seed, cell0, epoch0, n_slabs, d_out):
+        """rs_synth_channel: n_slabs CQI slabs [B][U][row] of the channels (epochs epoch0..) into device memory, in the
+        handle's CQI layout.  Twin of workload.synth_channel (+ pack_cqi for layout 2)."""
+        _check(lib().rs_synth_channel(self._h, int(seed), int(cell0), int(epoch0), int(n_slabs), C.c_void_p(d_out)))
 
     def _per_bearer(self, lead):
         return lead + ((self.U,) if self.nb == 1 else (self.U, 2))

@@ -240,3 +240,95 @@ def synth_traffic(seed: int, cell0: int, n_cells: int, tti0: int, n_ttis: int, u
                 arr[t] = np.where(onoff, np.where(on & aligned[t], pkt, 0), arr[t])
     out, st = arr.astype(np.int32), on.astype(np.uint8)
     return (out, st) if nb == 2 else (out[..., 0], st[..., 0])
+
+
+DOMAIN_CHANNEL = 0x43484E00  # "CHN\0"
+CH_IID, CH_FADING = 0, 1
+N_PATHS = 8
+_FOLD = np.uint64(0xD6E8FEB86659FD93)
+_M32 = np.uint64(0xFFFFFFFF)
+
+
+def cos_q14() -> np.ndarray:
+    """int16 [1024]: round(16384 cos(2 pi i / 1024)), the channel's cosine table (include/rs_cos_q14.inc is written
+    from this by tools/gen_cos_table.py)."""
+    i = np.arange(1024, dtype=np.float64)
+    return np.round(16384.0 * np.cos(2.0 * np.pi * i / 1024.0)).astype(np.int16)
+
+
+def _slope(raw, coherence):
+    """uint64 phase slopes uniform over [-W, W] mod 2^32, W = floor(2^31 / coherence) (0 for coherence 0)."""
+    coh = np.asarray(coherence, dtype=np.int64)
+    w = np.where(coh > 0, (1 << 31) // np.maximum(coh, 1), 0).astype(np.uint64)
+    return (((raw * (np.uint64(2) * w + np.uint64(1))) >> np.uint64(32)) - w) & _M32
+
+
+def _channel_paths(seed, cell0, n_cells, n_ues, coherence_rbgs, coherence_epochs):
+    """The per-(cell, UE) draws of a FADING channel: level draw uint64 [B][U] and theta, omega, nu uint64 [B][U][8]."""
+    key = _key(seed, DOMAIN_CHANNEL)
+    cell = np.arange(cell0, cell0 + n_cells, dtype=np.uint64)[:, None, None]
+    ue = np.arange(n_ues, dtype=np.uint64)[None, :, None]
+    idx = np.arange(1 + 2 * N_PATHS, dtype=np.uint64)[None, None, :]
+    with np.errstate(over="ignore"):
+        ctr = (cell << np.uint64(20)) ^ (ue << np.uint64(8)) ^ idx ^ ((ue >> np.uint64(12)) * _FOLD)
+        h = splitmix64(ctr ^ key)                                 # [B][U][17]
+    hi, lo = h >> np.uint64(32), h & _M32
+    shape = (n_cells, n_ues, 1)
+    omega = _slope(lo[..., 1:1 + N_PATHS], np.broadcast_to(np.asarray(coherence_rbgs), (n_cells, n_ues)).reshape(shape))
+    nu = _slope(hi[..., 1 + N_PATHS:], np.broadcast_to(np.asarray(coherence_epochs), (n_cells, n_ues)).reshape(shape))
+    return hi[..., 0], hi[..., 1:1 + N_PATHS], omega, nu
+
+
+def _offset_sum(theta, omega, nu, epoch0, n_epochs, n_rbgs):
+    tab = cos_q14().astype(np.int64)
+    g = np.arange(n_rbgs, dtype=np.uint64)
+    e = (np.arange(epoch0, epoch0 + n_epochs, dtype=np.int64) & 0xFFFFFFFF).astype(np.uint64)[:, None, None, None]
+    x = np.zeros((n_epochs,) + theta.shape[:2] + (n_rbgs,), dtype=np.int64)
+    for k in range(N_PATHS):
+        ph = (theta[None, :, :, k, None] + g * omega[None, :, :, k, None] + e * nu[None, :, :, k, None]) & _M32
+        x += tab[(ph >> np.uint64(22)).astype(np.intp)]
+    return x
+
+
+def channel_offset_sum(seed, cell0, n_cells, epoch0, n_epochs, n_ues, n_rbgs, coherence_rbgs, coherence_epochs):
+    """int64 [E][B][U][G]: the FADING channel's sum x of eight Q14 cosines before depth, rounding and clamping (standard
+    deviation 2^15; autocorrelation sinc(pi dg / coherence_rbgs) x sinc(pi de / coherence_epochs)).  The coherences are
+    scalars or [B][U]; x does not depend on the level or the depth.  For the statistical tests."""
+    _, th, om, nu = _channel_paths(seed, cell0, n_cells, n_ues, coherence_rbgs, coherence_epochs)
+    return _offset_sum(th, om, nu, epoch0, n_epochs, n_rbgs)
+
+
+def synth_channel(seed: int, cell0: int, n_cells: int, epoch0: int, n_epochs: int, ue_to_slice, channels,
+                  cell_profile=None, n_rbgs: int = 64) -> np.ndarray:
+    """uint8 [n_epochs][n_cells][U][n_rbgs], values 1..15: the synthetic channel's CQI of epochs epoch0.. (one value per
+    RBG; :func:`radiosaber_b200.sched.pack_cqi` gives layout 2).  ``rs_set_channels`` + ``rs_synth_channel`` is the
+    device twin, bit for bit.
+
+    channels: one dict per slice ([S]), or one list per slice profile ([P][S]), with the fields of ``rs_channel``:
+    ``kind`` (CH_IID / CH_FADING) and, for FADING, ``level_thr`` (14 ints), ``depth_q8``, ``coherence_rbgs``,
+    ``coherence_epochs`` (``sched.channel_spec`` makes them).  ue_to_slice [U] or [P][U]; cell b uses row
+    cell_profile[b].  The rules are those of include/rs_sched.h: IID is :func:`synth_cqi` itself; FADING is
+    clamp(L + ((x * depth_q8 + 2^22) >> 23), 1, 15) with the per-UE level L and x of :func:`channel_offset_sum`."""
+    rows = [list(channels)] if isinstance(channels[0], dict) else [list(p) for p in channels]
+    u2s = np.atleast_2d(np.asarray(ue_to_slice, dtype=np.int64))
+    U = u2s.shape[1]
+    cp = np.zeros(n_cells, dtype=np.int64) if cell_profile is None else np.asarray(cell_profile, dtype=np.int64)
+
+    def per_ue(a):   # [P][S](...) -> [B][U](...)
+        return a[cp[:, None], u2s[cp]]
+
+    def field(name):
+        return np.array([[int(e.get(name, 0)) for e in r] for r in rows], dtype=np.int64)
+
+    out = synth_cqi(seed, cell0, n_cells, epoch0, n_epochs, U, n_rbgs)
+    fading = per_ue(field("kind")) == CH_FADING
+    if not fading.any():
+        return out
+    thr = per_ue(np.array([[list(e.get("level_thr", [0] * 14)) for e in r] for r in rows], dtype=np.int64))
+    lv, th, om, nu = _channel_paths(seed, cell0, n_cells, U, per_ue(field("coherence_rbgs")),
+                                    per_ue(field("coherence_epochs")))
+    level = 1 + (lv.astype(np.int64)[..., None] >= thr).sum(axis=-1)                    # [B][U]
+    x = _offset_sum(th, om, nu, epoch0, n_epochs, n_rbgs)
+    off = (x * per_ue(field("depth_q8"))[None, :, :, None] + (1 << 22)) >> 23
+    cqi = np.clip(level[None, :, :, None] + off, 1, 15)
+    return np.where(fading[None, :, :, None], cqi, out).astype(np.uint8)
