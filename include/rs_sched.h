@@ -259,6 +259,37 @@ int rs_get_buffers(rs_handle* h, int64_t* queued, int32_t* n_records, double* he
 int rs_buffer_stats_device(rs_handle* h, uint64_t* d_stats);
 int rs_get_buffer_stats(rs_handle* h, uint64_t* stats);
 
+/* ---- head-of-line delay histograms of a buffered handle ---------------------------------------------
+ * With the histogram on, every TTI of every run call (rs_step, rs_run_host(_async), rs_run_device,
+ * rs_run_traces_host(_async), rs_run_traces_device) adds samples; the caller changes nothing else.  Only bearers with
+ * a FIFO count (backlogged bearers add nothing, as in rs_get_buffer_stats).  With q the queue and h the HoL delay step 2
+ * showed the scheduler at that TTI (what queue_out / hol_out receive):
+ *   row 0, served   one sample per bearer that sends this TTI, by the rule of rs_log_tti's stderr loop (the reference's
+ *                   DoStopSchedule lines): avail = tbs_bits[u] / 8; slots from priority nb-1 down to 0; a slot with
+ *                   q <= 0 is skipped (ids other than 1); sent = min(avail, q) (id 1: avail), avail -= sent; the loop
+ *                   stops when avail <= 0.  These are the samples of the reference's hol_delay lines, for every cell.
+ *   row 1, waiting  one sample per bearer with q > 0, served or not: the time-average view, starved bearers included.
+ *   bin             d = floor(h * bins_per_unit + 0.5), a product and a sum each rounded to double (no FMA), then
+ *                   min(d, n_bins - 1): the last bin holds every delay of at least n_bins - 1 bins.  With a clock in
+ *                   seconds, bins_per_unit = 1000 makes 1-TTI bins.
+ *   storage         uint64 [P][2][S][n_bins]; row p sums the cells of profile p, mapped to slices by that profile's
+ *                   ue_to_slice, as rs_stats_device does.  Integers, so any order of accumulation gives the same bits.
+ * The counts come from a reduction kernel launched after each TTI-kernel launch on the same stream; the schedules,
+ * state and buffers are the same bits with the histogram on and off.
+ *
+ * rs_enable_hol_hist: n_bins 1..RS_MAX_HOL_BINS, or 0 to switch the histogram off and free it; bins_per_unit finite
+ * and > 0.  RS_ERR_ARG on a handle without buffers, with 2^30 or more UEs (B x U), or with a [P][2][S][n_bins] block
+ * over 2 GiB.  Enabling (again) zeroes the counts, and only that does (rs_reset_state leaves them); rs_enable_buffers
+ * (again, or with 0) switches the histogram off.  Synchronous.  rs_hol_hist_bins: n_bins, 0 when off.
+ * rs_hol_hist_device writes DEVICE memory (P x 2 x S x n_bins uint64; feed it to an NCCL reduce, rs_reduce_hol_hist);
+ * rs_get_hol_hist copies to HOST.  Both are ordered after the handle's earlier work on its stream, like
+ * rs_buffer_stats_device; RS_ERR_ARG on a handle without the histogram. */
+#define RS_MAX_HOL_BINS 65536
+int rs_enable_hol_hist(rs_handle* h, int32_t n_bins, double bins_per_unit);
+int32_t rs_hol_hist_bins(const rs_handle* h);
+int rs_hol_hist_device(rs_handle* h, uint64_t* d_hist);
+int rs_get_hol_hist(rs_handle* h, uint64_t* hist);
+
 /* Synthetic arrivals into DEVICE int32 [n_ttis][B][U][nb] (bit-identical twin of radiosaber_b200/workload.py
  * synth_arrivals): pkt_bytes and pkts_q16 are HOST int32 [P][S] (P = rs_n_profiles; cell b reads the row of its
  * profile).  A bearer of slice s gets (q >> 16) + (draw16 < (q & 0xffff)) packets of pkt_bytes[s] bytes per TTI with

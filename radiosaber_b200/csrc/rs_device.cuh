@@ -2607,6 +2607,74 @@ __global__ void rs_buffer_stats_kernel(const BufMeta* meta, const DevCfg d, unsi
   }
 }
 
+/* ---- head-of-line delay histograms: uint64 [P][2][S][n_bins] += the samples of one TTI-kernel launch ---- */
+/* (rs_enable_hol_hist, include/rs_sched.h.)  Grid (x, T): TTI blockIdx.y, one thread per (cell, UE) of cells
+ * [cell_lo, cell_lo + n_cells); queue / hol [T][B][U][nb] and tbs_bits [T][B][U] as that launch wrote them (B = the
+ * handle's cells).  Row 0 books the bearers rs_log_tti's stderr loop prints (the bytes of tbs_bits / 8 go from slot
+ * nb-1 down, a slot with an empty queue skipped except for id 1, until none are left), row 1 every bearer with bytes
+ * queued; bearers without a FIFO add nothing.  Bins below smem_bins count in 32-bit shared counters [P][2][S][smem_bins]
+ * (native shared atomics), flushed once per CTA; the others are summed over the warp's lanes with the same (row, bin)
+ * and added to global memory.  A 32-bit counter holds a CTA's samples: the host keeps B x U below 2^30. */
+__device__ __forceinline__ void hol_hist_add(unsigned* s_cnt, unsigned long long* hist, int row, int bin, int n_bins,
+                                             int smem_bins) {
+  const bool global = row >= 0 && bin >= smem_bins;
+  if (row >= 0 && !global) atomicAdd(&s_cnt[row * smem_bins + bin], 1u);
+  if (__any_sync(0xffffffffu, global)) {   /* long delays: rare, so the match runs only when a lane has one */
+    const int key = global ? row * n_bins + bin : -1;
+    const unsigned same = __match_any_sync(0xffffffffu, key);
+    if (global && (threadIdx.x & 31) == __ffs(same) - 1) atomicAdd(&hist[key], (unsigned long long)__popc(same));
+  }
+}
+
+__global__ void rs_hol_hist_kernel(const int* queue, const double* hol, const int* tbs_bits, const BufMeta* meta,
+                                   const DevCfg d, int n_batch, int cell_lo, int n_cells, int n_bins,
+                                   double bins_per_unit, unsigned long long* hist, int n_profiles, int smem_bins) {
+  extern __shared__ unsigned s_cnt[];   /* [P][2][S][smem_bins] */
+  const int S = d.S, U = d.U, nb = d.nb, t = blockIdx.y;
+  const int n_smem = n_profiles * 2 * S * smem_bins;
+  for (int i = threadIdx.x; i < n_smem; i += blockDim.x) s_cnt[i] = 0;
+  __syncthreads();
+  const unsigned per_tti = (unsigned)n_cells * (unsigned)U, stride = gridDim.x * blockDim.x;
+  /* warp-uniform trip count: every lane takes part in the warp votes of every round */
+  for (unsigned base = blockIdx.x * blockDim.x; base < per_tti; base += stride) {
+    const unsigned r = base + threadIdx.x;
+    const bool valid = r < per_tti;
+    int b = cell_lo, u = 0, avail = 0, row0 = -1;
+    size_t tbu = 0;
+    if (valid) {
+      b = cell_lo + (int)(r / (unsigned)U);
+      u = (int)(r % (unsigned)U);
+      tbu = ((size_t)t * n_batch + b) * U + u;
+      avail = tbs_bits[tbu] / 8;
+      const int pf = d.cell_profile ? d.cell_profile[b] : 0;
+      row0 = pf * 2 * S + d.ue_to_slice[(size_t)pf * U + u];   /* [pf][0][s]; row 1 is S rows on */
+    }
+    for (int k = nb - 1; k >= 0; --k) {
+      int served_row = -1, waiting_row = -1, bin = 0;
+      if (valid) {
+        const size_t at = tbu * nb + k;
+        const int q = queue[at];
+        bool served = false;
+        if (avail > 0 && (d.algo == 1 || q > 0)) {
+          avail -= d.algo == 1 ? avail : min(avail, q);
+          served = true;
+        }
+        if (meta[((size_t)b * U + u) * nb + k].n >= 0) {   /* the bearer has a FIFO */
+          const double x = floor(__dadd_rn(__dmul_rn(hol[at], bins_per_unit), 0.5));
+          bin = x < (double)(n_bins - 1) ? (int)x : n_bins - 1;
+          if (served) served_row = row0;
+          if (q > 0) waiting_row = row0 + S;
+        }
+      }
+      hol_hist_add(s_cnt, hist, served_row, bin, n_bins, smem_bins);
+      hol_hist_add(s_cnt, hist, waiting_row, bin, n_bins, smem_bins);
+    }
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < n_smem; i += blockDim.x)
+    if (s_cnt[i]) atomicAdd(&hist[(size_t)(i / smem_bins) * n_bins + i % smem_bins], (unsigned long long)s_cnt[i]);
+}
+
 #endif  /* RS_CORE_ONLY */
 
 }  // namespace RS_NS

@@ -1,7 +1,8 @@
-/* rs_nccl.cpp -- include/rs_sched_nccl.h: the end-of-run NCCL reduce of the per-slice totals (SURVEY 8e), and
- * include/rs_sched_nccl_buffers.h: the same for the per-slice buffer totals.
+/* rs_nccl.cpp -- include/rs_sched_nccl.h: the end-of-run NCCL reduce of the per-slice totals (SURVEY 8e),
+ * include/rs_sched_nccl_buffers.h: the same for the per-slice buffer totals, and include/rs_sched_nccl_hol_hist.h: the
+ * same for the head-of-line delay histograms.
  * Uses only the public ABI of librs_sched.so plus NCCL and the CUDA runtime. */
-#include "../../include/rs_sched_nccl_buffers.h"
+#include "../../include/rs_sched_nccl_hol_hist.h"
 
 #include <cuda_runtime.h>
 #include <nccl.h>
@@ -102,6 +103,13 @@ int rs_reduce_stats(rs_handle* h, void* nccl_comm, int32_t root, uint64_t* stats
 int rs_reduce_buffer_stats(rs_handle* h, void* nccl_comm, int32_t root, uint64_t* stats_out) {
   return reduce_totals(h, nccl_comm, root, stats_out, 3, rs_buffer_stats_device, "rs_reduce_buffer_stats",
                        "rs_buffer_stats_device");
+}
+
+int rs_reduce_hol_hist(rs_handle* h, void* nccl_comm, int32_t root, uint64_t* hist_out) {
+  const int32_t bins = rs_hol_hist_bins(h);   /* [P][2][S][bins]: 2 x bins rows per slice */
+  if (h && bins == 0) return nfail("rs_hol_hist_device", "the handle has no delay histogram (rs_enable_hol_hist)");
+  return reduce_totals(h, nccl_comm, root, hist_out, 2 * bins, rs_hol_hist_device, "rs_reduce_hol_hist",
+                       "rs_hol_hist_device");
 }
 
 }  /* extern "C" */

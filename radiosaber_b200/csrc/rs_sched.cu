@@ -290,6 +290,12 @@ struct rs_handle {
   DevBuf<short> cos_q14;                       /* include/rs_cos_q14.inc */
   bool chn_set = false;
   DevBuf<unsigned char> buf_scratch;           /* rs_get_buffers */
+  /* head-of-line delay histograms (rs_enable_hol_hist): [P][2][S][hist_bins], 0 bins = off */
+  int hist_bins = 0;
+  int hist_ctas = 0;                           /* reducer CTAs per launch: four per SM */
+  double hist_per_unit = 0;
+  DevBuf<unsigned long long> hist;
+  DevBuf<int> hist_tbs;                        /* rs_run_device without tbs_bits: one launch's worth for the reducer */
   DevBuf<int> tbs1;
   DevBuf<short> vogel_tab;
   DevBuf<unsigned long long> stats;
@@ -363,6 +369,13 @@ const void* fixed_kernel(int algo, int which, bool trace) {
   return (algo == 7 || algo == 11) ? rs_kernel_tu6(algo, which, trace) : rs_kernel_tu5(algo, which, trace);
 }
 
+/* Bins of the delay histograms counted per CTA in 32-bit shared counters: the first 64 (where the samples of one slice
+ * crowd), fewer when the default 48 KB cannot hold 64 for every (profile, row, slice), 0 = all straight to global. */
+int hist_smem_bins(const rs_handle* h) {
+  const size_t rows = (size_t)2 * h->d.S * h->P;
+  return (int)std::min<size_t>({(size_t)h->hist_bins, 64, 48 * 1024 / sizeof(unsigned) / rows});
+}
+
 /* part < 0: the whole batch on the handle's stream; part p of h->parts: cells [p B / P, (p + 1) B / P) on stream / xs[p-1] */
 int launch_ttis(rs_handle* h, const rs::RunArgs& a0, bool trace, const rs::DevCfg* cfg = nullptr, int part = -1) {
   rs::RunArgs a = a0;
@@ -384,6 +397,17 @@ int launch_ttis(rs_handle* h, const rs::RunArgs& a0, bool trace, const rs::DevCf
   CU(cudaLaunchKernel(fn, grid, block, args, sm, st));
   CU(cudaGetLastError());
   h->launches++;
+  if (h->hist_bins > 0 && a.buf_k > 0) {   /* the histogram reads what this launch wrote, on the same stream */
+    const int smem_bins = hist_smem_bins(h);
+    const size_t per_tti = (size_t)n * h->d.U;   /* below 2^30 (rs_enable_hol_hist) */
+    /* one grid row per TTI; about four CTAs per SM over the whole grid */
+    const dim3 hgrid((unsigned)std::min<size_t>((per_tti + 255) / 256, std::max(1, (h->hist_ctas + a.T - 1) / a.T)), a.T);
+    rs::rs_hol_hist_kernel<<<hgrid, 256, sizeof(unsigned) * 2 * h->d.S * h->P * smem_bins, st>>>(
+        a.queue, a.hol, a.tbs_bits, h->buf_meta.p, h->d, h->B, a.cell_off, n, h->hist_bins, h->hist_per_unit, h->hist.p,
+        h->P, smem_bins);
+    CU(cudaGetLastError());
+    h->launches++;
+  }
   return RS_OK;
 }
 
@@ -567,7 +591,7 @@ void rs_destroy(rs_handle* h) {
   h->trace_tab.release(); h->ue_trace_off.release();
   h->holmul.release(); h->tbs1.release(); h->vogel_tab.release();
   h->buf_meta.release(); h->buf_time.release(); h->buf_bytes.release(); h->shown_q.release(); h->shown_hol.release();
-  h->synth_spec.release(); h->buf_scratch.release();
+  h->synth_spec.release(); h->buf_scratch.release(); h->hist.release(); h->hist_tbs.release();
   h->src_tab.release(); h->src_frames.release(); h->src_state.release();
   h->chn_tab.release(); h->cos_q14.release();
   if (h->own_stream) cudaStreamDestroy(h->own_stream);
@@ -1070,6 +1094,8 @@ int run_device_impl(rs_handle* h, int32_t n_ttis, const uint8_t* d_cqi, int64_t 
     const size_t per_launch = (size_t)std::min(ttis_per_launch, n_ttis) * B * U * h->d.nb;
     if (tr.queue_out) d_queue = tr.queue_out; else { CU(h->shown_q.alloc(per_launch)); d_queue = h->shown_q.p; q_tti = 0; }
     if (tr.hol_out) d_hol = tr.hol_out; else { CU(h->shown_hol.alloc(per_launch)); d_hol = h->shown_hol.p; h_tti = 0; }
+    /* the delay histograms read each TTI's tbs_bits: scratch of one launch when the caller does not ask for them */
+    if (h->hist_bins > 0 && !(d_out && d_out->tbs_bits)) CU(h->hist_tbs.alloc(per_launch / h->d.nb));
   }
   /* more than one launch in this call and a big batch: the two halves of the batch go down two streams (forked
    * here, joined at the end of the call), so the tail of one launch overlaps the head of the next */
@@ -1098,6 +1124,7 @@ int run_device_impl(rs_handle* h, int32_t n_ttis, const uint8_t* d_cqi, int64_t 
     }
     a.stage = h->stage_ok && (trace_row || ((((uintptr_t)d_cqi) & 15) == 0 && (cqi_tti_stride & 15) == 0)) ? 1 : 0;
     point_outputs(h, &a, d_out, (size_t)t0);
+    if (h->hist_bins > 0 && !a.tbs_bits) a.tbs_bits = h->hist_tbs.p;   /* launches reuse it, as shown_q */
     int rc = launch_ttis(h, a, trace_row != nullptr, nullptr, split ? 0 : -1);
     for (int q = 1; q < P && rc == RS_OK; ++q) rc = launch_ttis(h, a, trace_row != nullptr, nullptr, q);
     if (rc != RS_OK) { for (auto st : h->xs) cudaStreamSynchronize(st); return rc; }
@@ -1148,6 +1175,7 @@ int run_host_impl(rs_handle* h, int32_t n_ttis, const uint8_t* cqi, int32_t cqi_
     const int rc = alloc_slot(h, s, TC, out, active != nullptr, !trace_row && !slabs, queue != nullptr || buffered,
                               hol != nullptr || buffered, buffered);
     if (rc != RS_OK) { drain(h); return rc; }
+    if (h->hist_bins > 0) CU_DRAIN(s.tbs_bits.alloc((size_t)TC * B * h->d.U));   /* the delay histograms read it */
   }
   if (slabs)
     for (auto& sl : h->slab) {
@@ -1232,6 +1260,7 @@ int run_host_impl(rs_handle* h, int32_t n_ttis, const uint8_t* cqi, int32_t cqi_
       so.alloc_rbg = out->alloc_rbg ? s.alloc_rbg.p : nullptr;
       point_outputs(h, &a, &so, 0);
     }
+    if (h->hist_bins > 0 && !a.tbs_bits) a.tbs_bits = s.tbs_bits.p;
     int rc = launch_ttis(h, a, trace_row != nullptr, nullptr, split ? 0 : -1);
     for (int q = 1; q < P && rc == RS_OK; ++q) rc = launch_ttis(h, a, trace_row != nullptr, nullptr, q);
     if (rc != RS_OK) { drain(h); return rc; }
@@ -1248,7 +1277,7 @@ int run_host_impl(rs_handle* h, int32_t n_ttis, const uint8_t* cqi, int32_t cqi_
     for (int q = 1; q < P; ++q) CU_DRAIN(cudaStreamWaitEvent(h->copy_out, s.k_done_x[q - 1], 0));
     if (out) {
       if (a.rbg_to_ue) CU_DRAIN(cudaMemcpyAsync(out->rbg_to_ue + (size_t)t0 * B * G, s.rbg_to_ue.p, (size_t)T * B * G * 2, cudaMemcpyDeviceToHost, h->copy_out));
-      if (a.tbs_bits) CU_DRAIN(cudaMemcpyAsync(out->tbs_bits + (size_t)t0 * B * U, s.tbs_bits.p, (size_t)T * B * U * 4, cudaMemcpyDeviceToHost, h->copy_out));
+      if (so.tbs_bits) CU_DRAIN(cudaMemcpyAsync(out->tbs_bits + (size_t)t0 * B * U, s.tbs_bits.p, (size_t)T * B * U * 4, cudaMemcpyDeviceToHost, h->copy_out));
       if (a.mcs) CU_DRAIN(cudaMemcpyAsync(out->mcs + (size_t)t0 * B * U, s.mcs.p, (size_t)T * B * U, cudaMemcpyDeviceToHost, h->copy_out));
       if (a.final_cqi) CU_DRAIN(cudaMemcpyAsync(out->final_cqi + (size_t)t0 * B * U, s.final_cqi.p, (size_t)T * B * U, cudaMemcpyDeviceToHost, h->copy_out));
       if (a.slice_target) CU_DRAIN(cudaMemcpyAsync(out->slice_target + (size_t)t0 * B * S, s.slice_target.p, (size_t)T * B * S * 4, cudaMemcpyDeviceToHost, h->copy_out));
@@ -1654,6 +1683,8 @@ int rs_enable_buffers(rs_handle* h, int32_t max_records, const uint8_t* backlogg
   h->buf_k = 0;
   h->buf_meta.release(); h->buf_time.release(); h->buf_bytes.release(); h->shown_q.release(); h->shown_hol.release();
   h->buf_backlogged.clear();
+  h->hist_bins = 0;   /* the histogram is of the buffers: it goes with them */
+  h->hist.release(); h->hist_tbs.release();
   h->last_now = -HUGE_VAL;
   if (max_records == 0) return RS_OK;
   const size_t n = (size_t)h->B * h->d.U * h->d.nb;
@@ -2044,6 +2075,56 @@ int rs_get_buffer_stats(rs_handle* h, uint64_t* stats) {
   int rc = rs_buffer_stats_device(h, (uint64_t*)h->stats.p);   /* [P][3][S] fits the [P][4][S] scratch */
   if (rc != RS_OK) return rc;
   CU(cudaMemcpyAsync(stats, h->stats.p, sizeof(uint64_t) * 3 * h->d.S * h->P, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  return RS_OK;
+}
+
+int rs_enable_hol_hist(rs_handle* h, int32_t n_bins, double bins_per_unit) {
+  if (!h) return fail(RS_ERR_ARG, "null handle");
+  if (n_bins < 0 || n_bins > RS_MAX_HOL_BINS)
+    return fail(RS_ERR_ARG, "rs_enable_hol_hist: n_bins %d outside 0..%d", n_bins, RS_MAX_HOL_BINS);
+  if (n_bins > 0 && h->buf_k == 0)
+    return fail(RS_ERR_ARG, "rs_enable_hol_hist: the handle has no buffers (rs_enable_buffers)");
+  if (n_bins > 0 && !(std::isfinite(bins_per_unit) && bins_per_unit > 0))
+    return fail(RS_ERR_ARG, "rs_enable_hol_hist: bins_per_unit %g is not finite and > 0", bins_per_unit);
+  if (n_bins > 0 && (size_t)h->B * h->d.U >= ((size_t)1 << 30))
+    return fail(RS_ERR_ARG, "rs_enable_hol_hist: %d cells x %d UEs: the histogram takes fewer than 2^30 UEs", h->B, h->d.U);
+  const size_t words = (size_t)h->P * 2 * h->d.S * (size_t)n_bins;
+  if (words * sizeof(uint64_t) > ((size_t)2 << 30))
+    return fail(RS_ERR_ARG, "rs_enable_hol_hist: %d profiles x 2 x %d slices x %d bins of uint64 exceed 2 GiB", h->P, h->d.S,
+                n_bins);
+  const int rc = rs_sync(h);   /* the launches in flight add to the old counts */
+  if (rc != RS_OK) return rc;
+  h->hist_bins = 0;
+  h->hist.release(); h->hist_tbs.release();
+  if (n_bins == 0) return RS_OK;
+  int sms = 0;
+  CU(cudaSetDevice(h->device));
+  CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device));
+  CU(h->hist.alloc(words));
+  CU(cudaMemsetAsync(h->hist.p, 0, words * sizeof(uint64_t), h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  h->hist_ctas = 4 * sms;
+  h->hist_bins = n_bins;
+  h->hist_per_unit = bins_per_unit;
+  return RS_OK;
+}
+
+int32_t rs_hol_hist_bins(const rs_handle* h) { return h ? h->hist_bins : 0; }
+
+int rs_hol_hist_device(rs_handle* h, uint64_t* d_hist) {
+  if (!h || !d_hist) return fail(RS_ERR_ARG, "rs_hol_hist_device: bad argument");
+  if (h->hist_bins == 0) return fail(RS_ERR_ARG, "rs_hol_hist_device: the handle has no delay histogram (rs_enable_hol_hist)");
+  CU(cudaSetDevice(h->device));
+  CU(cudaMemcpyAsync(d_hist, h->hist.p, sizeof(uint64_t) * h->hist.n, cudaMemcpyDeviceToDevice, h->stream));
+  return RS_OK;
+}
+
+int rs_get_hol_hist(rs_handle* h, uint64_t* hist) {
+  if (!h || !hist) return fail(RS_ERR_ARG, "rs_get_hol_hist: bad argument");
+  if (h->hist_bins == 0) return fail(RS_ERR_ARG, "rs_get_hol_hist: the handle has no delay histogram (rs_enable_hol_hist)");
+  CU(cudaSetDevice(h->device));
+  CU(cudaMemcpyAsync(hist, h->hist.p, sizeof(uint64_t) * h->hist.n, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
   return RS_OK;
 }

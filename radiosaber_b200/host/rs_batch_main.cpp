@@ -25,6 +25,11 @@
  *                                               once for every config or once per --config
  *                                               (file p with config p); every line gains the per-slice queued_bytes,
  *                                               dropped_bytes and records left at the end
+ *            [--hol-bins N]                     with --buffers: head-of-line delay histograms of N 1-TTI bins counted on
+ *                                               the device (rs_enable_hol_hist, one rs_reduce_hol_hist with --gpus N);
+ *                                               every line gains per slice the samples of the bearers that sent
+ *                                               (hol_served) and of those with bytes queued (hol_waiting), and their
+ *                                               50th, 95th and 99th percentiles as bin indices (null without samples)
  *            [--channel FILE ...]               synthetic channel CQI drawn on the device (rs_set_channels,
  *                                               rs_synth_channel) in place of rs_synth_cqi's i.i.d. draws, the file named
  *                                               once for every config or once per --config; not with --traces
@@ -81,7 +86,7 @@
 
 #include "rs_sched.h"
 #include "rs_sched_nccl.h"
-#include "rs_sched_nccl_buffers.h"
+#include "rs_sched_nccl_hol_hist.h"
 
 namespace {
 
@@ -162,6 +167,7 @@ struct Args {
   int algo = 9, cells = 4096, ttis = 1000, log_cell = -1, trace_rows = 475;   /* 475 lines: enb-mac-entity.cc:181 */
   int gpus = 1;
   int buffers = -1;                  /* --buffers K; -1 = backlogged bearers only, as without the flag */
+  int hol_bins = 0;                  /* --hol-bins N; 0 = no delay histograms */
   uint64_t seed = 1;
   std::vector<std::string> configs, traffic, channel;
   std::string traces, mapping, log_prefix;
@@ -195,6 +201,7 @@ struct ShardResult {
   double ms = 0;                 /* host clock around the synchronised scheduling calls */
   std::vector<uint64_t> stats;   /* [P][4][S] of this shard's cells (single GPU) or of ALL cells (root after the reduce) */
   std::vector<uint64_t> buf_stats;   /* [P][3][S] (--buffers), the same way */
+  std::vector<uint64_t> hol_hist;    /* [P][2][S][hol_bins] (--hol-bins), the same way */
   std::string log_out, log_err, error;
 };
 
@@ -393,6 +400,7 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
           if (src.back().kind == RS_SRC_PERIODIC) src.back().frame_bytes = pr.frames[g].data();
         }
     check(rs_set_sources(h, src.data()), "rs_set_sources");
+    if (a.hol_bins > 0) check(rs_enable_hol_hist(h, a.hol_bins, 1000.0), "rs_enable_hol_hist");   /* the clock is in s */
   }
   const bool channel = !a.channel.empty();
   if (channel) {
@@ -539,6 +547,15 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
       check(rs_get_buffer_stats(h, res->buf_stats.data()), "rs_get_buffer_stats");
     }
   }
+  if (a.hol_bins > 0) {
+    res->hol_hist.assign((size_t)2 * S * P * a.hol_bins, 0);
+    if (comm) {
+      if (rs_reduce_hol_hist(h, comm, 0, res->hol_hist.data()) != RS_OK)
+        throw std::runtime_error(std::string("rs_reduce_hol_hist: ") + rs_nccl_last_error());
+    } else {
+      check(rs_get_hol_hist(h, res->hol_hist.data()), "rs_get_hol_hist");
+    }
+  }
   (void)rank;
   if (lg) {
     res->log_out = rs_log_stdout(lg, nullptr);
@@ -573,18 +590,22 @@ int main(int argc, char** argv) {
       else if (k == "--buffers") a.buffers = atoi(next().c_str());
       else if (k == "--traffic") a.traffic.push_back(next());
       else if (k == "--channel") a.channel.push_back(next());
+      else if (k == "--hol-bins") a.hol_bins = atoi(next().c_str());
       else throw std::runtime_error("unknown argument " + k);
     }
     if (a.configs.empty() || a.cells < 1 || a.ttis < 1 || a.trace_rows < 1 || a.gpus < 1 || a.gpus > a.cells) {
       fprintf(stderr, "usage: rs_batch --algo ID --config cfg.json [--config cfg2.json ...] --cells B --ttis T [--seed s] [--gpus N] "
                       "[--traces DIR --mapping FILE [--trace-rows N]] [--log-cell b --log-prefix P] [--buffers K --traffic FILE ...] "
-                      "[--channel FILE ...]\n");
+                      "[--channel FILE ...] [--hol-bins N]\n");
       return 2;
     }
     if (a.buffers != -1 && (a.buffers < 1 || a.buffers > RS_MAX_BUFFER_RECORDS))
       throw std::runtime_error("--buffers K: K records per bearer, 1.." + std::to_string(RS_MAX_BUFFER_RECORDS));
     if (a.buffers > 0 && a.traffic.empty()) throw std::runtime_error("--buffers needs --traffic FILE");
     if (a.buffers < 0 && !a.traffic.empty()) throw std::runtime_error("--traffic needs --buffers K");
+    if (a.hol_bins != 0 && (a.hol_bins < 1 || a.hol_bins > RS_MAX_HOL_BINS))
+      throw std::runtime_error("--hol-bins N: N bins of one TTI, 1.." + std::to_string(RS_MAX_HOL_BINS));
+    if (a.hol_bins > 0 && a.buffers < 0) throw std::runtime_error("--hol-bins needs --buffers K");
     if (!a.traffic.empty() && a.traffic.size() != 1 && a.traffic.size() != a.configs.size())
       throw std::runtime_error(std::to_string(a.traffic.size()) + " --traffic files for " + std::to_string(a.configs.size()) +
                                " --config files: give one for all or one per config");
@@ -726,6 +747,34 @@ int main(int argc, char** argv) {
         for (int k = 0; k < 3; ++k) {
           printf("], \"%s\": [", names[k]);
           for (int s = 0; s < S; ++s) printf("%s%llu", s ? ", " : "", (unsigned long long)bs[(size_t)k * S + s]);
+        }
+      }
+      if (a.hol_bins > 0) {   /* per slice: samples, and percentiles as bin indices (sched.hist_percentile's rule) */
+        const size_t nbins = (size_t)a.hol_bins;
+        const char* rows[2] = {"hol_served", "hol_waiting"};
+        for (int r = 0; r < 2; ++r) {
+          const uint64_t* hr = res[0].hol_hist.data() + ((size_t)p * 2 + r) * S * nbins;
+          printf("], \"%s\": [", rows[r]);
+          for (int s = 0; s < S; ++s) {
+            uint64_t n = 0;
+            for (size_t d = 0; d < nbins; ++d) n += hr[(size_t)s * nbins + d];
+            printf("%s%llu", s ? ", " : "", (unsigned long long)n);
+          }
+          for (int q : {50, 95, 99}) {
+            printf("], \"%s_p%d\": [", rows[r], q);
+            for (int s = 0; s < S; ++s) {
+              const uint64_t* hs = hr + (size_t)s * nbins;
+              uint64_t n = 0, cum = 0;
+              for (size_t d = 0; d < nbins; ++d) n += hs[d];
+              size_t d = 0;
+              for (; n > 0 && d < nbins; ++d) {   /* the smallest bin with 100 x cum >= q x n */
+                cum += hs[d];
+                if (100 * cum >= (uint64_t)q * n) break;
+              }
+              if (n == 0) printf("%snull", s ? ", " : "");
+              else printf("%s%zu", s ? ", " : "", d);
+            }
+          }
         }
       }
       printf("]}\n");

@@ -41,6 +41,7 @@ ABI_SYMBOLS = (
     "rs_buffer_stats_device", "rs_get_buffer_stats", "rs_arrival_spec",
     "rs_set_sources", "rs_synth_traffic", "rs_onoff_spec",
     "rs_set_channels", "rs_synth_channel", "rs_channel_spec",
+    "rs_enable_hol_hist", "rs_hol_hist_bins", "rs_hol_hist_device", "rs_get_hol_hist",
 )
 
 
@@ -196,6 +197,11 @@ def lib():
         L.rs_set_channels.argtypes = [C.c_void_p, C.POINTER(_Channel)]
         L.rs_synth_channel.argtypes = [C.c_void_p, C.c_uint64, C.c_int64, C.c_int64, C.c_int32, C.c_void_p]
         L.rs_channel_spec.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_double, C.POINTER(_Channel)]
+        L.rs_enable_hol_hist.argtypes = [C.c_void_p, C.c_int32, C.c_double]
+        L.rs_hol_hist_bins.argtypes = [C.c_void_p]
+        L.rs_hol_hist_bins.restype = C.c_int32
+        L.rs_hol_hist_device.argtypes = [C.c_void_p, C.c_void_p]
+        L.rs_get_hol_hist.argtypes = [C.c_void_p, C.c_void_p]
         _lib = L
     return _lib
 
@@ -600,6 +606,23 @@ class Scheduler:
         """rs_buffer_stats_device into a DEVICE buffer of n_profiles * 3 * S uint64."""
         _check(lib().rs_buffer_stats_device(self._h, C.c_void_p(d_stats)))
 
+    def enable_hol_hist(self, n_bins, bins_per_unit=1000.0):
+        """Count head-of-line delay histograms in every run call of this buffered handle (rs_enable_hol_hist; 0 = off):
+        row 0 the bearers that send, row 1 those with bytes queued; bin = floor(delay * bins_per_unit + 0.5), the last
+        bin holding everything from n_bins - 1 up.  Zeroes the counts.  Twin: workload.hol_hist."""
+        _check(lib().rs_enable_hol_hist(self._h, int(n_bins), float(bins_per_unit)))
+
+    def get_hol_hist(self):
+        """uint64 [P][2][S][n_bins]: the delay histograms counted since enable_hol_hist (rs_get_hol_hist)."""
+        n = int(lib().rs_hol_hist_bins(self._h))
+        hist = np.empty((self.n_profiles, 2, self.S, max(n, 1)), dtype=np.uint64)
+        _check(lib().rs_get_hol_hist(self._h, _ptr(hist)))
+        return hist
+
+    def hol_hist_device(self, d_hist):
+        """rs_hol_hist_device into a DEVICE buffer of n_profiles * 2 * S * n_bins uint64."""
+        _check(lib().rs_hol_hist_device(self._h, C.c_void_p(d_hist)))
+
     def synth_arrivals(self, seed, cell0, tti0, n_ttis, pkt_bytes, pkts_q16, d_out):
         """rs_synth_arrivals: int32 [n_ttis][B][U][nb] into device memory; pkt_bytes / pkts_q16: int [P][S] (packet
         size, packets per TTI in 16.16 fixed point) per slice of each profile.  Twin of workload.synth_arrivals."""
@@ -1002,6 +1025,24 @@ def test_sort_timed(keys, reps=20, depth_limit=-1, device=0):
     _check(lib().rs_test_sort_timed(int(device), _ptr(keys), keys.shape[0], keys.shape[1], int(depth_limit),
                                     _ptr(perm), int(reps), C.byref(ms)))
     return perm, float(ms.value)
+
+
+def hist_percentile(hist, q):
+    """The q-th percentile (an integer 0..100) of one histogram, as a bin index: the smallest bin d with
+    100 * (samples in bins 0..d) >= q * (all samples), in integers; None when it holds no samples.  rs_batch reports
+    its hol_*_p50 / p95 / p99 by the same rule."""
+    if isinstance(q, bool) or not isinstance(q, (int, np.integer)) or not 0 <= q <= 100:
+        raise ValueError(f"q = {q!r}: an integer percentile 0..100")
+    counts = [int(x) for x in np.asarray(hist).reshape(-1)]
+    n = sum(counts)
+    if n == 0:
+        return None
+    cum = 0
+    for d, c in enumerate(counts):
+        cum += c
+        if 100 * cum >= int(q) * n:
+            return d
+    raise AssertionError("unreachable: the last bin reaches every sample")
 
 
 def jain_index(stats: np.ndarray, n_ues_per_slice: np.ndarray) -> np.ndarray:

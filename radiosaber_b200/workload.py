@@ -332,3 +332,41 @@ def synth_channel(seed: int, cell0: int, n_cells: int, epoch0: int, n_epochs: in
     off = (x * per_ue(field("depth_q8"))[None, :, :, None] + (1 << 22)) >> 23
     cqi = np.clip(level[None, :, :, None] + off, 1, 15)
     return np.where(fading[None, :, :, None], cqi, out).astype(np.uint8)
+
+
+def hol_hist(queue, hol, tbs_bits, algo: int, ue_to_slice, backlogged, n_slices: int, n_bins: int,
+             bins_per_unit: float = 1000.0, cell_profile=None) -> np.ndarray:
+    """uint64 [P][2][S][n_bins]: the head-of-line delay histograms a buffered handle counts with ``rs_enable_hol_hist``
+    (the device twin, bit for bit), from what a run showed and sent.
+
+    queue int32 / hol float64 [T][B][U] ([..][U][2] with two bearers): the run's queue_out / hol_out; tbs_bits int32
+    [T][B][U]; backlogged bool [B][U] ([B][U][2]): bearers without a FIFO, which add nothing; ue_to_slice [U] or [P][U]
+    and cell_profile [B] (None = profile 0): cell b counts in row cell_profile[b] with that profile's slices.
+    Row 0 books the bearers that send (``rs_log_tti``'s stderr rule: tbs_bits / 8 bytes go from slot nb-1 down, a slot
+    with queue <= 0 skipped except for id 1, until none are left), row 1 every bearer with queue > 0; the bin is
+    min(floor(hol * bins_per_unit + 0.5), n_bins - 1), the product and the sum each rounded (numpy does not fuse)."""
+    tbs = np.asarray(tbs_bits, dtype=np.int64)
+    T, B, U = tbs.shape
+    q = np.asarray(queue, dtype=np.int64).reshape(T, B, U, -1)
+    h = np.asarray(hol, dtype=np.float64).reshape(q.shape)
+    nb = q.shape[3]
+    fifo = ~np.asarray(backlogged, dtype=bool).reshape(B, U, nb)
+    u2s = np.atleast_2d(np.asarray(ue_to_slice, dtype=np.int64))
+    P, S = u2s.shape[0], int(n_slices)
+    cp = np.zeros(B, dtype=np.int64) if cell_profile is None else np.asarray(cell_profile, dtype=np.int64)
+    row0 = ((cp * 2)[:, None] * S + u2s[cp]) * n_bins              # [B][U]: [pf][0][s][0]
+    d = np.floor(h * float(bins_per_unit) + 0.5)
+    bins = np.minimum(d, n_bins - 1).astype(np.int64)
+    avail = tbs // 8
+    idx, keep = [], []
+    for k in range(nb - 1, -1, -1):
+        qk = q[..., k]
+        served = (avail > 0) & ((qk > 0) | (algo == 1))
+        avail = np.where(served, avail - (avail if algo == 1 else np.minimum(avail, qk)), avail)
+        at = row0[None] + bins[..., k]
+        idx += [at, at + S * n_bins]
+        keep += [served & fifo[None, :, :, k], (qk > 0) & fifo[None, :, :, k]]
+    idx = np.concatenate([x.reshape(-1) for x in idx])
+    keep = np.concatenate([x.reshape(-1) for x in keep])
+    out = np.bincount(idx[keep], minlength=P * 2 * S * n_bins)
+    return out.astype(np.uint64).reshape(P, 2, S, n_bins)
