@@ -290,6 +290,40 @@ int32_t rs_hol_hist_bins(const rs_handle* h);
 int rs_hol_hist_device(rs_handle* h, uint64_t* d_hist);
 int rs_get_hol_hist(rs_handle* h, uint64_t* hist);
 
+/* ---- per-UE throughput histograms over caller-closed windows (any handle) ---------------------------------------
+ * The spread of the bytes a slice's UEs receive, cell-edge tail included, summarised on the device window by window.
+ * Every handle: backlogged or buffered, any CQI source, every id.  The caller closes each window; integers throughout:
+ *   UE bytes        c(b,u) = sum of cum_bytes[b][u][i] over the UE's slots (one, or two with n_bearers = 2), mod 2^64.
+ *   snapshot        snap[b][u], uint64 [B][U] in device memory: each UE's c when its open window started.
+ *   closing         every UE of every cell adds one sample, backlogged, buffered, idle or inactive alike:
+ *                   d = c(b,u) - snap[b][u] (mod 2^64), bin = min(d / bin_bytes, n_bins - 1) (integer division: the
+ *                   last bin holds every UE with at least (n_bins - 1) x bin_bytes bytes), then snap[b][u] := c(b,u).
+ *                   Two closes with no TTI between them add a bin-0 sample per UE.
+ *   row             [p][s]: p = the cell's profile when the window closes (so rs_set_cell_profiles between windows moves
+ *                   later samples), s = that profile's ue_to_slice[u], as rs_stats_device maps them.
+ *   storage         uint64 [P][S][n_bins]; any order of accumulation gives the same bits.
+ *   restarts        rs_reset_state zeroes the counters and sets snap := 0; rs_set_state with a non-NULL cum_bytes sets
+ *                   snap := the new counters.  Nothing else moves the snapshot (run calls, rs_step_cell,
+ *                   rs_enable_buffers, rs_set_cell_profiles leave it).
+ * The schedules, state and buffers are the same bits with the histogram on and off: nothing runs per TTI.
+ *
+ * rs_enable_ue_rate_hist: n_bins 1..RS_MAX_UE_RATE_BINS, or 0 to switch the histogram off and free it; bin_bytes >= 1.
+ * RS_ERR_ARG with 2^30 or more UEs (B x U) or a [P][S][n_bins] block over 2 GiB (32-bit per-CTA counters and
+ * indices).  Synchronous: waits for the work in flight, zeroes the counts and takes the snapshot, the first window
+ * starting there (warm-up before it is not counted); enabling again does the same.
+ * rs_close_ue_rate_window: one kernel on the handle's stream, asynchronous, ordered after the handle's earlier work as
+ * rs_stats_device is (the join of a split batch's part streams, the kernels of an rs_run_host_async /
+ * rs_run_traces_host_async call not yet waited for).  rs_ue_rate_hist_bins: n_bins, 0 when off.
+ * rs_ue_rate_hist_device writes DEVICE memory (P x S x n_bins uint64; feed it to an NCCL reduce,
+ * rs_reduce_ue_rate_hist); rs_get_ue_rate_hist copies to HOST; both ordered like rs_hol_hist_device.  Every call but
+ * rs_enable_ue_rate_hist returns RS_ERR_ARG on a handle without the histogram. */
+#define RS_MAX_UE_RATE_BINS 65536
+int rs_enable_ue_rate_hist(rs_handle* h, int32_t n_bins, int64_t bin_bytes);
+int rs_close_ue_rate_window(rs_handle* h);
+int32_t rs_ue_rate_hist_bins(const rs_handle* h);
+int rs_ue_rate_hist_device(rs_handle* h, uint64_t* d_hist);
+int rs_get_ue_rate_hist(rs_handle* h, uint64_t* hist);
+
 /* Synthetic arrivals into DEVICE int32 [n_ttis][B][U][nb] (bit-identical twin of radiosaber_b200/workload.py
  * synth_arrivals): pkt_bytes and pkts_q16 are HOST int32 [P][S] (P = rs_n_profiles; cell b reads the row of its
  * profile).  A bearer of slice s gets (q >> 16) + (draw16 < (q & 0xffff)) packets of pkt_bytes[s] bytes per TTI with

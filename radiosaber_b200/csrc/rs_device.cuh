@@ -2675,6 +2675,41 @@ __global__ void rs_hol_hist_kernel(const int* queue, const double* hol, const in
     if (s_cnt[i]) atomicAdd(&hist[(size_t)(i / smem_bins) * n_bins + i % smem_bins], (unsigned long long)s_cnt[i]);
 }
 
+/* ---- per-UE throughput histograms: uint64 [P][S][n_bins] += one sample per UE of the batch, closing a window ---- */
+/* (rs_enable_ue_rate_hist, include/rs_sched.h.)  One thread per (cell, UE), grid-stride: c = the sum of the UE's nb
+ * cum_bytes, d = c - snap (mod 2^64), snap := c, bin = min(d / bin_bytes, n_bins - 1), into row [profile][slice] of
+ * the cell's profile now.  Counting as rs_hol_hist_kernel: bins below smem_bins in 32-bit shared counters [P][S][smem_bins]
+ * flushed once per CTA, the others through hol_hist_add's warp match.  B x U < 2^30 (the host): 32-bit indices. */
+__global__ void rs_ue_rate_hist_kernel(const DevCfg d, unsigned long long* snap, int n_bins,
+                                       unsigned long long bin_bytes, unsigned long long* hist, int n_profiles,
+                                       int smem_bins) {
+  extern __shared__ unsigned s_cnt[];   /* [P][S][smem_bins] */
+  const int S = d.S, U = d.U, nb = d.nb;
+  const int n_smem = n_profiles * S * smem_bins;
+  for (int i = threadIdx.x; i < n_smem; i += blockDim.x) s_cnt[i] = 0;
+  __syncthreads();
+  const unsigned total = (unsigned)d.n_cells * (unsigned)U, stride = gridDim.x * blockDim.x;
+  /* warp-uniform trip count: every lane takes part in the warp votes of every round */
+  for (unsigned base = blockIdx.x * blockDim.x; base < total; base += stride) {
+    const unsigned r = base + threadIdx.x;
+    int row = -1, bin = 0;
+    if (r < total) {
+      const unsigned long long* cb = d.cum_bytes + (size_t)r * nb;
+      const unsigned long long c = nb == 2 ? cb[0] + cb[1] : cb[0];
+      const unsigned long long q = (c - snap[r]) / bin_bytes;
+      snap[r] = c;
+      bin = q < (unsigned long long)(n_bins - 1) ? (int)q : n_bins - 1;
+      const int b = (int)(r / (unsigned)U), u = (int)(r % (unsigned)U);
+      const int pf = d.cell_profile ? d.cell_profile[b] : 0;
+      row = pf * S + d.ue_to_slice[(size_t)pf * U + u];
+    }
+    hol_hist_add(s_cnt, hist, row, bin, n_bins, smem_bins);
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < n_smem; i += blockDim.x)
+    if (s_cnt[i]) atomicAdd(&hist[(size_t)(i / smem_bins) * n_bins + i % smem_bins], (unsigned long long)s_cnt[i]);
+}
+
 #endif  /* RS_CORE_ONLY */
 
 }  // namespace RS_NS

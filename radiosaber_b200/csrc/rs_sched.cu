@@ -296,6 +296,11 @@ struct rs_handle {
   double hist_per_unit = 0;
   DevBuf<unsigned long long> hist;
   DevBuf<int> hist_tbs;                        /* rs_run_device without tbs_bits: one launch's worth for the reducer */
+  /* per-UE throughput histograms (rs_enable_ue_rate_hist): [P][S][rate_bins], 0 bins = off; rate_snap [B][U] holds
+   * each UE's bytes (its slots summed) when its open window started */
+  int rate_bins = 0;
+  unsigned long long rate_bin_bytes = 0;
+  DevBuf<unsigned long long> rate_hist, rate_snap;
   DevBuf<int> tbs1;
   DevBuf<short> vogel_tab;
   DevBuf<unsigned long long> stats;
@@ -369,11 +374,11 @@ const void* fixed_kernel(int algo, int which, bool trace) {
   return (algo == 7 || algo == 11) ? rs_kernel_tu6(algo, which, trace) : rs_kernel_tu5(algo, which, trace);
 }
 
-/* Bins of the delay histograms counted per CTA in 32-bit shared counters: the first 64 (where the samples of one slice
- * crowd), fewer when the default 48 KB cannot hold 64 for every (profile, row, slice), 0 = all straight to global. */
-int hist_smem_bins(const rs_handle* h) {
-  const size_t rows = (size_t)2 * h->d.S * h->P;
-  return (int)std::min<size_t>({(size_t)h->hist_bins, 64, 48 * 1024 / sizeof(unsigned) / rows});
+/* Bins of a histogram of `rows` rows of n_bins (the delay and the throughput histograms) counted per CTA in 32-bit
+ * shared counters: the first 64 (where the samples of one slice crowd), fewer when the default 48 KB cannot hold 64 for
+ * every row, 0 = all straight to global. */
+int hist_smem_bins(size_t rows, int n_bins) {
+  return (int)std::min<size_t>({(size_t)n_bins, 64, 48 * 1024 / sizeof(unsigned) / rows});
 }
 
 /* part < 0: the whole batch on the handle's stream; part p of h->parts: cells [p B / P, (p + 1) B / P) on stream / xs[p-1] */
@@ -398,7 +403,7 @@ int launch_ttis(rs_handle* h, const rs::RunArgs& a0, bool trace, const rs::DevCf
   CU(cudaGetLastError());
   h->launches++;
   if (h->hist_bins > 0 && a.buf_k > 0) {   /* the histogram reads what this launch wrote, on the same stream */
-    const int smem_bins = hist_smem_bins(h);
+    const int smem_bins = hist_smem_bins((size_t)2 * h->d.S * h->P, h->hist_bins);
     const size_t per_tti = (size_t)n * h->d.U;   /* below 2^30 (rs_enable_hol_hist) */
     /* one grid row per TTI; about four CTAs per SM over the whole grid */
     const dim3 hgrid((unsigned)std::min<size_t>((per_tti + 255) / 256, std::max(1, (h->hist_ctas + a.T - 1) / a.T)), a.T);
@@ -592,6 +597,7 @@ void rs_destroy(rs_handle* h) {
   h->holmul.release(); h->tbs1.release(); h->vogel_tab.release();
   h->buf_meta.release(); h->buf_time.release(); h->buf_bytes.release(); h->shown_q.release(); h->shown_hol.release();
   h->synth_spec.release(); h->buf_scratch.release(); h->hist.release(); h->hist_tbs.release();
+  h->rate_hist.release(); h->rate_snap.release();
   h->src_tab.release(); h->src_frames.release(); h->src_state.release();
   h->chn_tab.release(); h->cos_q14.release();
   if (h->own_stream) cudaStreamDestroy(h->own_stream);
@@ -961,6 +967,7 @@ int rs_reset_state(rs_handle* h) {
   CU(cudaMemcpy(h->avg.p, avg.data(), BU * 8, cudaMemcpyHostToDevice));
   CU(cudaMemset(h->tx.p, 0, BU * 4));
   CU(cudaMemset(h->cum_bytes.p, 0, BU * 8));
+  if (h->rate_bins > 0) CU(cudaMemset(h->rate_snap.p, 0, (size_t)h->B * h->d.U * 8));   /* the open window restarts */
   CU(cudaMemset(h->cum_rbs.p, 0, BU * 8));
   CU(cudaMemset(h->offset.p, 0, BS * 8));
   CU(cudaMemset(h->ewma.p, 0, BS * 8));
@@ -976,6 +983,12 @@ int rs_set_state(rs_handle* h, const double* avg_rate, const int32_t* tx_bytes, 
   if (avg_rate) CU(cudaMemcpy(h->avg.p, avg_rate, BU * 8, cudaMemcpyHostToDevice));
   if (tx_bytes) CU(cudaMemcpy(h->tx.p, tx_bytes, BU * 4, cudaMemcpyHostToDevice));
   if (cum_bytes) CU(cudaMemcpy(h->cum_bytes.p, cum_bytes, BU * 8, cudaMemcpyHostToDevice));
+  if (cum_bytes && h->rate_bins > 0) {   /* the open window restarts from the new counters: each UE's slots summed */
+    const int nb = h->d.nb;
+    std::vector<uint64_t> snap((size_t)h->B * h->d.U);
+    for (size_t i = 0; i < snap.size(); ++i) snap[i] = nb == 2 ? cum_bytes[2 * i] + cum_bytes[2 * i + 1] : cum_bytes[i];
+    CU(cudaMemcpy(h->rate_snap.p, snap.data(), snap.size() * 8, cudaMemcpyHostToDevice));
+  }
   if (cum_rbs) CU(cudaMemcpy(h->cum_rbs.p, cum_rbs, BU * 8, cudaMemcpyHostToDevice));
   if (slice_offset) CU(cudaMemcpy(h->offset.p, slice_offset, BS * 8, cudaMemcpyHostToDevice));
   if (nvs_ewma) CU(cudaMemcpy(h->ewma.p, nvs_ewma, BS * 8, cudaMemcpyHostToDevice));
@@ -2125,6 +2138,78 @@ int rs_get_hol_hist(rs_handle* h, uint64_t* hist) {
   if (h->hist_bins == 0) return fail(RS_ERR_ARG, "rs_get_hol_hist: the handle has no delay histogram (rs_enable_hol_hist)");
   CU(cudaSetDevice(h->device));
   CU(cudaMemcpyAsync(hist, h->hist.p, sizeof(uint64_t) * h->hist.n, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  return RS_OK;
+}
+
+int rs_enable_ue_rate_hist(rs_handle* h, int32_t n_bins, int64_t bin_bytes) {
+  if (!h) return fail(RS_ERR_ARG, "null handle");
+  if (n_bins < 0 || n_bins > RS_MAX_UE_RATE_BINS)
+    return fail(RS_ERR_ARG, "rs_enable_ue_rate_hist: n_bins %d outside 0..%d", n_bins, RS_MAX_UE_RATE_BINS);
+  if (n_bins > 0 && bin_bytes < 1)
+    return fail(RS_ERR_ARG, "rs_enable_ue_rate_hist: bin_bytes %lld is not >= 1", (long long)bin_bytes);
+  const size_t BU = (size_t)h->B * h->d.U;
+  if (n_bins > 0 && BU >= ((size_t)1 << 30))
+    return fail(RS_ERR_ARG, "rs_enable_ue_rate_hist: %d cells x %d UEs: the histogram takes fewer than 2^30 UEs", h->B,
+                h->d.U);
+  const size_t words = (size_t)h->P * h->d.S * (size_t)n_bins;
+  if (words * sizeof(uint64_t) > ((size_t)2 << 30))
+    return fail(RS_ERR_ARG, "rs_enable_ue_rate_hist: %d profiles x %d slices x %d bins of uint64 exceed 2 GiB", h->P,
+                h->d.S, n_bins);
+  const int rc = rs_sync(h);   /* the launches in flight move the counters the snapshot takes */
+  if (rc != RS_OK) return rc;
+  h->rate_bins = 0;
+  h->rate_hist.release(); h->rate_snap.release();
+  if (n_bins == 0) return RS_OK;
+  int sms = 0;
+  CU(cudaSetDevice(h->device));
+  CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device));
+  CU(h->rate_hist.alloc(words));
+  CU(h->rate_snap.alloc(BU));
+  h->hist_ctas = 4 * sms;
+  h->rate_bins = n_bins;
+  h->rate_bin_bytes = (unsigned long long)bin_bytes;
+  /* the snapshot: one window closed from snap = 0, whose samples are then cleared */
+  CU(cudaMemsetAsync(h->rate_snap.p, 0, BU * sizeof(uint64_t), h->stream));
+  const int rc2 = rs_close_ue_rate_window(h);
+  if (rc2 != RS_OK) return rc2;
+  CU(cudaMemsetAsync(h->rate_hist.p, 0, words * sizeof(uint64_t), h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  return RS_OK;
+}
+
+int rs_close_ue_rate_window(rs_handle* h) {
+  if (!h) return fail(RS_ERR_ARG, "null handle");
+  if (h->rate_bins == 0)
+    return fail(RS_ERR_ARG, "rs_close_ue_rate_window: the handle has no throughput histogram (rs_enable_ue_rate_hist)");
+  CU(cudaSetDevice(h->device));
+  const size_t rows = (size_t)h->P * h->d.S, BU = (size_t)h->B * h->d.U;   /* BU below 2^30 */
+  const int smem_bins = hist_smem_bins(rows, h->rate_bins);
+  const unsigned ctas = (unsigned)std::min<size_t>((BU + 255) / 256, (size_t)std::max(1, h->hist_ctas));
+  rs::rs_ue_rate_hist_kernel<<<ctas, 256, sizeof(unsigned) * rows * smem_bins, h->stream>>>(
+      h->d, h->rate_snap.p, h->rate_bins, h->rate_bin_bytes, h->rate_hist.p, h->P, smem_bins);
+  CU(cudaGetLastError());
+  h->launches++;
+  return RS_OK;
+}
+
+int32_t rs_ue_rate_hist_bins(const rs_handle* h) { return h ? h->rate_bins : 0; }
+
+int rs_ue_rate_hist_device(rs_handle* h, uint64_t* d_hist) {
+  if (!h || !d_hist) return fail(RS_ERR_ARG, "rs_ue_rate_hist_device: bad argument");
+  if (h->rate_bins == 0)
+    return fail(RS_ERR_ARG, "rs_ue_rate_hist_device: the handle has no throughput histogram (rs_enable_ue_rate_hist)");
+  CU(cudaSetDevice(h->device));
+  CU(cudaMemcpyAsync(d_hist, h->rate_hist.p, sizeof(uint64_t) * h->rate_hist.n, cudaMemcpyDeviceToDevice, h->stream));
+  return RS_OK;
+}
+
+int rs_get_ue_rate_hist(rs_handle* h, uint64_t* hist) {
+  if (!h || !hist) return fail(RS_ERR_ARG, "rs_get_ue_rate_hist: bad argument");
+  if (h->rate_bins == 0)
+    return fail(RS_ERR_ARG, "rs_get_ue_rate_hist: the handle has no throughput histogram (rs_enable_ue_rate_hist)");
+  CU(cudaSetDevice(h->device));
+  CU(cudaMemcpyAsync(hist, h->rate_hist.p, sizeof(uint64_t) * h->rate_hist.n, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
   return RS_OK;
 }

@@ -30,6 +30,13 @@
  *                                               every line gains per slice the samples of the bearers that sent
  *                                               (hol_served) and of those with bytes queued (hol_waiting), and their
  *                                               50th, 95th and 99th percentiles as bin indices (null without samples)
+ *            [--rate-window W --rate-bins N     per-UE throughput histograms counted on the device (rs_enable_ue_rate_hist;
+ *             --rate-bin-bytes X]               one rs_reduce_ue_rate_hist with --gpus N): every W TTIs (W divides T)
+ *                                               each UE adds the bytes it received in those W TTIs, in N bins of X bytes
+ *                                               (the last holds the rest); every line gains per slice the samples
+ *                                               (ue_rate_samples) and their 5th, 50th and 95th percentiles as bin
+ *                                               indices (ue_rate_p5 / p50 / p95, null without samples).  The three go
+ *                                               together
  *            [--channel FILE ...]               synthetic channel CQI drawn on the device (rs_set_channels,
  *                                               rs_synth_channel) in place of rs_synth_cqi's i.i.d. draws, the file named
  *                                               once for every config or once per --config; not with --traces
@@ -75,6 +82,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <fstream>
+#include <initializer_list>
 #include <map>
 #include <sstream>
 #include <stdexcept>
@@ -86,7 +94,7 @@
 
 #include "rs_sched.h"
 #include "rs_sched_nccl.h"
-#include "rs_sched_nccl_hol_hist.h"
+#include "rs_sched_nccl_ue_rate.h"
 
 namespace {
 
@@ -168,6 +176,9 @@ struct Args {
   int gpus = 1;
   int buffers = -1;                  /* --buffers K; -1 = backlogged bearers only, as without the flag */
   int hol_bins = 0;                  /* --hol-bins N; 0 = no delay histograms */
+  int rate_window = 0, rate_bins = 0;   /* --rate-window W --rate-bins N; 0 = no throughput histograms */
+  long long rate_bin_bytes = 0;         /* --rate-bin-bytes X */
+  int rate_given = 0;                   /* bits 1, 2, 4: which of the three flags were given */
   uint64_t seed = 1;
   std::vector<std::string> configs, traffic, channel;
   std::string traces, mapping, log_prefix;
@@ -202,6 +213,7 @@ struct ShardResult {
   std::vector<uint64_t> stats;   /* [P][4][S] of this shard's cells (single GPU) or of ALL cells (root after the reduce) */
   std::vector<uint64_t> buf_stats;   /* [P][3][S] (--buffers), the same way */
   std::vector<uint64_t> hol_hist;    /* [P][2][S][hol_bins] (--hol-bins), the same way */
+  std::vector<uint64_t> rate_hist;   /* [P][S][rate_bins] (--rate-window), the same way */
   std::string log_out, log_err, error;
 };
 
@@ -339,6 +351,34 @@ int load_channel(const std::string& path, Profile* pr) {
   return report;
 }
 
+/* The S histograms of nbins bins at hist, as lists of an output line (each opened by "], " like the line's others):
+ * "<samples>" the samples per slice, and "<prefix>_p<q>" for each q the q-th percentile per slice as a bin index, by
+ * sched.hist_percentile's rule (the smallest bin d with 100 x samples in 0..d >= q x samples; null without samples). */
+void print_hist(const char* samples, const char* prefix, const uint64_t* hist, int S, size_t nbins,
+                std::initializer_list<int> qs) {
+  printf("], \"%s\": [", samples);
+  for (int s = 0; s < S; ++s) {
+    uint64_t n = 0;
+    for (size_t d = 0; d < nbins; ++d) n += hist[(size_t)s * nbins + d];
+    printf("%s%llu", s ? ", " : "", (unsigned long long)n);
+  }
+  for (int q : qs) {
+    printf("], \"%s_p%d\": [", prefix, q);
+    for (int s = 0; s < S; ++s) {
+      const uint64_t* hs = hist + (size_t)s * nbins;
+      uint64_t n = 0, cum = 0;
+      for (size_t d = 0; d < nbins; ++d) n += hs[d];
+      size_t d = 0;
+      for (; n > 0 && d < nbins; ++d) {   /* the smallest bin with 100 x cum >= q x n */
+        cum += hs[d];
+        if (100 * cum >= (uint64_t)q * n) break;
+      }
+      if (n == 0) printf("%snull", s ? ", " : "");
+      else printf("%s%zu", s ? ", " : "", d);
+    }
+  }
+}
+
 constexpr int R = 512, RBG = 8, G = R / RBG;   /* 100 MHz: bandwidth-manager.cpp:98-102, eesm-effective-sinr.h:82-103 */
 
 /* Cells [cell0, cell0 + nb) of the batch on GPU `gpu`.  comm != NULL: join the end-of-run reduce (root = rank 0). */
@@ -409,6 +449,8 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
     check(rs_set_channels(h, chn.data()), "rs_set_channels");
   }
   const int rep = su.report;
+  const int W = a.rate_window;   /* 0 = no throughput histograms */
+  if (W > 0) check(rs_enable_ue_rate_hist(h, a.rate_bins, a.rate_bin_bytes), "rs_enable_ue_rate_hist");
 
   /* ---- run in blocks of TB TTIs with everything resident on the device ------------------------------- */
   const int TB = 16;
@@ -464,6 +506,7 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
     /* rs_run_device reads slab t / rep from the start of the call: a chunk that starts between two reports ends at the
      * next one, so every chunk starts on a report or lies within one */
     if (t0 % rep) n = std::min(n, rep - t0 % rep);
+    if (W > 0) n = std::min(n, W - t0 % W);   /* and a chunk that would cross a window's end ends there */
     if (channel) {
       /* the reports of TTIs t0 .. t0 + n - 1, one slab each */
       check(rs_synth_channel(h, a.seed, cell0, t0 / rep, (t0 + n - 1) / rep - t0 / rep + 1, d_cqi), "rs_synth_channel");
@@ -488,6 +531,7 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
     }
     check(rs_sync(h), "rs_sync");
     res->ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - w0).count();
+    if (W > 0 && (t0 + n) % W == 0) check(rs_close_ue_rate_window(h), "rs_close_ue_rate_window");
     if (want_log) {
       for (int k = 0; k < n; ++k) {
         const size_t tb = (size_t)k * B + lc;
@@ -556,6 +600,15 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
       check(rs_get_hol_hist(h, res->hol_hist.data()), "rs_get_hol_hist");
     }
   }
+  if (W > 0) {
+    res->rate_hist.assign((size_t)S * P * a.rate_bins, 0);
+    if (comm) {
+      if (rs_reduce_ue_rate_hist(h, comm, 0, res->rate_hist.data()) != RS_OK)
+        throw std::runtime_error(std::string("rs_reduce_ue_rate_hist: ") + rs_nccl_last_error());
+    } else {
+      check(rs_get_ue_rate_hist(h, res->rate_hist.data()), "rs_get_ue_rate_hist");
+    }
+  }
   (void)rank;
   if (lg) {
     res->log_out = rs_log_stdout(lg, nullptr);
@@ -591,12 +644,15 @@ int main(int argc, char** argv) {
       else if (k == "--traffic") a.traffic.push_back(next());
       else if (k == "--channel") a.channel.push_back(next());
       else if (k == "--hol-bins") a.hol_bins = atoi(next().c_str());
+      else if (k == "--rate-window") { a.rate_window = atoi(next().c_str()); a.rate_given |= 1; }
+      else if (k == "--rate-bins") { a.rate_bins = atoi(next().c_str()); a.rate_given |= 2; }
+      else if (k == "--rate-bin-bytes") { a.rate_bin_bytes = strtoll(next().c_str(), nullptr, 10); a.rate_given |= 4; }
       else throw std::runtime_error("unknown argument " + k);
     }
     if (a.configs.empty() || a.cells < 1 || a.ttis < 1 || a.trace_rows < 1 || a.gpus < 1 || a.gpus > a.cells) {
       fprintf(stderr, "usage: rs_batch --algo ID --config cfg.json [--config cfg2.json ...] --cells B --ttis T [--seed s] [--gpus N] "
                       "[--traces DIR --mapping FILE [--trace-rows N]] [--log-cell b --log-prefix P] [--buffers K --traffic FILE ...] "
-                      "[--channel FILE ...] [--hol-bins N]\n");
+                      "[--channel FILE ...] [--hol-bins N] [--rate-window W --rate-bins N --rate-bin-bytes X]\n");
       return 2;
     }
     if (a.buffers != -1 && (a.buffers < 1 || a.buffers > RS_MAX_BUFFER_RECORDS))
@@ -606,6 +662,13 @@ int main(int argc, char** argv) {
     if (a.hol_bins != 0 && (a.hol_bins < 1 || a.hol_bins > RS_MAX_HOL_BINS))
       throw std::runtime_error("--hol-bins N: N bins of one TTI, 1.." + std::to_string(RS_MAX_HOL_BINS));
     if (a.hol_bins > 0 && a.buffers < 0) throw std::runtime_error("--hol-bins needs --buffers K");
+    if (a.rate_given != 0 && a.rate_given != 7)
+      throw std::runtime_error("--rate-window W, --rate-bins N and --rate-bin-bytes X go together");
+    if (a.rate_given && (a.rate_window < 1 || a.ttis % a.rate_window))
+      throw std::runtime_error("--rate-window W: W TTIs per window, >= 1 and dividing --ttis " + std::to_string(a.ttis));
+    if (a.rate_given && (a.rate_bins < 1 || a.rate_bins > RS_MAX_UE_RATE_BINS))
+      throw std::runtime_error("--rate-bins N: N bins, 1.." + std::to_string(RS_MAX_UE_RATE_BINS));
+    if (a.rate_given && a.rate_bin_bytes < 1) throw std::runtime_error("--rate-bin-bytes X: X bytes per bin, >= 1");
     if (!a.traffic.empty() && a.traffic.size() != 1 && a.traffic.size() != a.configs.size())
       throw std::runtime_error(std::to_string(a.traffic.size()) + " --traffic files for " + std::to_string(a.configs.size()) +
                                " --config files: give one for all or one per config");
@@ -749,34 +812,15 @@ int main(int argc, char** argv) {
           for (int s = 0; s < S; ++s) printf("%s%llu", s ? ", " : "", (unsigned long long)bs[(size_t)k * S + s]);
         }
       }
-      if (a.hol_bins > 0) {   /* per slice: samples, and percentiles as bin indices (sched.hist_percentile's rule) */
+      if (a.hol_bins > 0) {   /* per slice: samples, and percentiles as bin indices */
         const size_t nbins = (size_t)a.hol_bins;
         const char* rows[2] = {"hol_served", "hol_waiting"};
-        for (int r = 0; r < 2; ++r) {
-          const uint64_t* hr = res[0].hol_hist.data() + ((size_t)p * 2 + r) * S * nbins;
-          printf("], \"%s\": [", rows[r]);
-          for (int s = 0; s < S; ++s) {
-            uint64_t n = 0;
-            for (size_t d = 0; d < nbins; ++d) n += hr[(size_t)s * nbins + d];
-            printf("%s%llu", s ? ", " : "", (unsigned long long)n);
-          }
-          for (int q : {50, 95, 99}) {
-            printf("], \"%s_p%d\": [", rows[r], q);
-            for (int s = 0; s < S; ++s) {
-              const uint64_t* hs = hr + (size_t)s * nbins;
-              uint64_t n = 0, cum = 0;
-              for (size_t d = 0; d < nbins; ++d) n += hs[d];
-              size_t d = 0;
-              for (; n > 0 && d < nbins; ++d) {   /* the smallest bin with 100 x cum >= q x n */
-                cum += hs[d];
-                if (100 * cum >= (uint64_t)q * n) break;
-              }
-              if (n == 0) printf("%snull", s ? ", " : "");
-              else printf("%s%zu", s ? ", " : "", d);
-            }
-          }
-        }
+        for (int r = 0; r < 2; ++r)
+          print_hist(rows[r], rows[r], res[0].hol_hist.data() + ((size_t)p * 2 + r) * S * nbins, S, nbins, {50, 95, 99});
       }
+      if (a.rate_window > 0)
+        print_hist("ue_rate_samples", "ue_rate", res[0].rate_hist.data() + (size_t)p * S * a.rate_bins, S,
+                   (size_t)a.rate_bins, {5, 50, 95});
       printf("]}\n");
     }
     for (int r = 0; r < N; ++r) {

@@ -42,6 +42,8 @@ ABI_SYMBOLS = (
     "rs_set_sources", "rs_synth_traffic", "rs_onoff_spec",
     "rs_set_channels", "rs_synth_channel", "rs_channel_spec",
     "rs_enable_hol_hist", "rs_hol_hist_bins", "rs_hol_hist_device", "rs_get_hol_hist",
+    "rs_enable_ue_rate_hist", "rs_close_ue_rate_window", "rs_ue_rate_hist_bins", "rs_ue_rate_hist_device",
+    "rs_get_ue_rate_hist",
 )
 
 
@@ -202,6 +204,12 @@ def lib():
         L.rs_hol_hist_bins.restype = C.c_int32
         L.rs_hol_hist_device.argtypes = [C.c_void_p, C.c_void_p]
         L.rs_get_hol_hist.argtypes = [C.c_void_p, C.c_void_p]
+        L.rs_enable_ue_rate_hist.argtypes = [C.c_void_p, C.c_int32, C.c_int64]
+        L.rs_close_ue_rate_window.argtypes = [C.c_void_p]
+        L.rs_ue_rate_hist_bins.argtypes = [C.c_void_p]
+        L.rs_ue_rate_hist_bins.restype = C.c_int32
+        L.rs_ue_rate_hist_device.argtypes = [C.c_void_p, C.c_void_p]
+        L.rs_get_ue_rate_hist.argtypes = [C.c_void_p, C.c_void_p]
         _lib = L
     return _lib
 
@@ -623,6 +631,29 @@ class Scheduler:
         """rs_hol_hist_device into a DEVICE buffer of n_profiles * 2 * S * n_bins uint64."""
         _check(lib().rs_hol_hist_device(self._h, C.c_void_p(d_hist)))
 
+    def enable_ue_rate_hist(self, n_bins, bin_bytes):
+        """Count per-UE throughput histograms over windows this caller closes (rs_enable_ue_rate_hist; 0 = off): each
+        close_ue_rate_window adds, for every UE, bin = min(bytes since the last close // bin_bytes, n_bins - 1) to
+        [profile][slice].  Waits for the work in flight, zeroes the counts and starts the first window here.
+        Twin: workload.ue_rate_hist."""
+        _check(lib().rs_enable_ue_rate_hist(self._h, int(n_bins), int(bin_bytes)))
+
+    def close_ue_rate_window(self):
+        """rs_close_ue_rate_window: one sample per UE, on the handle's stream after its earlier work (asynchronous)."""
+        _check(lib().rs_close_ue_rate_window(self._h))
+
+    def get_ue_rate_hist(self):
+        """uint64 [P][S][n_bins]: the throughput histograms of the windows closed since enable_ue_rate_hist
+        (rs_get_ue_rate_hist)."""
+        n = int(lib().rs_ue_rate_hist_bins(self._h))
+        hist = np.empty((self.n_profiles, self.S, max(n, 1)), dtype=np.uint64)
+        _check(lib().rs_get_ue_rate_hist(self._h, _ptr(hist)))
+        return hist
+
+    def ue_rate_hist_device(self, d_hist):
+        """rs_ue_rate_hist_device into a DEVICE buffer of n_profiles * S * n_bins uint64."""
+        _check(lib().rs_ue_rate_hist_device(self._h, C.c_void_p(d_hist)))
+
     def synth_arrivals(self, seed, cell0, tti0, n_ttis, pkt_bytes, pkts_q16, d_out):
         """rs_synth_arrivals: int32 [n_ttis][B][U][nb] into device memory; pkt_bytes / pkts_q16: int [P][S] (packet
         size, packets per TTI in 16.16 fixed point) per slice of each profile.  Twin of workload.synth_arrivals."""
@@ -1030,7 +1061,7 @@ def test_sort_timed(keys, reps=20, depth_limit=-1, device=0):
 def hist_percentile(hist, q):
     """The q-th percentile (an integer 0..100) of one histogram, as a bin index: the smallest bin d with
     100 * (samples in bins 0..d) >= q * (all samples), in integers; None when it holds no samples.  rs_batch reports
-    its hol_*_p50 / p95 / p99 by the same rule."""
+    its hol_*_p50 / p95 / p99 and ue_rate_p5 / p50 / p95 by the same rule."""
     if isinstance(q, bool) or not isinstance(q, (int, np.integer)) or not 0 <= q <= 100:
         raise ValueError(f"q = {q!r}: an integer percentile 0..100")
     counts = [int(x) for x in np.asarray(hist).reshape(-1)]

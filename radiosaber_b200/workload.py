@@ -370,3 +370,24 @@ def hol_hist(queue, hol, tbs_bits, algo: int, ue_to_slice, backlogged, n_slices:
     keep = np.concatenate([x.reshape(-1) for x in keep])
     out = np.bincount(idx[keep], minlength=P * 2 * S * n_bins)
     return out.astype(np.uint64).reshape(P, 2, S, n_bins)
+
+
+def ue_rate_hist(cum_start, cum_end, ue_to_slice, n_slices: int, n_bins: int, bin_bytes: int,
+                 cell_profile=None) -> np.ndarray:
+    """uint64 [P][S][n_bins]: the samples one ``rs_close_ue_rate_window`` adds (the device twin, bit for bit), from the
+    byte counters at the window's start and end.
+
+    cum_start / cum_end: uint64 [B][U] ([B][U][2] with two bearers), ``get_state()["cum_bytes"]``; ue_to_slice [U] or
+    [P][U] and cell_profile [B] (None = profile 0): the profiles at close time.  Per UE, c = the sum of its slots and
+    d = c_end - c_start, both mod 2^64; bin = min(d // bin_bytes, n_bins - 1), in exact integers."""
+    a = np.asarray(cum_start, dtype=np.uint64)
+    b = np.asarray(cum_end, dtype=np.uint64)
+    B, U = b.shape[:2]
+    with np.errstate(over="ignore"):   # uint64 arithmetic wraps, as on the device
+        d = b.reshape(B, U, -1).sum(axis=2, dtype=np.uint64) - a.reshape(B, U, -1).sum(axis=2, dtype=np.uint64)
+    bins = np.minimum(d // np.uint64(bin_bytes), np.uint64(n_bins - 1)).astype(np.int64)
+    u2s = np.atleast_2d(np.asarray(ue_to_slice, dtype=np.int64))
+    P, S = u2s.shape[0], int(n_slices)
+    cp = np.zeros(B, dtype=np.int64) if cell_profile is None else np.asarray(cell_profile, dtype=np.int64)
+    idx = ((cp[:, None] * S + u2s[cp]) * n_bins + bins).reshape(-1)
+    return np.bincount(idx, minlength=P * S * n_bins).astype(np.uint64).reshape(P, S, n_bins)
