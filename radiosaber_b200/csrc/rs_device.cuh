@@ -360,30 +360,33 @@ __host__ __device__ inline size_t eq_offset(int len) { return (size_t)(len - 1) 
  * the cut.  Stoppers of the left scan (key <= pivot) and of the right scan (key >= pivot) are
  * listed in slots of the range itself; pair k = (k-th from the left, k-th from the right) is
  * swapped while the former lies left of the latter. */
+/* kWide: ranges may be long enough for the four-chunk trip (warp_sort_desc's never are: n <= 64). */
+template <bool kWide>
 __device__ __forceinline__ int warp_partition(const SortBufs& b, int f, int l, int lane, int levels_left) {
   unsigned short* a = b.a;
   if (lane == 0) median_to_first(a, f, l);
   __syncwarp();
-  const int p = a[f] >> 12;
+  /* key <= pivot and key >= pivot as compares of the raw entries (the key is the top four bits) */
+  const int p_lo = a[f] & 0xf000, p_hi = p_lo | 0xfff;
   const int m = l - f - 1, base = f + 1;
   const unsigned lt = (1u << lane) - 1u;
   int nl = 0, nr = 0;
   /* four chunks per trip while the range is long (the four loads are independent, so their
-   * latencies overlap), then one chunk at a time */
+   * latencies overlap), then one chunk at a time; c0 + 96 < m: only the fourth chunk can run past the range */
   int c0 = 0;
-  for (; c0 + 96 < m; c0 += 128) {
+  for (; kWide && c0 + 96 < m; c0 += 128) {
     int k[4];
     bool v[4];
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
       const int idx = c0 + 32 * q + lane;
-      v[q] = idx < m;
-      k[q] = v[q] ? (a[base + idx] >> 12) : 0;
+      v[q] = q < 3 || idx < m;
+      k[q] = v[q] ? a[base + idx] : 0;
     }
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
       const int idx = c0 + 32 * q + lane;
-      const bool fl = v[q] && k[q] <= p, fr = v[q] && k[q] >= p;
+      const bool fl = v[q] && k[q] <= p_hi, fr = v[q] && k[q] >= p_lo;
       const unsigned bl = __ballot_sync(kFull, fl), br = __ballot_sync(kFull, fr);
       if (fl) b.posl[base + nl + __popc(bl & lt)] = (unsigned short)(base + idx);
       if (fr) b.posr[base + nr + __popc(br & lt)] = (unsigned short)(base + idx);
@@ -394,8 +397,8 @@ __device__ __forceinline__ int warp_partition(const SortBufs& b, int f, int l, i
   for (; c0 < m; c0 += 32) {
     const int idx = c0 + lane;
     const bool valid = idx < m;
-    const int k = valid ? (a[base + idx] >> 12) : 0;
-    const bool fl = valid && k <= p, fr = valid && k >= p;
+    const int k = valid ? a[base + idx] : 0;
+    const bool fl = valid && k <= p_hi, fr = valid && k >= p_lo;
     const unsigned bl = __ballot_sync(kFull, fl), br = __ballot_sync(kFull, fr);
     if (fl) b.posl[base + nl + __popc(bl & lt)] = (unsigned short)(base + idx);
     if (fr) b.posr[base + nr + __popc(br & lt)] = (unsigned short)(base + idx);
@@ -507,7 +510,7 @@ __device__ __forceinline__ void sort_desc(const SortBufs& b, int n, int depth_li
     for (int s = warp; s < nseg; s += kWarps) {
       const unsigned sg = cur[s];
       const int f = sg & 0xffff, l = sg >> 16;
-      const int cut = warp_partition(b, f, l, lane, depth_limit - level);
+      const int cut = warp_partition<true>(b, f, l, lane, depth_limit - level);
       if (lane == 0 && cut >= 0) {   /* one slot request for both parts */
         const int nl_ = cut - f > kSortThreshold, nr_ = l - cut > kSortThreshold;
         if (nl_ + nr_) {
@@ -595,7 +598,7 @@ __device__ __forceinline__ void warp_sort_desc(const SortBufs& b, unsigned* stac
       __syncwarp();
       continue;
     }
-    const int cut = warp_partition(b, f, l, lane, depth_limit - depth);
+    const int cut = warp_partition<false>(b, f, l, lane, depth_limit - depth);
     if (cut >= 0) {
       if (l - cut > kSortThreshold) {
         if (lane == 0) stack[sp] = (unsigned)cut | ((unsigned)l << 12) | ((unsigned)(depth + 1) << 24);
