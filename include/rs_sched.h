@@ -324,6 +324,41 @@ int32_t rs_ue_rate_hist_bins(const rs_handle* h);
 int rs_ue_rate_hist_device(rs_handle* h, uint64_t* d_hist);
 int rs_get_ue_rate_hist(rs_handle* h, uint64_t* hist);
 
+/* ---- per-UE throughput over active time (UPT) histograms of a buffered handle ------------------------------------
+ * The bytes a UE received over a window divided by the TTIs it had data waiting: the service a bursty bearer got,
+ * where the throughput histogram above bins its offered load.  It rides on the throughput histogram's windows and
+ * snapshot (rs_close_ue_rate_window closes both); integers throughout:
+ *   active TTI      UE (b,u) is active at TTI t iff one of its slots showed q > 0 at step 2 of that TTI (what
+ *                   queue_out receives: after the TTI's arrival, before its departure).  A backlogged slot shows
+ *                   100 000 000, so a UE with one is active every TTI; a packet that arrives and leaves in the same TTI
+ *                   makes one active TTI; the run calls' `active` flags play no part.
+ *   active counts   n_a[b][u], uint32 [B][U] in device memory, the UE's active TTIs in the open window; a window must
+ *                   be shorter than 2^32 TTIs (not checked).
+ *   closing         d = c(b,u) - snap[b][u] (mod 2^64) as the throughput histogram takes it, before it moves snap;
+ *                   a UE with n_a > 0 adds one sample, bin = min((d / n_a) / bin_bytes, n_bins - 1) (two integer
+ *                   divisions, bin_bytes in bytes per TTI); a UE with n_a = 0 adds none; then n_a := 0.
+ *   bytes           the booked bytes (cum_bytes), as in every throughput this library reports: id 1 books its TBS
+ *                   uncapped, so with finite queues its bytes can exceed what left the FIFO, and so can its UPT.
+ *   row, storage    as the throughput histogram: [profile at close][that profile's slice], uint64 [P][S][n_bins].
+ *   restarts        rs_reset_state, rs_set_state with a non-NULL cum_bytes and rs_enable_ue_upt_hist zero n_a along
+ *                   with the snapshot change they make.
+ *   switching off   any rs_enable_ue_rate_hist call and rs_enable_buffers (again, or with 0); nothing else (run calls
+ *                   and rs_set_cell_profiles leave it).
+ * The counts come from a kernel launched after each TTI-kernel launch on the same stream; the schedules, state,
+ * buffers and the other histograms are the same bits with UPT on and off.
+ *
+ * rs_enable_ue_upt_hist: n_bins 1..RS_MAX_UE_RATE_BINS, or 0 to switch UPT off and free it; bin_bytes >= 1.
+ * RS_ERR_ARG on a handle without buffers, without the throughput histogram, or with a [P][S][n_bins] block over 2 GiB.
+ * Synchronous: waits for the work in flight, zeroes the counts and n_a and retakes the snapshot, which restarts the
+ * open window of both histograms (it adds no throughput samples and clears none).  rs_ue_upt_hist_bins: n_bins, 0 when
+ * off.  rs_ue_upt_hist_device writes DEVICE memory (P x S x n_bins uint64; feed it to an NCCL reduce,
+ * rs_reduce_ue_upt_hist); rs_get_ue_upt_hist copies to HOST; both ordered like rs_ue_rate_hist_device.  Every call but
+ * rs_enable_ue_upt_hist returns RS_ERR_ARG when UPT is off. */
+int rs_enable_ue_upt_hist(rs_handle* h, int32_t n_bins, int64_t bin_bytes);
+int32_t rs_ue_upt_hist_bins(const rs_handle* h);
+int rs_ue_upt_hist_device(rs_handle* h, uint64_t* d_hist);
+int rs_get_ue_upt_hist(rs_handle* h, uint64_t* hist);
+
 /* Synthetic arrivals into DEVICE int32 [n_ttis][B][U][nb] (bit-identical twin of radiosaber_b200/workload.py
  * synth_arrivals): pkt_bytes and pkts_q16 are HOST int32 [P][S] (P = rs_n_profiles; cell b reads the row of its
  * profile).  A bearer of slice s gets (q >> 16) + (draw16 < (q & 0xffff)) packets of pkt_bytes[s] bytes per TTI with

@@ -2713,6 +2713,65 @@ __global__ void rs_ue_rate_hist_kernel(const DevCfg d, unsigned long long* snap,
     if (s_cnt[i]) atomicAdd(&hist[(size_t)(i / smem_bins) * n_bins + i % smem_bins], (unsigned long long)s_cnt[i]);
 }
 
+/* ---- throughput over active time (rs_enable_ue_upt_hist, include/rs_sched.h) ---- */
+/* n_a [B][U] += the TTIs of one TTI-kernel launch at which the UE showed a slot with q > 0.  One thread per (cell, UE)
+ * of cells [cell_lo, cell_lo + n_cells), walking the launch's T TTIs of queue [T][B][U][nb] as that launch wrote it
+ * (B = n_batch, the handle's cells): for each t the threads read consecutive words.  One thread owns a UE, so a plain
+ * add.  B x U < 2^30 (the host): 32-bit indices within a TTI, 64-bit TTI offsets. */
+__global__ void rs_ue_active_kernel(const int* __restrict__ queue, unsigned* __restrict__ n_a, int n_batch, int cell_lo,
+                                    int n_cells, int U, int nb, int T) {
+  const unsigned r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= (unsigned)n_cells * (unsigned)U) return;
+  const unsigned ue = (unsigned)cell_lo * (unsigned)U + r;
+  const size_t per_tti = (size_t)n_batch * U * nb;
+  const int* q = queue + ue * (unsigned)nb;
+  unsigned k = 0;
+  if (nb == 2) {
+#pragma unroll 4
+    for (int t = 0; t < T; ++t) k += (q[(size_t)t * per_tti] > 0 || q[(size_t)t * per_tti + 1] > 0) ? 1u : 0u;
+  } else {
+#pragma unroll 4
+    for (int t = 0; t < T; ++t) k += q[(size_t)t * per_tti] > 0 ? 1u : 0u;
+  }
+  n_a[ue] += k;
+}
+
+/* Closing a window: one thread per (cell, UE), grid-stride; d = c - snap (mod 2^64) with c the sum of the UE's nb
+ * cum_bytes, read before rs_ue_rate_hist_kernel moves snap; a UE with n_a > 0 adds bin = min((d / n_a) / bin_bytes,
+ * n_bins - 1) to row [profile][slice] of the cell's profile now; n_a := 0.  Counting as rs_ue_rate_hist_kernel. */
+__global__ void rs_ue_upt_hist_kernel(const DevCfg d, const unsigned long long* snap, unsigned* n_a, int n_bins,
+                                      unsigned long long bin_bytes, unsigned long long* hist, int n_profiles,
+                                      int smem_bins) {
+  extern __shared__ unsigned s_cnt[];   /* [P][S][smem_bins] */
+  const int S = d.S, U = d.U, nb = d.nb;
+  const int n_smem = n_profiles * S * smem_bins;
+  for (int i = threadIdx.x; i < n_smem; i += blockDim.x) s_cnt[i] = 0;
+  __syncthreads();
+  const unsigned total = (unsigned)d.n_cells * (unsigned)U, stride = gridDim.x * blockDim.x;
+  /* warp-uniform trip count: every lane takes part in the warp votes of every round */
+  for (unsigned base = blockIdx.x * blockDim.x; base < total; base += stride) {
+    const unsigned r = base + threadIdx.x;
+    int row = -1, bin = 0;
+    if (r < total) {
+      const unsigned na = n_a[r];
+      if (na > 0) {
+        n_a[r] = 0;
+        const unsigned long long* cb = d.cum_bytes + (size_t)r * nb;
+        const unsigned long long c = nb == 2 ? cb[0] + cb[1] : cb[0];
+        const unsigned long long q = (c - snap[r]) / na / bin_bytes;
+        bin = q < (unsigned long long)(n_bins - 1) ? (int)q : n_bins - 1;
+        const int b = (int)(r / (unsigned)U), u = (int)(r % (unsigned)U);
+        const int pf = d.cell_profile ? d.cell_profile[b] : 0;
+        row = pf * S + d.ue_to_slice[(size_t)pf * U + u];
+      }
+    }
+    hol_hist_add(s_cnt, hist, row, bin, n_bins, smem_bins);
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < n_smem; i += blockDim.x)
+    if (s_cnt[i]) atomicAdd(&hist[(size_t)(i / smem_bins) * n_bins + i % smem_bins], (unsigned long long)s_cnt[i]);
+}
+
 #endif  /* RS_CORE_ONLY */
 
 }  // namespace RS_NS

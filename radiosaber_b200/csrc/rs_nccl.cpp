@@ -1,9 +1,9 @@
 /* rs_nccl.cpp -- include/rs_sched_nccl.h: the end-of-run NCCL reduce of the per-slice totals (SURVEY 8e),
  * include/rs_sched_nccl_buffers.h: the same for the per-slice buffer totals, include/rs_sched_nccl_hol_hist.h: the
- * same for the head-of-line delay histograms, and include/rs_sched_nccl_ue_rate.h: the same for the per-UE throughput
- * histograms.
+ * same for the head-of-line delay histograms, include/rs_sched_nccl_ue_rate.h: the same for the per-UE throughput
+ * histograms, and include/rs_sched_nccl_ue_upt.h: the same for the throughput over active time (UPT) histograms.
  * Uses only the public ABI of librs_sched.so plus NCCL and the CUDA runtime. */
-#include "../../include/rs_sched_nccl_ue_rate.h"
+#include "../../include/rs_sched_nccl_ue_upt.h"
 
 #include <cuda_runtime.h>
 #include <nccl.h>
@@ -119,6 +119,14 @@ int rs_reduce_ue_rate_hist(rs_handle* h, void* nccl_comm, int32_t root, uint64_t
     return nfail("rs_ue_rate_hist_device", "the handle has no throughput histogram (rs_enable_ue_rate_hist)");
   return reduce_totals(h, nccl_comm, root, hist_out, bins, rs_ue_rate_hist_device, "rs_reduce_ue_rate_hist",
                        "rs_ue_rate_hist_device");
+}
+
+int rs_reduce_ue_upt_hist(rs_handle* h, void* nccl_comm, int32_t root, uint64_t* hist_out) {
+  const int32_t bins = rs_ue_upt_hist_bins(h);   /* [P][S][bins]: bins rows per slice */
+  if (h && bins == 0)
+    return nfail("rs_ue_upt_hist_device", "the handle has no UPT histogram (rs_enable_ue_upt_hist)");
+  return reduce_totals(h, nccl_comm, root, hist_out, bins, rs_ue_upt_hist_device, "rs_reduce_ue_upt_hist",
+                       "rs_ue_upt_hist_device");
 }
 
 }  /* extern "C" */

@@ -301,6 +301,12 @@ struct rs_handle {
   int rate_bins = 0;
   unsigned long long rate_bin_bytes = 0;
   DevBuf<unsigned long long> rate_hist, rate_snap;
+  /* throughput over active time (rs_enable_ue_upt_hist): [P][S][upt_bins], 0 bins = off; upt_active [B][U] counts
+   * each UE's TTIs with data queued in the open window */
+  int upt_bins = 0;
+  unsigned long long upt_bin_bytes = 0;
+  DevBuf<unsigned long long> upt_hist;
+  DevBuf<unsigned> upt_active;
   DevBuf<int> tbs1;
   DevBuf<short> vogel_tab;
   DevBuf<unsigned long long> stats;
@@ -410,6 +416,13 @@ int launch_ttis(rs_handle* h, const rs::RunArgs& a0, bool trace, const rs::DevCf
     rs::rs_hol_hist_kernel<<<hgrid, 256, sizeof(unsigned) * 2 * h->d.S * h->P * smem_bins, st>>>(
         a.queue, a.hol, a.tbs_bits, h->buf_meta.p, h->d, h->B, a.cell_off, n, h->hist_bins, h->hist_per_unit, h->hist.p,
         h->P, smem_bins);
+    CU(cudaGetLastError());
+    h->launches++;
+  }
+  if (h->upt_bins > 0 && a.buf_k > 0) {   /* the active counts read the queues this launch showed, on the same stream */
+    const unsigned ues = (unsigned)n * (unsigned)h->d.U;   /* below 2^30 (rs_enable_ue_rate_hist) */
+    rs::rs_ue_active_kernel<<<(ues + 255) / 256, 256, 0, st>>>(a.queue, h->upt_active.p, h->B, a.cell_off, n, h->d.U,
+                                                               h->d.nb, a.T);
     CU(cudaGetLastError());
     h->launches++;
   }
@@ -597,7 +610,7 @@ void rs_destroy(rs_handle* h) {
   h->holmul.release(); h->tbs1.release(); h->vogel_tab.release();
   h->buf_meta.release(); h->buf_time.release(); h->buf_bytes.release(); h->shown_q.release(); h->shown_hol.release();
   h->synth_spec.release(); h->buf_scratch.release(); h->hist.release(); h->hist_tbs.release();
-  h->rate_hist.release(); h->rate_snap.release();
+  h->rate_hist.release(); h->rate_snap.release(); h->upt_hist.release(); h->upt_active.release();
   h->src_tab.release(); h->src_frames.release(); h->src_state.release();
   h->chn_tab.release(); h->cos_q14.release();
   if (h->own_stream) cudaStreamDestroy(h->own_stream);
@@ -968,6 +981,7 @@ int rs_reset_state(rs_handle* h) {
   CU(cudaMemset(h->tx.p, 0, BU * 4));
   CU(cudaMemset(h->cum_bytes.p, 0, BU * 8));
   if (h->rate_bins > 0) CU(cudaMemset(h->rate_snap.p, 0, (size_t)h->B * h->d.U * 8));   /* the open window restarts */
+  if (h->upt_bins > 0) CU(cudaMemset(h->upt_active.p, 0, (size_t)h->B * h->d.U * 4));
   CU(cudaMemset(h->cum_rbs.p, 0, BU * 8));
   CU(cudaMemset(h->offset.p, 0, BS * 8));
   CU(cudaMemset(h->ewma.p, 0, BS * 8));
@@ -988,6 +1002,7 @@ int rs_set_state(rs_handle* h, const double* avg_rate, const int32_t* tx_bytes, 
     std::vector<uint64_t> snap((size_t)h->B * h->d.U);
     for (size_t i = 0; i < snap.size(); ++i) snap[i] = nb == 2 ? cum_bytes[2 * i] + cum_bytes[2 * i + 1] : cum_bytes[i];
     CU(cudaMemcpy(h->rate_snap.p, snap.data(), snap.size() * 8, cudaMemcpyHostToDevice));
+    if (h->upt_bins > 0) CU(cudaMemset(h->upt_active.p, 0, snap.size() * 4));
   }
   if (cum_rbs) CU(cudaMemcpy(h->cum_rbs.p, cum_rbs, BU * 8, cudaMemcpyHostToDevice));
   if (slice_offset) CU(cudaMemcpy(h->offset.p, slice_offset, BS * 8, cudaMemcpyHostToDevice));
@@ -1698,6 +1713,8 @@ int rs_enable_buffers(rs_handle* h, int32_t max_records, const uint8_t* backlogg
   h->buf_backlogged.clear();
   h->hist_bins = 0;   /* the histogram is of the buffers: it goes with them */
   h->hist.release(); h->hist_tbs.release();
+  h->upt_bins = 0;    /* and so do the active counts */
+  h->upt_hist.release(); h->upt_active.release();
   h->last_now = -HUGE_VAL;
   if (max_records == 0) return RS_OK;
   const size_t n = (size_t)h->B * h->d.U * h->d.nb;
@@ -2160,6 +2177,8 @@ int rs_enable_ue_rate_hist(rs_handle* h, int32_t n_bins, int64_t bin_bytes) {
   if (rc != RS_OK) return rc;
   h->rate_bins = 0;
   h->rate_hist.release(); h->rate_snap.release();
+  h->upt_bins = 0;   /* UPT rides on the windows and snapshot replaced here */
+  h->upt_hist.release(); h->upt_active.release();
   if (n_bins == 0) return RS_OK;
   int sms = 0;
   CU(cudaSetDevice(h->device));
@@ -2186,6 +2205,13 @@ int rs_close_ue_rate_window(rs_handle* h) {
   const size_t rows = (size_t)h->P * h->d.S, BU = (size_t)h->B * h->d.U;   /* BU below 2^30 */
   const int smem_bins = hist_smem_bins(rows, h->rate_bins);
   const unsigned ctas = (unsigned)std::min<size_t>((BU + 255) / 256, (size_t)std::max(1, h->hist_ctas));
+  if (h->upt_bins > 0) {   /* first: it reads the snapshot the throughput histogram's kernel then moves */
+    const int upt_smem = hist_smem_bins(rows, h->upt_bins);
+    rs::rs_ue_upt_hist_kernel<<<ctas, 256, sizeof(unsigned) * rows * upt_smem, h->stream>>>(
+        h->d, h->rate_snap.p, h->upt_active.p, h->upt_bins, h->upt_bin_bytes, h->upt_hist.p, h->P, upt_smem);
+    CU(cudaGetLastError());
+    h->launches++;
+  }
   rs::rs_ue_rate_hist_kernel<<<ctas, 256, sizeof(unsigned) * rows * smem_bins, h->stream>>>(
       h->d, h->rate_snap.p, h->rate_bins, h->rate_bin_bytes, h->rate_hist.p, h->P, smem_bins);
   CU(cudaGetLastError());
@@ -2210,6 +2236,66 @@ int rs_get_ue_rate_hist(rs_handle* h, uint64_t* hist) {
     return fail(RS_ERR_ARG, "rs_get_ue_rate_hist: the handle has no throughput histogram (rs_enable_ue_rate_hist)");
   CU(cudaSetDevice(h->device));
   CU(cudaMemcpyAsync(hist, h->rate_hist.p, sizeof(uint64_t) * h->rate_hist.n, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  return RS_OK;
+}
+
+int rs_enable_ue_upt_hist(rs_handle* h, int32_t n_bins, int64_t bin_bytes) {
+  if (!h) return fail(RS_ERR_ARG, "null handle");
+  if (n_bins < 0 || n_bins > RS_MAX_UE_RATE_BINS)
+    return fail(RS_ERR_ARG, "rs_enable_ue_upt_hist: n_bins %d outside 0..%d", n_bins, RS_MAX_UE_RATE_BINS);
+  if (n_bins > 0 && bin_bytes < 1)
+    return fail(RS_ERR_ARG, "rs_enable_ue_upt_hist: bin_bytes %lld is not >= 1", (long long)bin_bytes);
+  if (n_bins > 0 && h->buf_k == 0)
+    return fail(RS_ERR_ARG, "rs_enable_ue_upt_hist: the handle has no buffers (rs_enable_buffers)");
+  if (n_bins > 0 && h->rate_bins == 0)
+    return fail(RS_ERR_ARG, "rs_enable_ue_upt_hist: the handle has no throughput histogram (rs_enable_ue_rate_hist)");
+  const size_t words = (size_t)h->P * h->d.S * (size_t)n_bins;
+  if (words * sizeof(uint64_t) > ((size_t)2 << 30))
+    return fail(RS_ERR_ARG, "rs_enable_ue_upt_hist: %d profiles x %d slices x %d bins of uint64 exceed 2 GiB", h->P,
+                h->d.S, n_bins);
+  const int rc = rs_sync(h);   /* the launches in flight add to the old counts and move the counters */
+  if (rc != RS_OK) return rc;
+  h->upt_bins = 0;
+  h->upt_hist.release(); h->upt_active.release();
+  if (n_bins == 0) return RS_OK;
+  CU(cudaSetDevice(h->device));
+  const size_t rows = (size_t)h->P * h->d.S, BU = (size_t)h->B * h->d.U;   /* BU below 2^30 (rs_enable_ue_rate_hist) */
+  CU(h->upt_hist.alloc(words));
+  CU(h->upt_active.alloc(BU));
+  /* the snapshot, retaken by the throughput histogram's kernel as one window of one bin into upt_hist (at least
+   * P x S words), whose samples are then cleared: the throughput histogram's own counts stay as they are */
+  const int smem_bins = hist_smem_bins(rows, 1);
+  const unsigned ctas = (unsigned)std::min<size_t>((BU + 255) / 256, (size_t)std::max(1, h->hist_ctas));
+  rs::rs_ue_rate_hist_kernel<<<ctas, 256, sizeof(unsigned) * rows * smem_bins, h->stream>>>(
+      h->d, h->rate_snap.p, 1, 1, h->upt_hist.p, h->P, smem_bins);
+  CU(cudaGetLastError());
+  h->launches++;
+  CU(cudaMemsetAsync(h->upt_hist.p, 0, words * sizeof(uint64_t), h->stream));
+  CU(cudaMemsetAsync(h->upt_active.p, 0, BU * sizeof(unsigned), h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  h->upt_bins = n_bins;
+  h->upt_bin_bytes = (unsigned long long)bin_bytes;
+  return RS_OK;
+}
+
+int32_t rs_ue_upt_hist_bins(const rs_handle* h) { return h ? h->upt_bins : 0; }
+
+int rs_ue_upt_hist_device(rs_handle* h, uint64_t* d_hist) {
+  if (!h || !d_hist) return fail(RS_ERR_ARG, "rs_ue_upt_hist_device: bad argument");
+  if (h->upt_bins == 0)
+    return fail(RS_ERR_ARG, "rs_ue_upt_hist_device: the handle has no UPT histogram (rs_enable_ue_upt_hist)");
+  CU(cudaSetDevice(h->device));
+  CU(cudaMemcpyAsync(d_hist, h->upt_hist.p, sizeof(uint64_t) * h->upt_hist.n, cudaMemcpyDeviceToDevice, h->stream));
+  return RS_OK;
+}
+
+int rs_get_ue_upt_hist(rs_handle* h, uint64_t* hist) {
+  if (!h || !hist) return fail(RS_ERR_ARG, "rs_get_ue_upt_hist: bad argument");
+  if (h->upt_bins == 0)
+    return fail(RS_ERR_ARG, "rs_get_ue_upt_hist: the handle has no UPT histogram (rs_enable_ue_upt_hist)");
+  CU(cudaSetDevice(h->device));
+  CU(cudaMemcpyAsync(hist, h->upt_hist.p, sizeof(uint64_t) * h->upt_hist.n, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
   return RS_OK;
 }

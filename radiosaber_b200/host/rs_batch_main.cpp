@@ -37,6 +37,13 @@
  *                                               (ue_rate_samples) and their 5th, 50th and 95th percentiles as bin
  *                                               indices (ue_rate_p5 / p50 / p95, null without samples).  The three go
  *                                               together
+ *            [--upt-bin-bytes X]                with --buffers and the three --rate-* flags: per-UE throughput over
+ *                                               active time histograms (rs_enable_ue_upt_hist; one rs_reduce_ue_upt_hist
+ *                                               with --gpus N): at each window's end every UE that had data queued in
+ *                                               k of its TTIs adds its bytes / k in --rate-bins bins of X bytes per TTI;
+ *                                               every line gains per slice the samples (upt_samples) and their 5th,
+ *                                               50th and 95th percentiles as bin indices (upt_p5 / p50 / p95, null
+ *                                               without samples)
  *            [--channel FILE ...]               synthetic channel CQI drawn on the device (rs_set_channels,
  *                                               rs_synth_channel) in place of rs_synth_cqi's i.i.d. draws, the file named
  *                                               once for every config or once per --config; not with --traces
@@ -94,7 +101,7 @@
 
 #include "rs_sched.h"
 #include "rs_sched_nccl.h"
-#include "rs_sched_nccl_ue_rate.h"
+#include "rs_sched_nccl_ue_upt.h"
 
 namespace {
 
@@ -179,6 +186,8 @@ struct Args {
   int rate_window = 0, rate_bins = 0;   /* --rate-window W --rate-bins N; 0 = no throughput histograms */
   long long rate_bin_bytes = 0;         /* --rate-bin-bytes X */
   int rate_given = 0;                   /* bits 1, 2, 4: which of the three flags were given */
+  long long upt_bin_bytes = 0;          /* --upt-bin-bytes X; 0 = no UPT histograms */
+  bool upt_given = false;
   uint64_t seed = 1;
   std::vector<std::string> configs, traffic, channel;
   std::string traces, mapping, log_prefix;
@@ -214,6 +223,7 @@ struct ShardResult {
   std::vector<uint64_t> buf_stats;   /* [P][3][S] (--buffers), the same way */
   std::vector<uint64_t> hol_hist;    /* [P][2][S][hol_bins] (--hol-bins), the same way */
   std::vector<uint64_t> rate_hist;   /* [P][S][rate_bins] (--rate-window), the same way */
+  std::vector<uint64_t> upt_hist;    /* [P][S][rate_bins] (--upt-bin-bytes), the same way */
   std::string log_out, log_err, error;
 };
 
@@ -451,6 +461,7 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
   const int rep = su.report;
   const int W = a.rate_window;   /* 0 = no throughput histograms */
   if (W > 0) check(rs_enable_ue_rate_hist(h, a.rate_bins, a.rate_bin_bytes), "rs_enable_ue_rate_hist");
+  if (a.upt_given) check(rs_enable_ue_upt_hist(h, a.rate_bins, a.upt_bin_bytes), "rs_enable_ue_upt_hist");
 
   /* ---- run in blocks of TB TTIs with everything resident on the device ------------------------------- */
   const int TB = 16;
@@ -609,6 +620,15 @@ void run_shard(const Setup& su, int gpu, int rank, int cell0, int nb, void* comm
       check(rs_get_ue_rate_hist(h, res->rate_hist.data()), "rs_get_ue_rate_hist");
     }
   }
+  if (a.upt_given) {
+    res->upt_hist.assign((size_t)S * P * a.rate_bins, 0);
+    if (comm) {
+      if (rs_reduce_ue_upt_hist(h, comm, 0, res->upt_hist.data()) != RS_OK)
+        throw std::runtime_error(std::string("rs_reduce_ue_upt_hist: ") + rs_nccl_last_error());
+    } else {
+      check(rs_get_ue_upt_hist(h, res->upt_hist.data()), "rs_get_ue_upt_hist");
+    }
+  }
   (void)rank;
   if (lg) {
     res->log_out = rs_log_stdout(lg, nullptr);
@@ -647,12 +667,14 @@ int main(int argc, char** argv) {
       else if (k == "--rate-window") { a.rate_window = atoi(next().c_str()); a.rate_given |= 1; }
       else if (k == "--rate-bins") { a.rate_bins = atoi(next().c_str()); a.rate_given |= 2; }
       else if (k == "--rate-bin-bytes") { a.rate_bin_bytes = strtoll(next().c_str(), nullptr, 10); a.rate_given |= 4; }
+      else if (k == "--upt-bin-bytes") { a.upt_bin_bytes = strtoll(next().c_str(), nullptr, 10); a.upt_given = true; }
       else throw std::runtime_error("unknown argument " + k);
     }
     if (a.configs.empty() || a.cells < 1 || a.ttis < 1 || a.trace_rows < 1 || a.gpus < 1 || a.gpus > a.cells) {
       fprintf(stderr, "usage: rs_batch --algo ID --config cfg.json [--config cfg2.json ...] --cells B --ttis T [--seed s] [--gpus N] "
                       "[--traces DIR --mapping FILE [--trace-rows N]] [--log-cell b --log-prefix P] [--buffers K --traffic FILE ...] "
-                      "[--channel FILE ...] [--hol-bins N] [--rate-window W --rate-bins N --rate-bin-bytes X]\n");
+                      "[--channel FILE ...] [--hol-bins N] [--rate-window W --rate-bins N --rate-bin-bytes X] "
+                      "[--upt-bin-bytes X]\n");
       return 2;
     }
     if (a.buffers != -1 && (a.buffers < 1 || a.buffers > RS_MAX_BUFFER_RECORDS))
@@ -669,6 +691,9 @@ int main(int argc, char** argv) {
     if (a.rate_given && (a.rate_bins < 1 || a.rate_bins > RS_MAX_UE_RATE_BINS))
       throw std::runtime_error("--rate-bins N: N bins, 1.." + std::to_string(RS_MAX_UE_RATE_BINS));
     if (a.rate_given && a.rate_bin_bytes < 1) throw std::runtime_error("--rate-bin-bytes X: X bytes per bin, >= 1");
+    if (a.upt_given && (a.buffers < 0 || a.rate_given != 7))
+      throw std::runtime_error("--upt-bin-bytes needs --buffers K and --rate-window W --rate-bins N --rate-bin-bytes X");
+    if (a.upt_given && a.upt_bin_bytes < 1) throw std::runtime_error("--upt-bin-bytes X: X bytes per TTI per bin, >= 1");
     if (!a.traffic.empty() && a.traffic.size() != 1 && a.traffic.size() != a.configs.size())
       throw std::runtime_error(std::to_string(a.traffic.size()) + " --traffic files for " + std::to_string(a.configs.size()) +
                                " --config files: give one for all or one per config");
@@ -821,6 +846,9 @@ int main(int argc, char** argv) {
       if (a.rate_window > 0)
         print_hist("ue_rate_samples", "ue_rate", res[0].rate_hist.data() + (size_t)p * S * a.rate_bins, S,
                    (size_t)a.rate_bins, {5, 50, 95});
+      if (a.upt_given)
+        print_hist("upt_samples", "upt", res[0].upt_hist.data() + (size_t)p * S * a.rate_bins, S, (size_t)a.rate_bins,
+                   {5, 50, 95});
       printf("]}\n");
     }
     for (int r = 0; r < N; ++r) {

@@ -44,6 +44,7 @@ ABI_SYMBOLS = (
     "rs_enable_hol_hist", "rs_hol_hist_bins", "rs_hol_hist_device", "rs_get_hol_hist",
     "rs_enable_ue_rate_hist", "rs_close_ue_rate_window", "rs_ue_rate_hist_bins", "rs_ue_rate_hist_device",
     "rs_get_ue_rate_hist",
+    "rs_enable_ue_upt_hist", "rs_ue_upt_hist_bins", "rs_ue_upt_hist_device", "rs_get_ue_upt_hist",
 )
 
 
@@ -210,6 +211,11 @@ def lib():
         L.rs_ue_rate_hist_bins.restype = C.c_int32
         L.rs_ue_rate_hist_device.argtypes = [C.c_void_p, C.c_void_p]
         L.rs_get_ue_rate_hist.argtypes = [C.c_void_p, C.c_void_p]
+        L.rs_enable_ue_upt_hist.argtypes = [C.c_void_p, C.c_int32, C.c_int64]
+        L.rs_ue_upt_hist_bins.argtypes = [C.c_void_p]
+        L.rs_ue_upt_hist_bins.restype = C.c_int32
+        L.rs_ue_upt_hist_device.argtypes = [C.c_void_p, C.c_void_p]
+        L.rs_get_ue_upt_hist.argtypes = [C.c_void_p, C.c_void_p]
         _lib = L
     return _lib
 
@@ -654,6 +660,25 @@ class Scheduler:
         """rs_ue_rate_hist_device into a DEVICE buffer of n_profiles * S * n_bins uint64."""
         _check(lib().rs_ue_rate_hist_device(self._h, C.c_void_p(d_hist)))
 
+    def enable_ue_upt_hist(self, n_bins, bin_bytes):
+        """Count histograms of each UE's throughput over the TTIs it had data queued (rs_enable_ue_upt_hist; 0 = off)
+        on a buffered handle with enable_ue_rate_hist on: each close_ue_rate_window adds, for every UE with k > 0
+        such TTIs in the window, bin = min(bytes in the window // k // bin_bytes, n_bins - 1) to [profile][slice].
+        Waits for the work in flight, zeroes the counts and restarts the open window.  Twin: workload.ue_upt_hist."""
+        _check(lib().rs_enable_ue_upt_hist(self._h, int(n_bins), int(bin_bytes)))
+
+    def get_ue_upt_hist(self):
+        """uint64 [P][S][n_bins]: the UPT histograms of the windows closed since enable_ue_upt_hist
+        (rs_get_ue_upt_hist)."""
+        n = int(lib().rs_ue_upt_hist_bins(self._h))
+        hist = np.empty((self.n_profiles, self.S, max(n, 1)), dtype=np.uint64)
+        _check(lib().rs_get_ue_upt_hist(self._h, _ptr(hist)))
+        return hist
+
+    def ue_upt_hist_device(self, d_hist):
+        """rs_ue_upt_hist_device into a DEVICE buffer of n_profiles * S * n_bins uint64."""
+        _check(lib().rs_ue_upt_hist_device(self._h, C.c_void_p(d_hist)))
+
     def synth_arrivals(self, seed, cell0, tti0, n_ttis, pkt_bytes, pkts_q16, d_out):
         """rs_synth_arrivals: int32 [n_ttis][B][U][nb] into device memory; pkt_bytes / pkts_q16: int [P][S] (packet
         size, packets per TTI in 16.16 fixed point) per slice of each profile.  Twin of workload.synth_arrivals."""
@@ -1061,7 +1086,7 @@ def test_sort_timed(keys, reps=20, depth_limit=-1, device=0):
 def hist_percentile(hist, q):
     """The q-th percentile (an integer 0..100) of one histogram, as a bin index: the smallest bin d with
     100 * (samples in bins 0..d) >= q * (all samples), in integers; None when it holds no samples.  rs_batch reports
-    its hol_*_p50 / p95 / p99 and ue_rate_p5 / p50 / p95 by the same rule."""
+    its hol_*_p50 / p95 / p99, ue_rate_p5 / p50 / p95 and upt_p5 / p50 / p95 by the same rule."""
     if isinstance(q, bool) or not isinstance(q, (int, np.integer)) or not 0 <= q <= 100:
         raise ValueError(f"q = {q!r}: an integer percentile 0..100")
     counts = [int(x) for x in np.asarray(hist).reshape(-1)]

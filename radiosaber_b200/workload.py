@@ -391,3 +391,28 @@ def ue_rate_hist(cum_start, cum_end, ue_to_slice, n_slices: int, n_bins: int, bi
     cp = np.zeros(B, dtype=np.int64) if cell_profile is None else np.asarray(cell_profile, dtype=np.int64)
     idx = ((cp[:, None] * S + u2s[cp]) * n_bins + bins).reshape(-1)
     return np.bincount(idx, minlength=P * S * n_bins).astype(np.uint64).reshape(P, S, n_bins)
+
+
+def ue_upt_hist(queue, cum_start, cum_end, ue_to_slice, n_slices: int, n_bins: int, bin_bytes: int,
+                cell_profile=None) -> np.ndarray:
+    """uint64 [P][S][n_bins]: the samples one ``rs_close_ue_rate_window`` adds to the throughput-over-active-time
+    histograms (``rs_enable_ue_upt_hist``; the device twin, bit for bit).
+
+    queue: the queues the window's TTIs showed, int32 [T][B][U] or [T][B][U][2] (``queue_out``, concatenated over the
+    window's run calls); cum_start / cum_end and the profiles as in ``ue_rate_hist``.  A UE is active at a TTI where one
+    of its slots shows q > 0; with k > 0 active TTIs it adds bin = min(d // k // bin_bytes, n_bins - 1), d its bytes
+    in the window mod 2^64; with k = 0 it adds nothing."""
+    a = np.asarray(cum_start, dtype=np.uint64)
+    b = np.asarray(cum_end, dtype=np.uint64)
+    B, U = b.shape[:2]
+    q = np.asarray(queue)
+    k = (q.reshape(q.shape[0], B, U, -1) > 0).any(axis=3).sum(axis=0).astype(np.uint64)
+    with np.errstate(over="ignore"):   # uint64 arithmetic wraps, as on the device
+        d = b.reshape(B, U, -1).sum(axis=2, dtype=np.uint64) - a.reshape(B, U, -1).sum(axis=2, dtype=np.uint64)
+    act = k > 0
+    bins = np.minimum(d[act] // k[act] // np.uint64(bin_bytes), np.uint64(n_bins - 1)).astype(np.int64)
+    u2s = np.atleast_2d(np.asarray(ue_to_slice, dtype=np.int64))
+    P, S = u2s.shape[0], int(n_slices)
+    cp = np.zeros(B, dtype=np.int64) if cell_profile is None else np.asarray(cell_profile, dtype=np.int64)
+    idx = ((cp[:, None] * S + u2s[cp]) * n_bins)[act] + bins
+    return np.bincount(idx, minlength=P * S * n_bins).astype(np.uint64).reshape(P, S, n_bins)
